@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — env agent-steps/s of the fused step+observe hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c5] [--dump-outputs DIR]
 
 One "step" = one lockstep Environment.step (+ the observe it ends in) over the whole batch of synthetic environments.
 --config selects the BASELINE.json configuration (default c2 = configs[1], the one the metric is quoted on):
@@ -267,6 +267,31 @@ def bench_config(args, env=None, extra=None):
 
 
 # ---- GPU arm -------------------------------------------------------------------------------------------------------------------
+DUMP_BYTES = 48_000_000  # --dump-outputs writes at most this much
+
+
+def last_step_sample(obs, rewards, done, steps):
+    """--dump-outputs: what the rollout returned for its last step (observations uint8[B,N,6,9,9], rewards float32[B,N],
+    done uint8[B], step counters int32[B]) as float32 host arrays, restricted to a fixed seeded sample of the environments
+    so that the files stay under DUMP_BYTES; `env_index` names the sampled environments."""
+    import torch
+    B, N = rewards.shape
+    per_env = 4 * (N * 6 * 9 * 9 + N + 2) + 8
+    count = max(1, min(B, DUMP_BYTES // per_env))
+    envs = np.sort(np.random.default_rng(0).choice(B, size=count, replace=False))
+    idx = torch.as_tensor(envs, device=rewards.device)
+    out = {name: t.index_select(0, idx).float().cpu().numpy()
+           for name, t in (("obs", obs), ("rewards", rewards), ("done", done), ("steps", steps))}
+    out["env_index"] = envs.astype(np.float64)
+    return out
+
+
+def write_dump(directory, arrays):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def greedy_script(env, T, seed, device):
     """Navi-greedy actions with epsilon 0.1 (SURVEY 8(d) stream G) for T steps from the env's current state: each agent follows
     a set direction bit of its own cell (channels 2..5 of its observation), else stays.  The env is stepped while the script
@@ -357,6 +382,7 @@ def run_ours(args):
 
     # warm-up: W whole-batch steps, then keep stepping until the clocks have had ~0.3 s of load
     arm(False)
+    pos0, steps0 = env.agents_pos.clone(), env.steps.clone()
     for s in range(args.warmup):
         env.step(actions[s % A], out_obs=replay[s % R])
     t0 = time.perf_counter()
@@ -367,6 +393,9 @@ def run_ours(args):
             s += 1
         torch.cuda.synchronize(dev)
     env.check()
+    # the warm-up runs for a fixed time, so its number of steps varies: the timed region starts from the state before it, so
+    # that the same arguments give the same inputs in every run
+    env.set_state(agents_pos=pos0, steps=steps0)
 
     out_ring = 2
     rew_ring = torch.empty((out_ring, B, N), dtype=torch.float32, device=dev)
@@ -404,6 +433,9 @@ def run_ours(args):
     ep0 = int(env.episode_counts().sum()) if cap > 0 else 0
     ms_local = timed_rollout(K)
     env.check()
+    if args.dump_outputs and rank == 0:
+        last = (K - 1) % R, (K - 1) % out_ring
+        dump = last_step_sample(replay[last[0]], rew_ring[last[1]], done_ring[last[1]], steps_ring[last[1]])
     ms_all = sharding.gather_floats(ms_local, dev)
     ms = max(ms_all)
     value = world * B * N * K / (ms * 1e-3)
@@ -531,6 +563,8 @@ def run_ours(args):
             goals = env.goals_pos[:S].cpu().numpy()
             line["cpu_baseline"] = cpu_baseline(maps, agents, goals, N, L, seconds=args.cpu_seconds)
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            write_dump(args.dump_outputs, dump)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -558,6 +592,8 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--learner-every", type=int, default=4, help="c5: one learner update every this many actor steps")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the timed rollout returned for its last step (rank 0) as DIR/<name>.npy (c2, c3, c4)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     c = CONFIGS[args.config]
@@ -567,6 +603,8 @@ def main():
     args.density = args.density if args.density >= 0 else c["density"]
     args.max_steps = args.max_steps or c["max_steps"]
     args.scaling = args.scaling or c["scaling"]
+    if args.dump_outputs and (args.impl != "ours" or args.config == "c5"):
+        ap.error("--dump-outputs is implemented for the rollout of --impl ours (configs c2, c3, c4)")
 
     if args.impl == "reference":
         run_reference(args)

@@ -46,6 +46,33 @@ def random_instance(rng, L, N, density):
     return m, a.astype(np.uint8), g.astype(np.uint8)
 
 
+# high-occupancy small boards (map_length, num_agents, density, seed): every conflict kind of environment.py:320-406 fires
+RANDOM_GRID_CASES = [
+    (3, 5, 0.0, 0), (3, 8, 0.0, 1), (4, 12, 0.0, 2), (4, 15, 0.0, 3), (5, 20, 0.0, 4), (6, 30, 0.0, 5),
+    (6, 20, 0.15, 6), (8, 30, 0.2, 7), (10, 40, 0.3, 8), (12, 64, 0.1, 9), (2, 3, 0.0, 10), (2, 4, 0.0, 11),
+]
+
+
+def random_grid_trials(L, N, density, seed, trials=6, steps=40):
+    """-> [(map, agents, goals, actions uint8[steps,N])] of one RANDOM_GRID_CASES entry: uniform actions, everybody
+    moving, and moving with 20 % staying, in turn."""
+    rng = np.random.default_rng(seed)
+    out = []
+    for _ in range(trials):
+        m, a, g = random_instance(rng, L, N, density)
+        acts = np.empty((steps, N), dtype=np.uint8)
+        for s in range(steps):
+            mode = s % 3
+            if mode == 0:
+                acts[s] = rng.integers(0, 5, size=N)
+            elif mode == 1:
+                acts[s] = rng.integers(1, 5, size=N)          # everybody moves
+            else:
+                acts[s] = np.where(rng.random(N) < 0.2, 0, rng.integers(1, 5, size=N))
+        out.append((m, a, g, acts))
+    return out
+
+
 # ---- instance-generator statistics (SURVEY 8f-3): the same numbers are computed for the live reference
 # (tests/golden/make_golden.py -> generator_stats.npz), the host generator and the device generator ----
 GEN_CONFIGS = [(20, 6), (12, 4)]  # (map_length, num_agents): the reference default (config.py) and a small, fragmented one

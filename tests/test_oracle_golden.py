@@ -5,7 +5,7 @@ import hashlib
 import numpy as np
 import pytest
 
-from helpers import golden, instances
+from helpers import RANDOM_GRID_CASES, golden, instances
 from oracle import oracle
 
 
@@ -93,3 +93,26 @@ def test_actor_td():
     for case in range(5):
         td = oracle.actor_td(z[f"td_rew_{case}"], z[f"td_q_{case}"], z[f"td_act_{case}"])
         assert np.array_equal(td, z[f"td_out_{case}"]), case
+
+
+@pytest.mark.parametrize("case", range(len(RANDOM_GRID_CASES)))
+def test_random_grids_recorded(case):
+    """The oracle on the high-occupancy random boards of helpers.RANDOM_GRID_CASES against its recorded trajectories
+    (tests/golden/make_random_grids.py; test_oracle_vs_reference.py checks the same boards against the live reference)."""
+    z = golden("random_grids.npz")
+    pre = f"c{case}_"
+    for t in range(z[pre + "map"].shape[0]):
+        env = oracle.OracleEnv()
+        env.load(z[pre + "map"][t], z[pre + "agents"][t], z[pre + "goals"][t])
+        assert sha8(np.ascontiguousarray(env.navi_map, dtype=np.uint8).tobytes()) == z[pre + "navi_sha8"][t]
+        obs, pos = env.observe()
+        assert np.array_equal(pos, z[pre + "pos"][t, 0])
+        assert sha8(obs.astype(np.uint8).tobytes()) == z[pre + "obs_sha8"][t, 0]
+        for s, acts in enumerate(z[pre + "actions"][t]):
+            (obs, pos), r, d, info = env.step(acts.tolist())
+            assert info == {"step": s}
+            assert np.array_equal(pos, z[pre + "pos"][t, s + 1]), (t, s)
+            assert np.array_equal(np.asarray(r, dtype=np.float32), z[pre + "rewards"][t, s]), (t, s)
+            assert int(d) == z[pre + "done"][t, s], (t, s)
+            assert sha8(obs.astype(np.uint8).tobytes()) == z[pre + "obs_sha8"][t, s + 1], (t, s)
+        assert np.array_equal(np.packbits(obs.astype(np.uint8).ravel()), z[pre + "obs_last_packed"][t])

@@ -1,6 +1,7 @@
-"""CPU, dev container only: the C oracle (oracle/mapf_oracle.c) against the LIVE reference loaded from
-/root/reference through oracle/ref_loader.py.  Skipped where the reference is not mounted (GPU box);
-there the oracle is pinned by the committed golden vectors instead (tests/test_oracle_golden.py).
+"""CPU: the C oracle (oracle/mapf_oracle.c) against the LIVE reference loaded through oracle/ref_loader.py
+(MAPF_REFERENCE_DIR).  The tests that need the live reference are skipped where it is not installed; there the
+oracle is pinned by the committed golden vectors instead (tests/test_oracle_golden.py).  The known-answer hashes
+need only the committed copy of the reference's test instances and run everywhere.
 
 Covers what the golden files cannot hold in bulk: random small grids at high occupancy (where the
 swap / vertex / back-propagation logic of environment.py:335-406 actually fires), the SURVEY
@@ -11,10 +12,10 @@ import hashlib
 import numpy as np
 import pytest
 
-from helpers import random_instance
+from helpers import RANDOM_GRID_CASES, instances, random_grid_trials, random_instance
 from oracle import oracle, ref_loader
 
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted")
+needs_reference = pytest.mark.skipif(not ref_loader.available(), reason="the reference is not installed (MAPF_REFERENCE_DIR)")
 
 
 def _ref_env(m, a, g):
@@ -44,7 +45,7 @@ KNOWN = {
 @pytest.mark.parametrize("N,k", sorted(KNOWN))
 def test_known_answer_hashes_oracle(N, k):
     """The oracle alone reproduces the hashes the surveyor took from the reference (Appendix B)."""
-    maps, agents, goals = ref_loader.load_pkl(N)
+    maps, agents, goals = instances(N)
     acts = np.random.default_rng(0).integers(0, 5, size=(64, N))
     env = _ora_env(maps[k], agents[k], goals[k])
     navi_padded = np.pad(env.navi_map, ((0, 0), (0, 0), (4, 4), (4, 4)))
@@ -65,25 +66,14 @@ def test_known_answer_hashes_oracle(N, k):
     assert (navi_sha, h.hexdigest()[:16], coll, int(pos.sum())) == want
 
 
-@pytest.mark.parametrize("L,N,density,seed", [
-    (3, 5, 0.0, 0), (3, 8, 0.0, 1), (4, 12, 0.0, 2), (4, 15, 0.0, 3), (5, 20, 0.0, 4), (6, 30, 0.0, 5),
-    (6, 20, 0.15, 6), (8, 30, 0.2, 7), (10, 40, 0.3, 8), (12, 64, 0.1, 9), (2, 3, 0.0, 10), (2, 4, 0.0, 11),
-])
+@needs_reference
+@pytest.mark.parametrize("L,N,density,seed", RANDOM_GRID_CASES)
 def test_random_grids_step_observe(L, N, density, seed):
     """High-occupancy small boards: every conflict kind of environment.py:320-406 fires."""
-    rng = np.random.default_rng(seed)
-    for trial in range(6):
-        m, a, g = random_instance(rng, L, N, density)
+    for trial, (m, a, g, steps) in enumerate(random_grid_trials(L, N, density, seed)):
         ref, ora = _ref_env(m, a, g), _ora_env(m, a, g)
         assert np.array_equal(ref.navi_map[:, :, 4:-4, 4:-4].astype(np.uint8), ora.navi_map)
-        for s in range(40):
-            mode = s % 3
-            if mode == 0:
-                acts = rng.integers(0, 5, size=N)
-            elif mode == 1:
-                acts = rng.integers(1, 5, size=N)          # everybody moves
-            else:
-                acts = np.where(rng.random(N) < 0.2, 0, rng.integers(1, 5, size=N))
+        for s, acts in enumerate(steps.astype(np.int64)):
             (ro, rp), rr, rd, ri = ref.step(acts.tolist())
             (oo, op), orr, od, oi = ora.step(acts.tolist())
             assert np.array_equal(rp, op), (trial, s)
@@ -92,6 +82,7 @@ def test_random_grids_step_observe(L, N, density, seed):
             assert np.array_equal(ro.astype(np.uint8), oo.astype(np.uint8)), (trial, s)
 
 
+@needs_reference
 def test_finish_and_step_after_done():
     """environment.py:415-419: all rewards become `finish`; the env keeps stepping after done."""
     m = np.zeros((3, 3), dtype=np.uint8)
@@ -103,6 +94,7 @@ def test_finish_and_step_after_done():
         assert np.array_equal(rp, op) and list(map(float, rr)) == list(map(float, orr)) and bool(rd) == od and ri == oi
 
 
+@needs_reference
 def test_distances_vs_compute_heuristics_live():
     search = ref_loader.load_module("search")
     rng = np.random.default_rng(3)
@@ -117,6 +109,7 @@ def test_distances_vs_compute_heuristics_live():
             assert np.array_equal(dist[i], want)
 
 
+@needs_reference
 def test_sumtree_vs_buffer_py():
     buf = ref_loader.load_module("buffer")
     rng = np.random.default_rng(5)
@@ -138,6 +131,7 @@ def test_sumtree_vs_buffer_py():
             assert np.array_equal(ri, oi) and np.array_equal(rp, op), rnd
 
 
+@needs_reference
 def test_actor_td_vs_local_buffer_finish():
     buf = ref_loader.load_module("buffer")
     rng = np.random.default_rng(7)

@@ -1,7 +1,7 @@
 """The batched PyTorch restatement of the Q-network glue (mapf_rl_b200/qnet.py) against the live reference
-model (model.py:139-263), CPU fp32, dev container only (the reference is not on the GPU box).  The network is
-outside the hand-written kernels; this pins that a reference checkpoint / seed gives the same Q-values through
-the batched path, to fp32 round-off (1e-5 relative)."""
+model (model.py:139-263), CPU fp32, where the reference is installed (MAPF_REFERENCE_DIR); the architecture test runs
+everywhere.  The network is outside the hand-written kernels; this pins that a reference checkpoint / seed gives the
+same Q-values through the batched path, to fp32 round-off (1e-5 relative)."""
 import numpy as np
 import pytest
 import torch
@@ -9,7 +9,7 @@ import torch
 from helpers import instances
 from oracle import oracle, ref_loader
 
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not mounted")
+needs_reference = pytest.mark.skipif(not ref_loader.available(), reason="the reference is not installed (MAPF_REFERENCE_DIR)")
 
 
 def nets():
@@ -22,6 +22,22 @@ def nets():
     return ref, mine
 
 
+def test_architecture_of_reference_model():
+    """Without the reference: the layer shapes and the parameter count SURVEY.md section 2 took from model.py:147-170
+    (conv 6->128 3x3, three residual blocks, 1x1 conv ->16, GRUCell 784->256, 2-head attention comm block with a GRU
+    update, dueling head over 5 actions; 2,050,582 parameters), so a reference checkpoint still has a place for every tensor."""
+    from mapf_rl_b200 import qnet
+    sd = qnet.Network().state_dict()
+    assert tuple(sd["obs_encoder.0.weight"].shape) == (128, 6, 3, 3)
+    assert [tuple(sd[f"obs_encoder.{i}.block{j}.weight"].shape) for i in (2, 3, 4) for j in (1, 2)] == [(128, 128, 3, 3)] * 6
+    assert tuple(sd["obs_encoder.5.weight"].shape) == (16, 128, 1, 1)
+    assert tuple(sd["recurrent.weight_ih"].shape) == (3 * 256, 16 * 7 * 7) and tuple(sd["recurrent.weight_hh"].shape) == (3 * 256, 256)
+    assert tuple(sd["comm.update_cell.weight_hh"].shape) == (3 * 256, 256)
+    assert tuple(sd["adv.weight"].shape) == (5, 256) and tuple(sd["state.weight"].shape) == (1, 256)
+    assert sum(v.numel() for v in sd.values()) == 2050582
+
+
+@needs_reference
 def test_same_seed_same_weights_and_checkpoint_compatible():
     ref, mine = nets()
     sd_r, sd_m = ref.state_dict(), mine.state_dict()
@@ -32,6 +48,7 @@ def test_same_seed_same_weights_and_checkpoint_compatible():
     assert sum(p.numel() for p in mine.parameters()) == 2050582  # SURVEY section 2
 
 
+@needs_reference
 def test_step_matches_reference_per_env():
     ref, mine = nets()
     maps, agents, goals = instances(16)
@@ -61,6 +78,7 @@ def test_step_matches_reference_per_env():
             e.step(rng.integers(0, 5, size=16))
 
 
+@needs_reference
 def test_bootstrap_matches_reference():
     ref, mine = nets()
     cfg = ref_loader.load_module("config")
