@@ -18,7 +18,8 @@
 // Randomness is counter-based (Philox4x32-10): the instance with global index g uses key (seed) and counters
 // (g, purpose, index), so any sharding of a batch over GPUs draws the instances a single GPU would.  The RNG stream of the
 // reference (numpy / random globals) is NOT reproduced: parity with the reference goes through Environment.load; this
-// generator is tested distributionally.
+// generator is tested distributionally against the reference, and instance by instance against a host restatement of the
+// rules above (tests/generator_ref.py).
 #pragma once
 #include "mapf_common.cuh"
 

@@ -1,6 +1,7 @@
 """GPU: the device-side instance generator (mapf_env_reset, Environment.reset / __init__ of
 environment.py:100-138, 146-196) — distributional parity only (the reference's RNG stream is not reproduced,
-SURVEY 8c), plus exact consistency of everything derived from a generated instance with the oracle."""
+SURVEY 8c), plus exact consistency of everything derived from a generated instance with the oracle.  Instance-by-instance
+equality with a host restatement of the generator is in test_generator_ref.py."""
 import numpy as np
 import pytest
 
