@@ -46,6 +46,7 @@ extern "C" {
                               IndexError on the same input; two agents on one cell latch MAPF_EUNIQUE) */
 #define MAPF_EINTERNAL (-8) /* the rollout scheduler gave up waiting for a chunk hand-over (a bug, never expected) */
 #define MAPF_EINDEX (-9)   /* sum tree: a leaf index outside [0, capacity) was skipped (numpy raises IndexError) */
+#define MAPF_EPRIORITY (-10) /* sum tree: a sampled leaf has priority 0 (the reference asserts priorities > 0, buffer.py:74) */
 
 /* Reward codes: the position of an agent's reward in reward_fn (config.py:8-12).  Every step entry point can emit these
  * u8 codes instead of / next to the fp32 rewards: a reward takes one of five values, so the host side of an actor reads
@@ -289,7 +290,9 @@ int mapf_per_update(mapf_per *tree, const int64_t *d_idx, const double *d_prio, 
 
 /* SumTree.batch_sample (buffer.py:56-78) with caller-supplied uniforms u in [0,1):
  * prefix_i = i*interval + u_i*interval.  d_weight_out (optional) = (p / min_batch p)^(-beta)
- * (worker.py:165-166; fp32 powf, 1e-6 relative).  d_idx_out is non-decreasing (stratified prefixes). */
+ * (worker.py:165-166; fp32 powf, 1e-6 relative).  d_idx_out is non-decreasing (stratified prefixes).  A sampled leaf
+ * whose priority is not > 0 (buffer.py:74 asserts) is returned as the reference finds it and latches MAPF_EPRIORITY
+ * (mapf_per_status). */
 int mapf_per_sample(mapf_per *tree, const double *d_uniforms, int64_t batch, int64_t *d_idx_out,
                     double *d_prio_out, float *d_weight_out, double beta, void *stream);
 
@@ -333,7 +336,10 @@ typedef struct mapf_per_cycle_args {
 int mapf_per_cycle(mapf_per *tree, const mapf_per_cycle_args *args, void *stream);
 
 /* Synchronous: MAPF_EINDEX if an update since the last call was handed a leaf index outside [0, capacity) (such entries
- * are skipped), else MAPF_OK; clears the latch.  One tree handle is used from one stream at a time. */
+ * are skipped), MAPF_EPRIORITY if a sample (mapf_per_sample, mapf_per_cycle) returned a leaf whose priority is not > 0
+ * (indices and priorities are still the reference's; the weights of that batch are undefined), else MAPF_OK.  Reports
+ * one condition per call, MAPF_EINDEX first, and clears only its latch, so a second condition is reported by the next
+ * call.  One tree handle is used from one stream at a time. */
 int mapf_per_status(mapf_per *tree, void *stream);
 
 /* LocalBuffer.finish TD (buffer.py:170-177) for `episodes` episodes of up to `capacity` steps:

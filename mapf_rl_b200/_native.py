@@ -10,7 +10,7 @@ from . import build as _build
 _lib = None
 
 MAPF_OK, MAPF_EINVAL, MAPF_ECUDA, MAPF_EACTION, MAPF_EUNIQUE, MAPF_ENOMEM, MAPF_ENOSPACE = 0, -1, -2, -3, -4, -5, -6
-MAPF_ESTATE, MAPF_EINTERNAL, MAPF_EINDEX = -7, -8, -9
+MAPF_ESTATE, MAPF_EINTERNAL, MAPF_EINDEX, MAPF_EPRIORITY = -7, -8, -9, -10
 ABI_VERSION = 2
 # reward codes (MAPF_RCODE_*): index into reward_fn in config.REWARD_ORDER; 5 = reset step (reward 0)
 RCODE_RESET = 5
@@ -138,4 +138,6 @@ def check(code: int):
             raise RuntimeError(msg)  # 'unique' (environment.py:428) / 'no empty position' (environment.py:31)
         if code in (MAPF_ESTATE, MAPF_EINDEX):
             raise IndexError(msg)    # what numpy raises on an out-of-range coordinate / leaf index
+        if code == MAPF_EPRIORITY:
+            raise AssertionError(msg)  # assert np.all(priorities > 0) (buffer.py:74)
         raise MapfError(code, msg)

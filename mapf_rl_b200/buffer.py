@@ -174,7 +174,10 @@ class SumTree:
 
     def check(self):
         """Synchronous: IndexError if an update was handed a leaf index outside [0, capacity) since the last call (numpy
-        raises at once; the kernels skip the entry and latch)."""
+        raises at once; the kernels skip the entry and latch); AssertionError if a sample (`sample_device`, `cycle`)
+        returned a leaf whose priority is not > 0 (the reference asserts at once, buffer.py:74; the kernels return the
+        leaf the reference's descent finds, and the importance weights of that batch are undefined).  One condition is
+        raised per call, the index one first; a second latched condition is raised by the next call."""
         _native.check(self._lib.mapf_per_status(self._h, self._stream()))
 
     # -- reference numpy API -------------------------------------------------------------------

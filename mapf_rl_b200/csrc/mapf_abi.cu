@@ -1186,13 +1186,18 @@ int mapf_per_status(mapf_per *t, void *stream)
     int32_t bits = 0;
     MAPF_CUDA(cudaMemcpyAsync(&bits, t->scratch.err, 4, cudaMemcpyDeviceToHost, st));
     MAPF_CUDA(cudaStreamSynchronize(st));
-    if (bits) {
-        MAPF_CUDA(cudaMemsetAsync(t->scratch.err, 0, 4, st));
-        MAPF_CUDA(cudaStreamSynchronize(st));
+    // one condition per call, and only its bit is cleared: a second latched condition surfaces on the next call
+    const int32_t bit = (bits & MAPF_ERRBIT_INDEX) ? MAPF_ERRBIT_INDEX : (bits & MAPF_ERRBIT_PRIORITY);
+    if (!bit) return MAPF_OK;
+    const int32_t rest = bits & ~bit;
+    MAPF_CUDA(cudaMemcpyAsync(t->scratch.err, &rest, 4, cudaMemcpyHostToDevice, st));
+    MAPF_CUDA(cudaStreamSynchronize(st));
+    if (bit == MAPF_ERRBIT_INDEX) {
         mapf_set_error("sum tree: leaf index outside [0, capacity) (skipped)");
         return MAPF_EINDEX;
     }
-    return MAPF_OK;
+    mapf_set_error("sum tree: a sampled leaf's priority is not > 0 (buffer.py:74 asserts priorities > 0)");
+    return MAPF_EPRIORITY;
 }
 
 int mapf_actor_td_n(const float *d_rew, const float *d_q, const uint8_t *d_act, const int32_t *d_size, int32_t episodes,

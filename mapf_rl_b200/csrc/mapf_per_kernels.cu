@@ -302,10 +302,12 @@ __device__ __forceinline__ bool descend(double &p, const double left)
 // SumTree.batch_sample, buffer.py:56-78.  One thread per sample; the top of the tree comes from shared memory (`top_ready`:
 // the update has just left its refreshed copy there), the rest in round trips of three levels (file header).  `tree` may have
 // been written by this CTA just before (a barrier lies between; plain loads: ld.global.cg compiles to LDG.STRONG.GPU, which
-// measured ~2.5x the latency of a weak load here).  Nodes by 1-based heap index j (children 2j, 2j + 1).
+// measured ~2.5x the latency of a weak load here).  Nodes by 1-based heap index j (children 2j, 2j + 1).  A sampled leaf
+// whose priority is not > 0 -- the reference asserts (buffer.py:74) -- is returned as the reference's descent finds it and
+// latched in *err (mapf_per_status).
 __device__ void sample_cta(const double *tree, int64_t capacity, int layer, const double *__restrict__ uniforms,
                            int64_t batch, int64_t *__restrict__ idx_out, double *__restrict__ prio_out,
-                           float *__restrict__ weight_out, double beta, unsigned char *smem, const bool top_ready)
+                           float *__restrict__ weight_out, double beta, unsigned char *smem, const bool top_ready, int32_t *err)
 {
     __shared__ double s_min[32];
     double *s_top = reinterpret_cast<double *>(smem);
@@ -387,6 +389,7 @@ __device__ void sample_cta(const double *tree, int64_t capacity, int layer, cons
         if (i == (int64_t)threadIdx.x) pr_first = pr;
         prio_out[i] = pr;                     // :72
         idx_out[i] = node - (capacity - 1);   // :73
+        if (!(pr > 0.0)) atomicOr(err, MAPF_ERRBIT_PRIORITY);  // :74 asserts priorities > 0; the batch's weights are then undefined
         local_min = fmin(local_min, pr);
     }
     PER_STAMP(46);
@@ -405,10 +408,10 @@ __device__ void sample_cta(const double *tree, int64_t capacity, int layer, cons
 __global__ void __launch_bounds__(kPerThreads)
 per_sample_kernel(const double *__restrict__ tree, int64_t capacity, int layer, const double *__restrict__ uniforms,
                   int64_t batch, int64_t *__restrict__ idx_out, double *__restrict__ prio_out,
-                  float *__restrict__ weight_out, double beta)
+                  float *__restrict__ weight_out, double beta, int32_t *err)
 {
     extern __shared__ __align__(16) unsigned char per_smem[];
-    sample_cta(tree, capacity, layer, uniforms, batch, idx_out, prio_out, weight_out, beta, per_smem, false);
+    sample_cta(tree, capacity, layer, uniforms, batch, idx_out, prio_out, weight_out, beta, per_smem, false, err);
 }
 
 // Learner TD error -> priority -> stale mask (worker.py:300-308, 192-201), one thread per transition
@@ -487,7 +490,7 @@ per_cycle_kernel(double *tree, unsigned long long *stamps, unsigned long long ep
     }
     if (a.n_sample > 0)
         sample_cta(tree, capacity, layer, a.d_uniforms, a.n_sample, a.d_sample_idx_out, a.d_sample_prio_out, a.d_sample_weight_out,
-                   a.beta, per_smem, top_ready);
+                   a.beta, per_smem, top_ready, err);
 }
 
 // LocalBuffer.finish, buffer.py:170-177: |sum_j gamma^j r[t+j] + max_a q[t,a] - q[t,a_t]| over j < forward_steps (rewards past
@@ -564,7 +567,7 @@ int mapf_launch_per_sample(mapf_per *t, const double *d_uniforms, int64_t batch,
     const size_t smem = per_sample_smem(t->layer);
     MAPF_CUDA(per_smem_optin((const void *)per_sample_kernel, smem));
     per_sample_kernel<<<1, kPerThreads, smem, st>>>(t->tree, t->capacity, t->layer, d_uniforms, batch, d_idx_out, d_prio_out,
-                                                    d_weight_out, beta);
+                                                    d_weight_out, beta, t->scratch.err);
     MAPF_CUDA(cudaGetLastError());
     return MAPF_OK;
 }

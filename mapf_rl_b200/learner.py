@@ -117,6 +117,9 @@ class BatchedLearner:
         if self.counter % self.target_update_freq == 0:                                                      # :336-337
             self.tar_model.load_state_dict(self.model.state_dict())
         if want_stats:
+            # synchronising anyway: surface a latched tree condition (a sampled leaf of priority 0 would make the next
+            # batch's importance weights NaN or 0, and the loss takes them as they are)
+            st.priority_tree.check()
             self.loss = float(loss.item())
             return dict(loss=self.loss, td_abs_mean=float(out["td"].abs().mean().item()),
                         prio_min=float(out["prio"].min().item()), kernel_td_vs_torch=float((out["td"] - td.detach().reshape(-1)).abs().max().item()))
