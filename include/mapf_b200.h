@@ -56,7 +56,8 @@ extern "C" {
 #define MAPF_RCODE_STAY_OFF_GOAL 2
 #define MAPF_RCODE_COLLISION 3
 #define MAPF_RCODE_FINISH 4
-#define MAPF_RCODE_RESET 5 /* reward 0: the step re-generated the environment (mapf_env_set_autoreset) */
+#define MAPF_RCODE_RESET 5 /* reward 0: the step re-generated the environment (mapf_env_set_autoreset); on a sized
+                              handle (mapf_env_enable_sizes) also the code of every absent agent slot a >= n_e */
 #define MAPF_RCODE_STAY_ON MAPF_RCODE_STAY_ON_GOAL
 #define MAPF_RCODE_STAY_OFF MAPF_RCODE_STAY_OFF_GOAL
 
@@ -272,6 +273,35 @@ int mapf_env_status(mapf_env *env, void *stream);
  * multi-GPU job draw the instances a single GPU would.  Distributional parity only (SURVEY 8c). */
 int mapf_env_reset(mapf_env *env, const uint8_t *d_mask, uint64_t seed, uint64_t env_offset, float density,
                    void *stream);
+
+/* ---- per-environment agent count and map side (the reference's curriculum, worker.py:424-425) ---- */
+/* A SIZED handle keeps, next to the maxima (N, L) it was created with, a setting (n_e, l_e), 1 <= n_e <= N,
+ * 2 <= l_e <= L, per slot e.  Agents a < n_e on cells inside l_e x l_e get exactly what a handle created with (n_e, l_e)
+ * gives for the same instance and actions.  Agents a >= n_e are absent: their actions are never read, they hold no cell
+ * and take no part in conflicts, `done`, the 'unique' check or the comm mask (rows and columns 0); every step and observe
+ * writes their 486 observation bytes as zeros, their reward as 0 with code MAPF_RCODE_RESET; positions and goals read 255,
+ * distances MAPF_DIST_UNREACHABLE, heuristic bits 0.  Cells outside l_e are off the map: a move there is a collision, the
+ * observation shows 0 on every channel, the map reads 0 and the BFS does not enter them.
+ * mapf_env_load / mapf_env_reset on a sized handle give the loaded / reset slots (N, L).  A sized handle does not serve
+ * mapf_env_rollout, mapf_env_rollout_ex, mapf_env_set_autoreset, mapf_env_step_host or mapf_env_step_host_codes
+ * (MAPF_EINVAL). */
+
+/* Opts the handle in (allocates u8 n[B], l[B], initialised to (N, L)).  A handle that never calls it runs the uniform
+ * kernels.  MAPF_EINVAL once the handle has used episode handling or the host-buffer steps. */
+int mapf_env_enable_sizes(mapf_env *env);
+/* mapf_env_load with a setting per instance: d_num_agents u8[n], d_map_length u8[n].  Map cells outside l_e and agent
+ * rows >= n_e of d_maps u8[n, L, L] / d_agents, d_goals u8[n, N, 2] are ignored.  A setting outside the maxima returns
+ * MAPF_EINVAL before any launch; a coordinate >= l_e latches MAPF_ESTATE. */
+int mapf_env_load_sized(mapf_env *env, const int32_t *d_env_ids, int32_t n, const uint8_t *d_maps, const uint8_t *d_agents,
+                        const uint8_t *d_goals, const uint8_t *d_num_agents, const uint8_t *d_map_length, void *stream);
+/* mapf_env_reset drawing each reset slot's setting uniformly from d_levels u8[K, 2] = (n, l) pairs: index (w * K) >> 32,
+ * w = one Philox word of the slot's own stream (seed, env_offset + e) under a purpose of its own.  The slot's instance is
+ * then the one a uniform (n, l) handle's mapf_env_reset draws for that stream, whatever the sharding.  K < 1 or a level
+ * outside the maxima returns MAPF_EINVAL before any launch. */
+int mapf_env_reset_levels(mapf_env *env, const uint8_t *d_mask, uint64_t seed, uint64_t env_offset, float density,
+                          const uint8_t *d_levels, int32_t num_levels, void *stream);
+/* The slots' settings: d_num_agents_out u8[B], d_map_length_out u8[B] (either may be NULL). */
+int mapf_env_get_sizes(mapf_env *env, uint8_t *d_num_agents_out, uint8_t *d_map_length_out, void *stream);
 
 /* ---- buffer.SumTree (buffer.py:16-105) ------------------------------------------------------ */
 /* capacity must be a power of two (buffer.py:23).  Tree nodes are fp64 like the reference. */

@@ -12,7 +12,8 @@ _lib = None
 MAPF_OK, MAPF_EINVAL, MAPF_ECUDA, MAPF_EACTION, MAPF_EUNIQUE, MAPF_ENOMEM, MAPF_ENOSPACE = 0, -1, -2, -3, -4, -5, -6
 MAPF_ESTATE, MAPF_EINTERNAL, MAPF_EINDEX, MAPF_EPRIORITY = -7, -8, -9, -10
 ABI_VERSION = 2
-# reward codes (MAPF_RCODE_*): index into reward_fn in config.REWARD_ORDER; 5 = reset step (reward 0)
+# reward codes (MAPF_RCODE_*): index into reward_fn in config.REWARD_ORDER; 5 = reset step (reward 0), and on a sized
+# handle an absent agent slot
 RCODE_RESET = 5
 
 
@@ -82,6 +83,10 @@ SIGNATURES = {
     "mapf_env_set_state": (C.c_int, [_vp, _vp, _vp, _vp]),
     "mapf_env_status": (C.c_int, [_vp, _vp]),
     "mapf_env_reset": (C.c_int, [_vp, _vp, _u64, _u64, _f32, _vp]),
+    "mapf_env_enable_sizes": (C.c_int, [_vp]),
+    "mapf_env_load_sized": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "mapf_env_reset_levels": (C.c_int, [_vp, _vp, _u64, _u64, _f32, _vp, _i32, _vp]),
+    "mapf_env_get_sizes": (C.c_int, [_vp, _vp, _vp, _vp]),
     "mapf_per_create": (C.c_int, [_i64, _i32, C.POINTER(_vp)]),
     "mapf_per_destroy": (C.c_int, [_vp]),
     "mapf_per_tree_ptr": (_vp, [_vp]),

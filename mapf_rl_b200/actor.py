@@ -12,6 +12,9 @@ Per step, as in the reference:
         initial priorities |TD| of LocalBuffer.finish      buffer.py:170-177 (actor_td kernel)
         GlobalBuffer.add: leaves = td ** alpha             worker.py:87-94   (sum-tree update kernel)
         env.reset                                          worker.py:422-428 (device generator + BFS)
+With a `Curriculum` (sized environment batch), every reset draws each slot's (num_agents, map_length) from the
+curriculum's current levels (worker.py:424-425) and finished episodes of the counted environments record their setting
+and done flag in it (worker.py:73-82).  Absent agents' rows of the store are zeros.
 Every environment owns one episode slot of the store while its episode runs; a finished episode is published
 (priorities inserted, size / done recorded) and the environment takes the next free slot of the ring, whose
 old leaves are zeroed first so a half-overwritten episode is never sampled.  The only host synchronisation
@@ -38,8 +41,17 @@ class BatchedActor:
     def __init__(self, env: BatchedEnvironment, net, store: ReplayStore, epsilon=0.1, seed: int = 0,
                  density: Optional[float] = None, max_steps: int = config.max_steps,
                  on_step: Optional[Callable] = None, on_episode: Optional[Callable] = None,
-                 on_begin: Optional[Callable] = None):
+                 on_begin: Optional[Callable] = None, curriculum=None, curriculum_envs=None):
+        """curriculum: a `Curriculum` whose levels the resets draw from (needs `BatchedEnvironment(..., sized=True)`);
+        curriculum_envs: the environments whose finished episodes it counts (default: all; the reference counts its
+        low-epsilon actors, ids 10-15, only)."""
         torch = _torch()
+        assert curriculum is None or env.sized, "a curriculum needs a sized environment batch"
+        self.curriculum = curriculum
+        self._counted = np.ones(env.num_envs, dtype=bool)
+        if curriculum_envs is not None:
+            self._counted[:] = False
+            self._counted[np.asarray(curriculum_envs, dtype=np.int64)] = True
         assert store.max_num_agents == env.num_agents, "the store is laid out for the batch's agent count"
         assert store.capacity >= 2 * env.num_envs, "capacity >= 2 * num_envs (a power of two): every env owns a slot while it runs"
         assert max_steps <= store.max_steps
@@ -97,7 +109,8 @@ class BatchedActor:
         mask[idt] = 1
         self.resets += 1
         # fresh instances: slot e of reset number r draws global stream (seed, r * B + e)
-        self.env.reset(mask=None if first else mask, seed=self.seed, env_offset=self.resets * self.B, density=self.density)
+        self.env.reset(mask=None if first else mask, seed=self.seed, env_offset=self.resets * self.B, density=self.density,
+                       levels=self.curriculum.levels if self.curriculum is not None else None)
         # a generator that could not place its agents latches MAPF_ERRBIT_RESET and leaves the slot as it was: surface it
         # here instead of stepping stale positions on a new map (one 4-byte status read per batch of episode ends; the
         # Q-network forward between two steps is three orders of magnitude longer)
@@ -186,6 +199,11 @@ class BatchedActor:
         st.size += int(size_h.sum())
         st.counter += int(size_h.sum())
         self.episodes += len(ids)
+        if self.curriculum is not None:
+            counted = ids[self._counted[ids]]
+            if counted.size:
+                n_e, l_e = (x.cpu().numpy() for x in self.env.sizes)
+                self.curriculum.record(n_e[counted], l_e[counted], self.env._done[torch.as_tensor(counted, device=self.dev)].cpu().numpy() != 0)
         if self.on_episode is not None:
             self.on_episode(self, ids, self._slot_host[ids].copy(), size_h, done.cpu().numpy(), td)
 

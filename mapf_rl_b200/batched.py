@@ -24,7 +24,12 @@ class BatchedEnvironment:
     OBS_SHAPE = config.obs_shape  # (6, 9, 9)
 
     def __init__(self, num_envs: int, num_agents: int = config.num_agents, map_length: int = config.map_length,
-                 device=None, obs_radius: int = config.obs_radius, reward_fn: dict = config.reward_fn):
+                 device=None, obs_radius: int = config.obs_radius, reward_fn: dict = config.reward_fn, sized: bool = False):
+        """sized=True: every environment carries its own agent count n_e <= num_agents and map side l_e <= map_length
+        (the reference's curriculum trains on a mix of settings, worker.py:424-425).  Agents a >= n_e are absent: their
+        actions are ignored, their observation rows are zeros, their reward 0 (code 5), positions 255; cells outside l_e are
+        off the map.  Agents a < n_e see exactly what a (n_e, l_e) handle gives.  `rollout`, `set_autoreset` and the
+        host-buffer steps are not available on a sized handle."""
         torch = _torch()
         if not torch.cuda.is_available():
             raise RuntimeError("mapf_rl_b200 needs a CUDA device: the environment kernels have no CPU fallback")
@@ -41,6 +46,9 @@ class BatchedEnvironment:
         h = C.c_void_p()
         _native.check(self._lib.mapf_env_create(C.byref(cfg), C.byref(h)))
         self._h = h
+        self.sized = bool(sized)
+        if self.sized:
+            _native.check(self._lib.mapf_env_enable_sizes(h))
         B, N = self.num_envs, self.num_agents
         self._rewards = torch.empty((B, N), dtype=torch.float32, device=self.device)
         self._done = torch.empty((B,), dtype=torch.uint8, device=self.device)
@@ -89,33 +97,79 @@ class BatchedEnvironment:
         return int(self._lib.mapf_env_arena_bytes(self._h))
 
     # -- Environment.load (environment.py:198-215) ----------------------------------------------
-    def load(self, maps, agents_pos, goals_pos, env_ids=None):
+    def load(self, maps, agents_pos, goals_pos, env_ids=None, num_agents=None, map_length=None):
         """maps [n,L,L] (0 free / non-zero obstacle, any dtype), agents_pos / goals_pos [n,N,2].
-        env_ids: which slots to load (default 0..n-1).  Recomputes the heuristic maps of those slots."""
+        env_ids: which slots to load (default 0..n-1).  Recomputes the heuristic maps of those slots.
+        Sized handle: num_agents / map_length [n] give each instance's setting (default N / L); map cells outside
+        l_e x l_e and agent rows >= n_e are ignored, and a coordinate of a present agent >= l_e raises IndexError."""
         torch = _torch()
         L, N = self.map_length, self.num_agents
         n = int(maps.shape[0])
         m = self._dev_u8(maps, (n, L, L), as_mask=True)
-        a = self._coords_u8(agents_pos, (n, N, 2))
-        g = self._coords_u8(goals_pos, (n, N, 2))
+        if num_agents is not None or map_length is not None:
+            assert self.sized, "per-environment sizes need a sized handle (BatchedEnvironment(..., sized=True))"
+            ns = np.broadcast_to(np.asarray(N if num_agents is None else num_agents, dtype=np.int64), (n,))
+            ls = np.broadcast_to(np.asarray(L if map_length is None else map_length, dtype=np.int64), (n,))
+            if n and (ns.min() < 1 or ns.max() > N or ls.min() < 2 or ls.max() > L):
+                raise ValueError(f"sizes outside 1 <= num_agents <= {N}, 2 <= map_length <= {L}")
+            a = self._coords_sized(agents_pos, ns, ls)
+            g = self._coords_sized(goals_pos, ns, ls)
+        else:
+            a = self._coords_u8(agents_pos, (n, N, 2))
+            g = self._coords_u8(goals_pos, (n, N, 2))
         ids_ptr = None
         if env_ids is not None:
             ids = torch.as_tensor(env_ids, dtype=torch.int32).to(self.device).contiguous()
             assert ids.numel() == n
             ids_ptr = C.c_void_p(ids.data_ptr())
-        _native.check(self._lib.mapf_env_load(self._h, ids_ptr, n, C.c_void_p(m.data_ptr()), C.c_void_p(a.data_ptr()),
-                                              C.c_void_p(g.data_ptr()), self._stream()))
+        if num_agents is not None or map_length is not None:
+            nd = torch.as_tensor(np.ascontiguousarray(ns, dtype=np.uint8)).to(self.device)
+            ld = torch.as_tensor(np.ascontiguousarray(ls, dtype=np.uint8)).to(self.device)
+            _native.check(self._lib.mapf_env_load_sized(self._h, ids_ptr, n, C.c_void_p(m.data_ptr()), C.c_void_p(a.data_ptr()),
+                                                        C.c_void_p(g.data_ptr()), C.c_void_p(nd.data_ptr()),
+                                                        C.c_void_p(ld.data_ptr()), self._stream()))
+        else:
+            _native.check(self._lib.mapf_env_load(self._h, ids_ptr, n, C.c_void_p(m.data_ptr()), C.c_void_p(a.data_ptr()),
+                                                  C.c_void_p(g.data_ptr()), self._stream()))
         # synchronous (keeps the inputs alive until the stream has consumed them); raises IndexError if the device-side
         # validation found a coordinate outside the map / a slot id outside the batch, RuntimeError('unique') for two
         # agents on one cell (environment.py:424-428 raises that at the next step)
         self.check()
 
+    def _coords_sized(self, x, ns, ls):
+        """[n,N,2] coordinates of a sized load -> uint8 tensor on this device; rows a >= n_e are ignored (sent as 0), a
+        present agent's coordinate outside [0, l_e) raises IndexError."""
+        torch = _torch()
+        n, N = len(ns), self.num_agents
+        t = np.asarray(x.cpu() if isinstance(x, torch.Tensor) else x)
+        assert t.shape == (n, N, 2), f"expected shape {(n, N, 2)}, got {t.shape}"
+        present = np.arange(N)[None, :] < ns[:, None]
+        t = np.where(present[..., None], t.astype(np.int64), 0)
+        bad = present & ((t < 0) | (t >= ls[:, None, None])).any(-1)
+        if bad.any():
+            i, a = np.argwhere(bad)[0]
+            raise IndexError(f"coordinate {tuple(t[i, a])} of agent {a} outside the {ls[i]}x{ls[i]} map of instance {i}")
+        return torch.as_tensor(t.astype(np.uint8)).to(self.device).contiguous()
+
+    @property
+    def sizes(self):
+        """(num_agents uint8[B], map_length uint8[B]) CUDA tensors: each environment's setting (sized handle)."""
+        torch = _torch()
+        assert self.sized, "sizes of a handle created without sized=True"
+        n = torch.empty((self.num_envs,), dtype=torch.uint8, device=self.device)
+        l = torch.empty((self.num_envs,), dtype=torch.uint8, device=self.device)
+        _native.check(self._lib.mapf_env_get_sizes(self._h, C.c_void_p(n.data_ptr()), C.c_void_p(l.data_ptr()), self._stream()))
+        return n, l
+
     # -- Environment.reset generator, device side (environment.py:146-196) ----------------------
-    def reset(self, mask=None, seed: int = 0, env_offset: Optional[int] = None, density: Optional[float] = None):
+    def reset(self, mask=None, seed: int = 0, env_offset: Optional[int] = None, density: Optional[float] = None, levels=None):
         """Draw new random instances on the device for slots with mask != 0 (default: all).  Slot e draws Philox stream
         (seed, env_offset + e).  Without an explicit `env_offset` the handle counts its resets and uses
         resets * num_envs, so repeated `reset(mask)` calls at episode ends never hand a slot the instance it (or another
-        slot) had before; pass `env_offset` to pin the instances (sharding, reproducing a run)."""
+        slot) had before; pass `env_offset` to pin the instances (sharding, reproducing a run).
+        levels (sized handle): a sequence of (num_agents, map_length) settings; each reset slot draws one uniformly from its
+        own stream and generates the instance a uniform handle of that setting draws for the stream.  Without `levels`
+        a sized handle resets its slots to (N, L)."""
         if env_offset is None:
             env_offset = self._resets * self.num_envs
         self._resets += 1
@@ -124,6 +178,16 @@ class BatchedEnvironment:
             mk = self._dev_u8(mask, (self.num_envs,))
             mptr = C.c_void_p(mk.data_ptr())
         dens = -1.0 if density is None else float(density)
+        if levels is not None:
+            assert self.sized, "levels need a sized handle (BatchedEnvironment(..., sized=True))"
+            lv = np.asarray(levels, dtype=np.int64).reshape(-1, 2)
+            if lv.size == 0 or lv.min() < 0 or lv.max() > 255:
+                raise ValueError(f"levels must be a non-empty list of (num_agents, map_length) pairs, got {levels!r}")
+            ld = _torch().as_tensor(np.ascontiguousarray(lv, dtype=np.uint8)).to(self.device)
+            _native.check(self._lib.mapf_env_reset_levels(self._h, mptr, C.c_uint64(seed), C.c_uint64(env_offset),
+                                                          C.c_float(dens), C.c_void_p(ld.data_ptr()), int(lv.shape[0]),
+                                                          self._stream()))
+            return
         _native.check(self._lib.mapf_env_reset(self._h, mptr, C.c_uint64(seed), C.c_uint64(env_offset),
                                                C.c_float(dens), self._stream()))
 
@@ -399,7 +463,10 @@ class BatchedEnvironment:
     def set_state(self, agents_pos=None, steps=None):
         torch = _torch()
         p = s = None
-        if agents_pos is not None:
+        if agents_pos is not None and self.sized:   # rows of absent agents are ignored (they read back as 255)
+            ns, ls = (x.cpu().numpy().astype(np.int64) for x in self.sizes)
+            p = self._coords_sized(agents_pos, ns, ls)
+        elif agents_pos is not None:
             p = self._coords_u8(agents_pos, (self.num_envs, self.num_agents, 2))
         if steps is not None:
             s = torch.as_tensor(steps, dtype=torch.int32).to(self.device).contiguous()

@@ -10,6 +10,9 @@
 
 // launchers (other translation units)
 int mapf_launch_pack_load(mapf_env *, const int32_t *, int, const uint8_t *, const uint8_t *, const uint8_t *, cudaStream_t);
+int mapf_launch_pack_load_sized(mapf_env *, const int32_t *, int, const uint8_t *, const uint8_t *, const uint8_t *, const uint8_t *,
+                                const uint8_t *, cudaStream_t);
+int mapf_launch_reset_levels(mapf_env *, const uint8_t *, uint64_t, uint64_t, float, const uint8_t *, int, cudaStream_t);
 int mapf_launch_validate_state(mapf_env *, const int32_t *, int, cudaStream_t);
 int mapf_launch_bfs(mapf_env *, const int32_t *, int, int32_t *, cudaStream_t);
 int mapf_launch_step(mapf_env *, const uint8_t *, uint8_t *, const int64_t *, const StepOut &, cudaStream_t);
@@ -259,6 +262,9 @@ int mapf_env_destroy(mapf_env *env)
     if (env->pg_join) cudaEventDestroy(env->pg_join);
     cudaFree(env->steps);
     cudaFree(env->err);
+    cudaFree(env->sz_n);
+    cudaFree(env->sz_l);
+    cudaFree(env->sz_full);
     cudaFree(env->ro_work);
     cudaFree(env->ro_progress);
     cudaFree(env->ro_episode);
@@ -330,6 +336,34 @@ static int hp_drain(mapf_env *env, cudaStream_t st)
         if (_rc != MAPF_OK) return _rc;             \
     } while (0)
 
+// entry points a sized handle (mapf_env_enable_sizes) does not serve
+#define MAPF_REFUSE_SIZED(env, what)                                                              \
+    if ((env)->sz_n) {                                                                            \
+        mapf_set_error(what ": not available on a sized handle (per-environment agent count and map side)"); \
+        return MAPF_EINVAL;                                                                       \
+    }
+
+// (n, l) pairs of a sized handle's levels / sizes, read to the host: 1 <= n <= N, 2 <= l <= L, n <= l * l
+static int check_sizes(const mapf_env *env, const uint8_t *d_n, const uint8_t *d_l, size_t stride, int count, cudaStream_t st,
+                       const char *what)
+{
+    const size_t bytes = (size_t)(count - 1) * stride + 1;  // element i at i * stride
+    std::string h(2 * bytes, '\0');
+    uint8_t *hn = reinterpret_cast<uint8_t *>(&h[0]), *hl = hn + bytes;
+    MAPF_CUDA(cudaMemcpyAsync(hn, d_n, bytes, cudaMemcpyDeviceToHost, st));
+    MAPF_CUDA(cudaMemcpyAsync(hl, d_l, bytes, cudaMemcpyDeviceToHost, st));
+    MAPF_CUDA(cudaStreamSynchronize(st));
+    for (int i = 0; i < count; ++i) {
+        const int n = hn[(size_t)i * stride], l = hl[(size_t)i * stride];
+        if (n < 1 || n > env->d.N || l < 2 || l > env->d.L || n > l * l) {
+            mapf_set_error(std::string(what) + ": agent count " + std::to_string(n) + " / map side " + std::to_string(l) +
+                           " outside 1 <= n <= " + std::to_string(env->d.N) + ", 2 <= l <= " + std::to_string(env->d.L) + ", n <= l * l");
+            return MAPF_EINVAL;
+        }
+    }
+    return MAPF_OK;
+}
+
 int mapf_env_load(mapf_env *env, const int32_t *d_env_ids, int32_t n, const uint8_t *d_maps, const uint8_t *d_agents,
                   const uint8_t *d_goals, void *stream)
 {
@@ -341,11 +375,100 @@ int mapf_env_load(mapf_env *env, const int32_t *d_env_ids, int32_t n, const uint
     }
     if (n == 0) return MAPF_OK;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    int rc = mapf_launch_pack_load(env, d_env_ids, n, d_maps, d_agents, d_goals, st);
+    // a sized handle records (N, L) for the loaded slots
+    int rc = env->sz_n ? mapf_launch_pack_load_sized(env, d_env_ids, n, d_maps, d_agents, d_goals, nullptr, nullptr, st)
+                       : mapf_launch_pack_load(env, d_env_ids, n, d_maps, d_agents, d_goals, st);
     if (rc != MAPF_OK) return rc;
     rc = mapf_launch_validate_state(env, d_env_ids, n, st);  // coordinates inside the map, one agent per cell
     if (rc != MAPF_OK) return rc;
     return mapf_launch_bfs(env, d_env_ids, n, nullptr, st);
+}
+
+int mapf_env_enable_sizes(mapf_env *env)
+{
+    REQUIRE_ENV(env);
+    if (env->sz_n) return MAPF_OK;
+    if (env->ar_max_steps > 0 || env->hp_stream || env->d_actions) {
+        mapf_set_error("mapf_env_enable_sizes: the handle already uses episode handling or the host-buffer steps");
+        return MAPF_EINVAL;
+    }
+    const EnvDims &d = env->d;
+    int64_t total = env->arena_bytes;
+    int rc = dev_alloc(&env->sz_n, (size_t)d.B, &total);
+    if (rc == MAPF_OK) rc = dev_alloc(&env->sz_l, (size_t)d.B, &total);
+    if (rc == MAPF_OK) rc = dev_alloc(&env->sz_full, 2, &total);
+    if (rc == MAPF_OK) {
+        const uint8_t full[2] = {(uint8_t)d.N, (uint8_t)d.L};
+        cudaError_t e = cudaMemset(env->sz_n, d.N, (size_t)d.B);
+        if (e == cudaSuccess) e = cudaMemset(env->sz_l, d.L, (size_t)d.B);
+        if (e == cudaSuccess) e = cudaMemcpy(env->sz_full, full, 2, cudaMemcpyHostToDevice);
+        if (e == cudaSuccess) e = cudaDeviceSynchronize();
+        if (e != cudaSuccess) rc = mapf_cuda_fail(e, "mapf_env_enable_sizes");
+    }
+    if (rc != MAPF_OK) {
+        cudaFree(env->sz_n), cudaFree(env->sz_l), cudaFree(env->sz_full);
+        env->sz_n = env->sz_l = env->sz_full = nullptr;
+        return rc;
+    }
+    env->arena_bytes = total;
+    return MAPF_OK;
+}
+
+int mapf_env_load_sized(mapf_env *env, const int32_t *d_env_ids, int32_t n, const uint8_t *d_maps, const uint8_t *d_agents,
+                        const uint8_t *d_goals, const uint8_t *d_num_agents, const uint8_t *d_map_length, void *stream)
+{
+    REQUIRE_ENV(env);
+    MAPF_DRAIN(env, static_cast<cudaStream_t>(stream));
+    if (!env->sz_n) {
+        mapf_set_error("mapf_env_load_sized: the handle is not sized (mapf_env_enable_sizes)");
+        return MAPF_EINVAL;
+    }
+    if (n < 0 || n > env->d.B || !d_maps || !d_agents || !d_goals || !d_num_agents || !d_map_length) {
+        mapf_set_error("mapf_env_load_sized: bad arguments");
+        return MAPF_EINVAL;
+    }
+    if (n == 0) return MAPF_OK;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    int rc = check_sizes(env, d_num_agents, d_map_length, 1, n, st, "mapf_env_load_sized");
+    if (rc != MAPF_OK) return rc;
+    rc = mapf_launch_pack_load_sized(env, d_env_ids, n, d_maps, d_agents, d_goals, d_num_agents, d_map_length, st);
+    if (rc != MAPF_OK) return rc;
+    rc = mapf_launch_validate_state(env, d_env_ids, n, st);  // coordinates inside the slot's map, one agent per cell
+    if (rc != MAPF_OK) return rc;
+    return mapf_launch_bfs(env, d_env_ids, n, nullptr, st);
+}
+
+int mapf_env_reset_levels(mapf_env *env, const uint8_t *d_mask, uint64_t seed, uint64_t env_offset, float density,
+                          const uint8_t *d_levels, int32_t num_levels, void *stream)
+{
+    REQUIRE_ENV(env);
+    MAPF_DRAIN(env, static_cast<cudaStream_t>(stream));
+    if (!env->sz_n) {
+        mapf_set_error("mapf_env_reset_levels: the handle is not sized (mapf_env_enable_sizes)");
+        return MAPF_EINVAL;
+    }
+    if (density >= 1.0f || !d_levels || num_levels < 1) {
+        mapf_set_error("mapf_env_reset_levels: density < 1 and at least one level required");
+        return MAPF_EINVAL;
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int rc = check_sizes(env, d_levels, d_levels + 1, 2, num_levels, st, "mapf_env_reset_levels");
+    if (rc != MAPF_OK) return rc;
+    return mapf_launch_reset_levels(env, d_mask, seed, env_offset, density, d_levels, num_levels, st);
+}
+
+int mapf_env_get_sizes(mapf_env *env, uint8_t *d_num_agents_out, uint8_t *d_map_length_out, void *stream)
+{
+    REQUIRE_ENV(env);
+    MAPF_DRAIN(env, static_cast<cudaStream_t>(stream));
+    if (!env->sz_n) {
+        mapf_set_error("mapf_env_get_sizes: the handle is not sized (mapf_env_enable_sizes)");
+        return MAPF_EINVAL;
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (d_num_agents_out) MAPF_CUDA(cudaMemcpyAsync(d_num_agents_out, env->sz_n, (size_t)env->d.B, cudaMemcpyDeviceToDevice, st));
+    if (d_map_length_out) MAPF_CUDA(cudaMemcpyAsync(d_map_length_out, env->sz_l, (size_t)env->d.B, cudaMemcpyDeviceToDevice, st));
+    return MAPF_OK;
 }
 
 int mapf_env_bfs_navi(mapf_env *env, const int32_t *d_env_ids, int32_t n, int32_t *d_dist_out, void *stream)
@@ -482,6 +605,7 @@ int mapf_env_rollout_plan(mapf_env *env, int32_t T, int32_t action_slots, int32_
 int mapf_env_rollout_ex(mapf_env *env, const mapf_rollout_io *io, void *stream)
 {
     REQUIRE_ENV(env);
+    MAPF_REFUSE_SIZED(env, "mapf_env_rollout");
     MAPF_DRAIN(env, static_cast<cudaStream_t>(stream));
     if (!io || !io->d_actions || !io->d_obs || !io->d_done) {
         mapf_set_error("mapf_env_rollout: NULL buffer");
@@ -626,6 +750,7 @@ int mapf_env_set_autoreset(mapf_env *env, int32_t max_steps, uint64_t seed, uint
                            void *stream)
 {
     REQUIRE_ENV(env);
+    MAPF_REFUSE_SIZED(env, "mapf_env_set_autoreset");
     MAPF_DRAIN(env, static_cast<cudaStream_t>(stream));
     if (max_steps < 0 || density >= 1.0f) {
         mapf_set_error("mapf_env_set_autoreset: max_steps >= 0 and density < 1 required");
@@ -689,6 +814,7 @@ int mapf_env_step_host(mapf_env *env, const uint8_t *h_actions, uint8_t *h_obs, 
                        int32_t *h_steps, uint8_t *d_obs_opt, void *stream)
 {
     REQUIRE_ENV(env);
+    MAPF_REFUSE_SIZED(env, "mapf_env_step_host");
     MAPF_DRAIN(env, static_cast<cudaStream_t>(stream));
     if (!h_actions || !h_rewards || !h_done) {
         mapf_set_error("mapf_env_step_host: NULL buffer");
@@ -810,6 +936,7 @@ int mapf_env_step_host_codes(mapf_env *env, const uint8_t *h_actions, uint8_t *h
                              uint8_t *d_obs, void *stream)
 {
     REQUIRE_ENV(env);
+    MAPF_REFUSE_SIZED(env, "mapf_env_step_host_codes");
     if (!h_actions || !h_codes || !h_done || !d_obs) {
         mapf_set_error("mapf_env_step_host_codes: NULL buffer");
         return MAPF_EINVAL;
@@ -1044,6 +1171,8 @@ int mapf_env_reset(mapf_env *env, const uint8_t *d_mask, uint64_t seed, uint64_t
         mapf_set_error("mapf_env_reset: density must be < 1");
         return MAPF_EINVAL;
     }
+    if (env->sz_n)  // a sized handle draws at (N, L) and records it: the one-level form of mapf_env_reset_levels
+        return mapf_launch_reset_levels(env, d_mask, seed, env_offset, density, env->sz_full, 1, static_cast<cudaStream_t>(stream));
     return mapf_launch_reset(env, d_mask, seed, env_offset, density, static_cast<cudaStream_t>(stream));
 }
 

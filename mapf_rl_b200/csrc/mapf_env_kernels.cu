@@ -20,11 +20,15 @@ __device__ __forceinline__ int lane_id() { return threadIdx.x & 31; }
 
 // ---------------------------------------------------------------------------------------------
 // pack: u8 maps -> padded obstacle bitmaps; copy coordinates; steps = 0      (environment.py:198-215)
+// SIZED: instance i has in_n[i] agents on an in_l[i] map (NULL: N and L); map cells outside it and agent rows beyond it are
+// ignored -- the bitmap is zero there, the rows read 255 -- and the slot's sizes are recorded.
 // ---------------------------------------------------------------------------------------------
-__global__ void pack_load_kernel(EnvDims d, const int32_t *__restrict__ env_ids, int n, const uint8_t *__restrict__ maps,
-                                 const uint8_t *__restrict__ agents, const uint8_t *__restrict__ goals,
-                                 uint32_t *__restrict__ obst, uint8_t *__restrict__ pos, uint8_t *__restrict__ goal,
-                                 int32_t *__restrict__ steps, int32_t *__restrict__ err)
+template <bool SIZED>
+__device__ __forceinline__ void pack_load_body(const EnvDims &d, const int32_t *__restrict__ env_ids, int n, const uint8_t *__restrict__ maps,
+                                               const uint8_t *__restrict__ agents, const uint8_t *__restrict__ goals,
+                                               uint32_t *__restrict__ obst, uint8_t *__restrict__ pos, uint8_t *__restrict__ goal,
+                                               int32_t *__restrict__ steps, int32_t *__restrict__ err, const uint8_t *in_n = nullptr,
+                                               const uint8_t *in_l = nullptr, uint8_t *sz_n = nullptr, uint8_t *sz_l = nullptr)
 {
     int i = blockIdx.x;
     if (i >= n) return;
@@ -33,25 +37,47 @@ __global__ void pack_load_kernel(EnvDims d, const int32_t *__restrict__ env_ids,
         if (threadIdx.x == 0) atomicOr(err, MAPF_ERRBIT_STATE);
         return;
     }
+    const int NA = SIZED && in_n ? (int)in_n[i] : d.N, LM = SIZED && in_l ? (int)in_l[i] : d.L;
     const uint8_t *m = maps + (size_t)i * d.L * d.L;
     uint32_t *o = obst + (size_t)e * d.obst_stride;
     for (int w = threadIdx.x; w < d.obst_stride; w += blockDim.x) {
         int row = w / d.RWS, ww = w - row * d.RWS;
         uint32_t bits = 0;
         int x = row - 4;
-        if (row < d.R && ww < d.RW && x >= 0 && x < d.L) {
+        if (row < d.R && ww < d.RW && x >= 0 && x < LM) {
             for (int b = 0; b < 32; ++b) {
                 int y = ww * 32 + b - 4;
-                if (y >= 0 && y < d.L && m[x * d.L + y] != 0) bits |= 1u << b;
+                if (y >= 0 && y < LM && m[x * d.L + y] != 0) bits |= 1u << b;
             }
         }
         o[w] = bits;
     }
     for (int k = threadIdx.x; k < 2 * d.N; k += blockDim.x) {
-        pos[(size_t)e * 2 * d.N + k] = agents[(size_t)i * 2 * d.N + k];
-        goal[(size_t)e * 2 * d.N + k] = goals[(size_t)i * 2 * d.N + k];
+        const bool present = !SIZED || k < 2 * NA;
+        pos[(size_t)e * 2 * d.N + k] = present ? agents[(size_t)i * 2 * d.N + k] : (uint8_t)255;
+        goal[(size_t)e * 2 * d.N + k] = present ? goals[(size_t)i * 2 * d.N + k] : (uint8_t)255;
     }
-    if (threadIdx.x == 0) steps[e] = 0;
+    if (threadIdx.x == 0) {
+        steps[e] = 0;
+        if constexpr (SIZED) sz_n[e] = (uint8_t)NA, sz_l[e] = (uint8_t)LM;
+    }
+}
+
+__global__ void pack_load_kernel(EnvDims d, const int32_t *__restrict__ env_ids, int n, const uint8_t *__restrict__ maps,
+                                 const uint8_t *__restrict__ agents, const uint8_t *__restrict__ goals,
+                                 uint32_t *__restrict__ obst, uint8_t *__restrict__ pos, uint8_t *__restrict__ goal,
+                                 int32_t *__restrict__ steps, int32_t *__restrict__ err)
+{
+    pack_load_body<false>(d, env_ids, n, maps, agents, goals, obst, pos, goal, steps, err);
+}
+
+__global__ void pack_load_sized_kernel(EnvDims d, const int32_t *__restrict__ env_ids, int n, const uint8_t *__restrict__ maps,
+                                       const uint8_t *__restrict__ agents, const uint8_t *__restrict__ goals,
+                                       uint32_t *__restrict__ obst, uint8_t *__restrict__ pos, uint8_t *__restrict__ goal,
+                                       int32_t *__restrict__ steps, int32_t *__restrict__ err, const uint8_t *__restrict__ in_n,
+                                       const uint8_t *__restrict__ in_l, uint8_t *__restrict__ sz_n, uint8_t *__restrict__ sz_l)
+{
+    pack_load_body<true>(d, env_ids, n, maps, agents, goals, obst, pos, goal, steps, err, in_n, in_l, sz_n, sz_l);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -59,35 +85,42 @@ __global__ void pack_load_kernel(EnvDims d, const int32_t *__restrict__ env_ids,
 // outside the map must never reach it.  Out-of-range coordinates are clamped into the map and latched as
 // MAPF_ERRBIT_STATE (the reference raises IndexError on the same input); two agents on one cell are latched as
 // MAPF_ERRBIT_UNIQUE (the reference raises RuntimeError('unique') at the next step, environment.py:424-428).
-// One warp per environment.
+// One warp per environment.  SIZED: against the slot's own side, over its present agents; absent rows are set to 255.
 // ---------------------------------------------------------------------------------------------
-__global__ void validate_state_kernel(EnvDims d, const int32_t *__restrict__ env_ids, int n, uint8_t *__restrict__ pos,
-                                      uint8_t *__restrict__ goal, int32_t *__restrict__ err)
+template <bool SIZED>
+__device__ __forceinline__ void validate_state_body(const EnvDims &d, const int32_t *__restrict__ env_ids, int n, uint8_t *__restrict__ pos,
+                                                    uint8_t *__restrict__ goal, int32_t *__restrict__ err,
+                                                    const uint8_t *sz_n = nullptr, const uint8_t *sz_l = nullptr)
 {
     const int i = blockIdx.x * 4 + (threadIdx.x >> 5);
     if (i >= n) return;
     const int lane = threadIdx.x & 31;
     const int e = env_ids ? env_ids[i] : i;
     if (e < 0 || e >= d.B) return;  // latched by pack_load_kernel
+    const int NA = SIZED ? (int)sz_n[e] : d.N, LM = SIZED ? (int)sz_l[e] : d.L;
     uchar2 *pp = reinterpret_cast<uchar2 *>(pos) + (size_t)e * d.N;
     uchar2 *gg = reinterpret_cast<uchar2 *>(goal) + (size_t)e * d.N;
     bool bad = false;
     for (int a = lane; a < d.N; a += 32) {
+        if (SIZED && a >= NA) {
+            pp[a] = gg[a] = make_uchar2(255, 255);
+            continue;
+        }
         uchar2 p = pp[a], g = gg[a];
-        if (p.x >= d.L || p.y >= d.L) {
+        if (p.x >= LM || p.y >= LM) {
             bad = true;
-            p.x = min((int)p.x, d.L - 1), p.y = min((int)p.y, d.L - 1);
+            p.x = min((int)p.x, LM - 1), p.y = min((int)p.y, LM - 1);
             pp[a] = p;
         }
-        if (g.x >= d.L || g.y >= d.L) {
+        if (g.x >= LM || g.y >= LM) {
             bad = true;
-            g.x = min((int)g.x, d.L - 1), g.y = min((int)g.y, d.L - 1);
+            g.x = min((int)g.x, LM - 1), g.y = min((int)g.y, LM - 1);
             gg[a] = g;
         }
     }
     __syncwarp();
     bool dup = false;
-    for (int a = lane; a < d.N; a += 32) {
+    for (int a = lane; a < NA; a += 32) {
         const uchar2 p = pp[a];
         for (int b = 0; b < a; ++b) {
             const uchar2 q = pp[b];
@@ -97,6 +130,19 @@ __global__ void validate_state_kernel(EnvDims d, const int32_t *__restrict__ env
     bad = __any_sync(MAPF_FULL_MASK, bad);
     dup = __any_sync(MAPF_FULL_MASK, dup);
     if (lane == 0 && (bad || dup)) atomicOr(err, (bad ? MAPF_ERRBIT_STATE : 0) | (dup ? MAPF_ERRBIT_UNIQUE : 0));
+}
+
+__global__ void validate_state_kernel(EnvDims d, const int32_t *__restrict__ env_ids, int n, uint8_t *__restrict__ pos,
+                                      uint8_t *__restrict__ goal, int32_t *__restrict__ err)
+{
+    validate_state_body<false>(d, env_ids, n, pos, goal, err);
+}
+
+__global__ void validate_state_sized_kernel(EnvDims d, const int32_t *__restrict__ env_ids, int n, uint8_t *__restrict__ pos,
+                                            uint8_t *__restrict__ goal, int32_t *__restrict__ err, const uint8_t *__restrict__ sz_n,
+                                            const uint8_t *__restrict__ sz_l)
+{
+    validate_state_body<true>(d, env_ids, n, pos, goal, err, sz_n, sz_l);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -120,6 +166,37 @@ bfs_navi_kernel(EnvDims d, const int32_t *__restrict__ env_ids, const uint8_t *_
     // the slot's live buffer (mapf_common.cuh)
     uint32_t *nv = (navi_alt && navi_sel[e]) ? navi_alt : navi;
     bfs_navi_warp<RW, RPL, APW>(d, e, a, i, alive, obst, goal, nv, dist_out);
+}
+
+// The same on a sized handle: the free cells are clipped to the slot's side l_e, and only its n_e present agents search
+// (groups of absent agents own no rows and store nothing; a warp with none present leaves).  With dist_out every agent's
+// distances are written: an absent agent searches an empty map, so its rows read MAPF_DIST_UNREACHABLE.  The free rows are
+// kept in registers (KEEP): the side differs from group to group of a warp.
+template <int RW, int RPL, int APW>
+__global__ void __launch_bounds__(kBfsWarps * 32, RW * RPL <= 9 ? 8 : 1)
+bfs_navi_sized_kernel(EnvDims d, const int32_t *__restrict__ env_ids, const uint8_t *__restrict__ env_mask, int n,
+                      const uint32_t *__restrict__ obst, const uint8_t *__restrict__ goal, uint32_t *__restrict__ navi,
+                      int32_t *__restrict__ dist_out, const uint8_t *__restrict__ sz_n, const uint8_t *__restrict__ sz_l)
+{
+    constexpr int LW = 32 / APW;
+    const int g = (blockIdx.x * kBfsWarps + (threadIdx.x >> 5)) * APW + lane_id() / LW;
+    bool alive = g < n * d.N;
+    const int i = alive ? g / d.N : 0, a = alive ? g - i * d.N : 0;
+    int e = env_ids ? env_ids[i] : i;
+    if (e < 0 || e >= d.B) alive = false, e = 0;           // bad slot id: latched by pack_load_kernel
+    if (alive && env_mask && !env_mask[e]) alive = false;  // masked re-computation after a device-side reset
+    const bool present = a < (int)sz_n[e];
+    if (!dist_out && !present) alive = false;
+    if (!__any_sync(MAPF_FULL_MASK, alive)) return;
+    EnvDims df = d;  // the free cells: l_e x l_e, none for an absent agent
+    df.L = present ? (int)sz_l[e] : 0;
+    const uint32_t *ob = obst + (size_t)e * d.obst_stride;
+    const uchar2 gg = present ? __ldcg(reinterpret_cast<const uchar2 *>(goal) + (size_t)e * d.N + a) : make_uchar2(0, 0);
+    BfsFree<RW, RPL> F;
+    bfs_load_free<RW, RPL, APW>(df, ob, F);
+    if (dist_out) bfs_navi_search<RW, RPL, APW, false, true, true>(d, e, a, i, alive, ob, F, gg.x, gg.y, navi, dist_out);
+    else if (d.L < LW * RPL) bfs_navi_search<RW, RPL, APW, true, false, true>(d, e, a, i, alive, ob, F, gg.x, gg.y, navi, nullptr);
+    else bfs_navi_search<RW, RPL, APW, false, false, true>(d, e, a, i, alive, ob, F, gg.x, gg.y, navi, nullptr);
 }
 
 // The heuristic maps of the pre-generated NEXT instances of the listed slots (episode handling of mapf_env_rollout): reads
@@ -170,25 +247,33 @@ pregen_bfs_kernel(EnvDims d, const uint32_t *__restrict__ list, int min_count, u
 // ---------------------------------------------------------------------------------------------
 constexpr int kCommWarps = 4;
 
-__global__ void __launch_bounds__(kCommWarps * 32)
-comm_mask_kernel(EnvDims d, const uint8_t *__restrict__ pos, int k_nearest, uint8_t *__restrict__ out)
+// SIZED: only the n_e present agents take part; rows and columns of absent agents are 0
+template <bool SIZED>
+__device__ __forceinline__ void comm_mask_body(const EnvDims &d, const uint8_t *__restrict__ pos, int k_nearest, uint8_t *__restrict__ out,
+                                               const int tid, const uint8_t *sz_n = nullptr)
 {
     __shared__ uint16_t s_pos[kCommWarps][MAPF_MAX_AGENTS];
     __shared__ uint32_t s_bits[kCommWarps][MAPF_MAX_AGENTS][MAPF_MAX_AGENTS / 32];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int lane = tid & 31, warp = tid >> 5;  // (tid read by the kernel, within its launch bounds)
     const int e = blockIdx.x * kCommWarps + warp;
     if (e >= d.B) return;
     const int N = d.N;
+    const int NA = SIZED ? (int)sz_n[e] : N;
     for (int a = lane; a < N; a += 32) s_pos[warp][a] = reinterpret_cast<const uint16_t *>(pos)[(size_t)e * N + a];
     __syncwarp();
-    for (int i = lane; i < N; i += 32) {
+    if constexpr (SIZED) {
+        for (int i = NA + lane; i < N; i += 32)
+#pragma unroll
+            for (int w = 0; w < MAPF_MAX_AGENTS / 32; ++w) s_bits[warp][i][w] = 0;
+    }
+    for (int i = lane; i < NA; i += 32) {
         const int xi = s_pos[warp][i] & 0xff, yi = s_pos[warp][i] >> 8;
         // three smallest keys, ascending.  Only agents inside the field of view can end up in the mask, and those lie within
         // d^2 <= 2 r^2; an agent farther away can neither be one nor displace one from the three nearest: start at that bound
         // (the insertion below then runs for the few close agents only)
         constexpr uint32_t kFar = (uint32_t)(2 * MAPF_OBS_RADIUS * MAPF_OBS_RADIUS + 1) << 8;
         uint32_t b0 = kFar, b1 = kFar, b2 = kFar;
-        for (int j = 0; j < N; ++j) {
+        for (int j = 0; j < NA; ++j) {
             const int dx = xi - (s_pos[warp][j] & 0xff), dy = yi - (s_pos[warp][j] >> 8);
             uint32_t key = ((uint32_t)(dx * dx + dy * dy) << 8) | (uint32_t)j;
             if (key < b2) {
@@ -237,6 +322,19 @@ comm_mask_kernel(EnvDims d, const uint8_t *__restrict__ pos, int k_nearest, uint
     }
 }
 
+__global__ void __launch_bounds__(kCommWarps * 32)
+comm_mask_kernel(EnvDims d, const uint8_t *__restrict__ pos, int k_nearest, uint8_t *__restrict__ out)
+{
+    comm_mask_body<false>(d, pos, k_nearest, out, threadIdx.x);
+}
+
+__global__ void __launch_bounds__(kCommWarps * 32)
+comm_mask_sized_kernel(EnvDims d, const uint8_t *__restrict__ pos, int k_nearest, uint8_t *__restrict__ out,
+                       const uint8_t *__restrict__ sz_n)
+{
+    comm_mask_body<true>(d, pos, k_nearest, out, threadIdx.x, sz_n);
+}
+
 // ---------------------------------------------------------------------------------------------
 // attribute reads: unpack state for parity dumps / drop-in attributes
 // ---------------------------------------------------------------------------------------------
@@ -252,8 +350,11 @@ __global__ void unpack_map_kernel(EnvDims d, const uint32_t *__restrict__ obst, 
     map_out[idx] = (w >> ((y + 4) & 31)) & 1u;
 }
 
-__global__ void unpack_navi_kernel(EnvDims d, const uint32_t *__restrict__ navi, const uint32_t *__restrict__ navi_alt,
-                                   const uint8_t *__restrict__ navi_sel, uint8_t *__restrict__ navi_out)
+// SIZED: absent agents read 0 (their maps are not recomputed once a slot has fewer agents)
+template <bool SIZED>
+__device__ __forceinline__ void unpack_navi_body(const EnvDims &d, const uint32_t *__restrict__ navi, const uint32_t *__restrict__ navi_alt,
+                                                 const uint8_t *__restrict__ navi_sel, uint8_t *__restrict__ navi_out,
+                                                 const uint8_t *sz_n = nullptr)
 {
     size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     size_t total = (size_t)d.B * d.N * 4 * d.L * d.L;
@@ -262,12 +363,31 @@ __global__ void unpack_navi_kernel(EnvDims d, const uint32_t *__restrict__ navi,
     int x = (idx / d.L) % d.L;
     int k = (idx / ((size_t)d.L * d.L)) % 4;
     size_t ea = idx / ((size_t)4 * d.L * d.L);
+    if constexpr (SIZED) {
+        if ((int)(ea % d.N) >= (int)sz_n[ea / d.N]) {
+            navi_out[idx] = 0;
+            return;
+        }
+    }
     const int pr = x + 4, pc = y + 4;
     const int bx = min(pr >> 3, d.NB - 1), by = min(pc >> 3, d.NB - 1);
     const uint32_t *live = (navi_alt && navi_sel[ea / d.N]) ? navi_alt : navi;
     const uint2 v = reinterpret_cast<const uint2 *>(live + ea * d.navi_agent_stride)[((size_t)(bx * d.NB + by) << 4) + (pr - 8 * bx)];
     const uint32_t half = k < 2 ? v.x : v.y;
     navi_out[idx] = (half >> (16 * (k & 1) + (pc - 8 * by))) & 1u;
+}
+
+__global__ void unpack_navi_kernel(EnvDims d, const uint32_t *__restrict__ navi, const uint32_t *__restrict__ navi_alt,
+                                   const uint8_t *__restrict__ navi_sel, uint8_t *__restrict__ navi_out)
+{
+    unpack_navi_body<false>(d, navi, navi_alt, navi_sel, navi_out);
+}
+
+__global__ void unpack_navi_sized_kernel(EnvDims d, const uint32_t *__restrict__ navi, const uint32_t *__restrict__ navi_alt,
+                                         const uint8_t *__restrict__ navi_sel, uint8_t *__restrict__ navi_out,
+                                         const uint8_t *__restrict__ sz_n)
+{
+    unpack_navi_body<true>(d, navi, navi_alt, navi_sel, navi_out, sz_n);
 }
 
 }  // namespace
@@ -282,11 +402,24 @@ int mapf_launch_pack_load(mapf_env *env, const int32_t *d_env_ids, int n, const 
     return MAPF_OK;
 }
 
+// sized handle: d_n / d_l u8[n] per instance (NULL: N and L)
+int mapf_launch_pack_load_sized(mapf_env *env, const int32_t *d_env_ids, int n, const uint8_t *d_maps, const uint8_t *d_agents,
+                                const uint8_t *d_goals, const uint8_t *d_n, const uint8_t *d_l, cudaStream_t st)
+{
+    pack_load_sized_kernel<<<n, 128, 0, st>>>(env->d, d_env_ids, n, d_maps, d_agents, d_goals, env->obst, env->pos, env->goal,
+                                              env->steps, env->err, d_n, d_l, env->sz_n, env->sz_l);
+    MAPF_CUDA(cudaGetLastError());
+    return MAPF_OK;
+}
+
 // slots env_ids[0..n) (NULL: slots 0..n-1)
 int mapf_launch_validate_state(mapf_env *env, const int32_t *d_env_ids, int n, cudaStream_t st)
 {
     if (n <= 0) return MAPF_OK;
-    validate_state_kernel<<<(n + 3) / 4, 128, 0, st>>>(env->d, d_env_ids, n, env->pos, env->goal, env->err);
+    if (env->sz_n)
+        validate_state_sized_kernel<<<(n + 3) / 4, 128, 0, st>>>(env->d, d_env_ids, n, env->pos, env->goal, env->err, env->sz_n, env->sz_l);
+    else
+        validate_state_kernel<<<(n + 3) / 4, 128, 0, st>>>(env->d, d_env_ids, n, env->pos, env->goal, env->err);
     MAPF_CUDA(cudaGetLastError());
     return MAPF_OK;
 }
@@ -309,6 +442,9 @@ static int launch_bfs_rw(mapf_env *env, const int32_t *ids, const uint8_t *mask,
             pregen_bfs_kernel<RW, RPL, APW><<<grid, kBfsWarps * 32, 0, st>>>(d, env->ro_prio, pregen_min, env->ro_work + 3, env->pg_obst, \
                                                                              env->pg_goal, env->navi, env->navi_alt, env->navi_sel, \
                                                                              env->pg_n, env->pg_cnt, env->pg_epi);                   \
+        else if (env->sz_n)                                                                                                         \
+            bfs_navi_sized_kernel<RW, RPL, APW><<<grid, kBfsWarps * 32, 0, st>>>(d, ids, mask, n, env->obst, env->goal, env->navi,   \
+                                                                                 dist, env->sz_n, env->sz_l);                        \
         else                                                                                                                        \
             bfs_navi_kernel<RW, RPL, APW><<<grid, kBfsWarps * 32, 0, st>>>(d, ids, mask, n, env->obst, env->goal, env->navi,         \
                                                                            env->navi_alt, env->navi_sel, dist);                      \
@@ -388,7 +524,8 @@ int mapf_launch_pregen_bfs(mapf_env *env, int min_count, cudaStream_t st)
 int mapf_launch_comm_mask(mapf_env *env, int k_nearest, uint8_t *d_out, cudaStream_t st)
 {
     const int grid = (env->d.B + kCommWarps - 1) / kCommWarps;
-    comm_mask_kernel<<<grid, kCommWarps * 32, 0, st>>>(env->d, env->pos, k_nearest, d_out);
+    if (env->sz_n) comm_mask_sized_kernel<<<grid, kCommWarps * 32, 0, st>>>(env->d, env->pos, k_nearest, d_out, env->sz_n);
+    else comm_mask_kernel<<<grid, kCommWarps * 32, 0, st>>>(env->d, env->pos, k_nearest, d_out);
     MAPF_CUDA(cudaGetLastError());
     return MAPF_OK;
 }
@@ -403,7 +540,11 @@ int mapf_launch_unpack(mapf_env *env, uint8_t *d_map, uint8_t *d_navi, cudaStrea
     }
     if (d_navi) {
         size_t total = (size_t)d.B * d.N * 4 * d.L * d.L;
-        unpack_navi_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(d, env->navi, env->navi_alt, env->navi_sel, d_navi);
+        if (env->sz_n)
+            unpack_navi_sized_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(d, env->navi, env->navi_alt, env->navi_sel, d_navi,
+                                                                                      env->sz_n);
+        else
+            unpack_navi_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(d, env->navi, env->navi_alt, env->navi_sel, d_navi);
         MAPF_CUDA(cudaGetLastError());
     }
     return MAPF_OK;

@@ -39,7 +39,8 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k)
     return c;
 }
 
-enum : uint32_t { PURPOSE_DENSITY = 0, PURPOSE_MAP = 1, PURPOSE_AGENT = 2 };
+// PURPOSE_LEVEL: the setting a sized handle's reset draws for the slot (reset_levels_kernel), counter (g, 3, 0)
+enum : uint32_t { PURPOSE_DENSITY = 0, PURPOSE_MAP = 1, PURPOSE_AGENT = 2, PURPOSE_LEVEL = 3 };
 
 #ifdef MAPF_ENABLE_DIAG
 // diagnosis build: cycles of the generator's phases for environment 0 (profiles/tools/r2_generator_phases.py); accumulated in
@@ -177,13 +178,17 @@ __device__ __forceinline__ bool test_cell(const Bits<RW, RPL> &m, int code, int 
 }
 
 // All 32 lanes of the warp call together.  Writes obst / pos / goal of environment e and steps[e] = 0.
+// The instance has N <= d.N agents on an L <= d.L map (a sized handle's slot; rows N.. of pos / goal are not written).  The
+// draw does not depend on the template's capacity: the map is keyed by row and quad, and the picks run in lane-major row
+// order, in which rows past L are empty.
 template <int RW, int RPL>
 __device__ __forceinline__ void reset_env_warp(const EnvDims &d, const int e, const uint64_t seed, const uint64_t g,
                                                const float density, uint32_t *__restrict__ obst, uint8_t *__restrict__ pos,
-                                               uint8_t *__restrict__ goal, int32_t *__restrict__ steps, int32_t *__restrict__ err)
+                                               uint8_t *__restrict__ goal, int32_t *__restrict__ steps, int32_t *__restrict__ err,
+                                               const int L, const int N)
 {
     const int lane = threadIdx.x & 31;
-    const int L = d.L, N = d.N;
+    const int NS = d.N;  // row stride of pos / goal
     const uint2 key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
     const uint32_t g_lo = (uint32_t)g, g_hi = (uint32_t)(g >> 32);
 
@@ -334,7 +339,7 @@ __device__ __forceinline__ void reset_env_warp(const EnvDims &d, const int e, co
             }
             MAPF_RESET_TICK(5);  // second pick + bookkeeping
             if (lane == 0) {
-                const size_t o = ((size_t)e * N + i) * 2;
+                const size_t o = ((size_t)e * NS + i) * 2;
                 pos[o] = (uint8_t)(s >> 8);
                 pos[o + 1] = (uint8_t)((s & 0xff) - 4);
                 goal[o] = (uint8_t)(t >> 8);
@@ -370,6 +375,14 @@ __device__ __forceinline__ void reset_env_warp(const EnvDims &d, const int e, co
     if (e == 0 && lane == 0)
         for (int i = 0; i < 8; ++i) g_reset_cycles[i] = (unsigned long long)_acc[i];
 #endif
+}
+
+template <int RW, int RPL>
+__device__ __forceinline__ void reset_env_warp(const EnvDims &d, const int e, const uint64_t seed, const uint64_t g,
+                                               const float density, uint32_t *__restrict__ obst, uint8_t *__restrict__ pos,
+                                               uint8_t *__restrict__ goal, int32_t *__restrict__ steps, int32_t *__restrict__ err)
+{
+    reset_env_warp<RW, RPL>(d, e, seed, g, density, obst, pos, goal, steps, err, d.L, d.N);
 }
 
 }  // namespace

@@ -138,16 +138,23 @@ struct EnvRegs {
 // been re-generated -- nobody moves, rewards are 0, done is 0 and the step counter stays 0 (the call emits the new
 // episode's first observation).  Actions are software-pipelined: out.act_next holds this step's actions (the kernel loads
 // the first step's), `next_actions` (NULL on the last step of an item) is where the next step's are requested from.
-template <int RW, int K, bool DO_STEP, bool DO_OBS = true, bool RESIDENT = false>
+// SIZED (sized handle, never RESIDENT): the environment has n_e = sz_n[e] agents on an l_e = sz_l[e] map
+// inside the handle's N x L layout.  Agents a >= n_e are absent: their actions are never read, they hold no cell, their
+// reward is 0 with code MAPF_RCODE_RESET and their 486-bit stream is zero.  A move outside l_e is a collision; the bitmap
+// and the heuristic maps are zero outside l_e, so the gather itself needs no clipping.
+template <int RW, int K, bool DO_STEP, bool DO_OBS = true, bool RESIDENT = false, bool SIZED = false>
 __device__ __forceinline__ void env_step_gather(const StepParams &p, const int e, const int lane, uint32_t *s_obst,
                                                 uint32_t *s_agent, uint32_t *s_bits, uint16_t *s_tgt, uint16_t *s_cell,
                                                 const int head, const uint64_t pol_keep, EnvRegs<K> &out,
                                                 const uint8_t *s_act = nullptr, uint64_t *s_tiles = nullptr,
-                                                const bool reset_step = false, const uint8_t *next_actions = nullptr)
+                                                const bool reset_step = false, const uint8_t *next_actions = nullptr,
+                                                const uint8_t *sz_n = nullptr, const uint8_t *sz_l = nullptr)
 {
     constexpr int RWS = RW + 1;
     const EnvDims &d = p.d;
     const int N = d.N, L = d.L;
+    int NA = N, LB = L;  // agents present, bounds of a move
+    if constexpr (SIZED) NA = __ldg(sz_n + e), LB = __ldg(sz_l + e);
     // The cell -> agent grid of the step phase lives in the bit-stream buffer (the two are never live at
     // the same time).  It is never cleared: an entry is trusted only if it round-trips through s_cell.
     uint8_t *s_occ = reinterpret_cast<uint8_t *>(s_bits);
@@ -201,7 +208,7 @@ __device__ __forceinline__ void env_step_gather(const StepParams &p, const int e
 #pragma unroll
         for (int k = 0; k < K; ++k) {
             const int a = k * 32 + lane;
-            valid[k] = a < N;
+            valid[k] = a < NA;
             px[k] = py[k] = 0;
             if constexpr (DO_STEP) gx[k] = gy[k] = act[k] = 0;
             if constexpr (RESIDENT) {
@@ -295,7 +302,7 @@ __device__ __forceinline__ void env_step_gather(const StepParams &p, const int e
                 tcell[k] = tx[k] * L + ty[k];
                 if (mover[k]) {
                     // round 1: out of range / obstacle, environment.py:320-332
-                    bool bad = tx[k] < 0 || ty[k] < 0 || tx[k] >= L || ty[k] >= L;
+                    bool bad = tx[k] < 0 || ty[k] < 0 || tx[k] >= LB || ty[k] >= LB;
                     if (!bad) bad = (s_obst[(tx[k] + 4) * RWS + ((ty[k] + 4) >> 5)] >> ((ty[k] + 4) & 31)) & 1u;
                     if (bad) {
                         code[k] = RC_COLLISION;
@@ -448,6 +455,11 @@ __device__ __forceinline__ void env_step_gather(const StepParams &p, const int e
                     const int c = reset_step ? RC_RESET : (done ? RC_FINISH : code[k]);
                     if (p.rewards) p.rewards[(size_t)e * N + a] = reward_of(p, c);
                     if (p.codes) p.codes[(size_t)e * N + a] = (uint8_t)c;
+                } else if constexpr (SIZED) {
+                    if (a < N) {
+                        if (p.rewards) p.rewards[(size_t)e * N + a] = 0.0f;
+                        if (p.codes) p.codes[(size_t)e * N + a] = (uint8_t)RC_RESET;
+                    }
                 }
             }
             if (lane == 0) {
@@ -464,6 +476,9 @@ __device__ __forceinline__ void env_step_gather(const StepParams &p, const int e
                     if (valid[k])
                         reinterpret_cast<uchar2 *>(p.pos_out)[(size_t)e * N + k * 32 + lane] =
                             make_uchar2((unsigned char)px[k], (unsigned char)py[k]);
+                    else if constexpr (SIZED) {
+                        if (k * 32 + lane < N) reinterpret_cast<uchar2 *>(p.pos_out)[(size_t)e * N + k * 32 + lane] = make_uchar2(255, 255);
+                    }
             }
             asm volatile("cp.async.wait_all;" ::: "memory");
             __syncwarp();  // s_obst visible
@@ -578,10 +593,19 @@ __device__ __forceinline__ void env_step_gather(const StepParams &p, const int e
                 };
                 FieldWalk<0>::run(0ull, val, emit, mid);
                 if (((o + 485) >> 5) == 16) S[16] = __funnelshift_l(prev, 0u, o);
+            } else if constexpr (SIZED) {
+                // an absent agent's 486 bits are zero (words it shares with its neighbours: see below)
+                if (a < N) {
+#pragma unroll
+                    for (int m = 1; m < 16; ++m) S[m] = 0;
+                    if (((o + 485) >> 5) == 16) S[16] = 0;
+                }
             }
             __syncwarp();
             // first word: shared with the previous agent's last word unless this agent starts a word
-            if (valid[k]) {
+            bool streams = valid[k];
+            if constexpr (SIZED) streams = a < N;
+            if (streams) {
                 if (o == 0 || a == 0) S[0] = x0;
                 else S[0] |= x0;
             }

@@ -17,14 +17,14 @@
 namespace {
 
 // ---- K1+K2: every warp steps an env, then expands and stores its own observation block.
-template <int RW, int K, bool DO_STEP, int WARPS, int MINB>
-__global__ void __launch_bounds__(WARPS * 32, MINB)
-step_observe_kernel(const StepParams p)
+// (threadIdx.x is read by the kernel: the range its launch bounds give it is what lets the compiler form e with an OR)
+template <int RW, int K, bool DO_STEP, int WARPS, bool SIZED>
+__device__ __forceinline__ void step_observe_body(const StepParams &p, uint32_t *smem, const int tid, const uint8_t *sz_n = nullptr,
+                                                  const uint8_t *sz_l = nullptr)
 {
-    extern __shared__ __align__(16) uint32_t smem[];
     const EnvDims &d = p.d;
-    const int lane = threadIdx.x & 31;
-    const int warp = threadIdx.x >> 5;
+    const int lane = tid & 31;
+    const int warp = tid >> 5;
     const int N = d.N;
 
     uint32_t *s_obst = smem + (size_t)warp * p.warp_smem_words;
@@ -46,11 +46,30 @@ step_observe_kernel(const StepParams p)
         uint8_t *obs_env = p.obs + (size_t)(p.obs_rows ? p.obs_rows[e] : (int64_t)e) * env_bytes;
         const int head = (int)(reinterpret_cast<uintptr_t>(obs_env) & 15);  // bytes before the 16-B boundary
         EnvRegs<K> r;
-        env_step_gather<RW, K, DO_STEP>(p, e, lane, s_obst, s_agent, s_bits, s_tgt, s_cell, head, pol_keep, r);
+        env_step_gather<RW, K, DO_STEP, true, false, SIZED>(p, e, lane, s_obst, s_agent, s_bits, s_tgt, s_cell, head, pol_keep, r,
+                                                            nullptr, nullptr, false, nullptr, sz_n, sz_l);
         expand_store_block(p, obs_env, head, env_bytes, s_bits, lane, obs_policy, pol_stream);
         __syncwarp();
         clear_agent_bits<RW, K>(s_agent, r);  // the agent bits this env set
     }
+}
+
+template <int RW, int K, bool DO_STEP, int WARPS, int MINB>
+__global__ void __launch_bounds__(WARPS * 32, MINB)
+step_observe_kernel(const StepParams p)
+{
+    extern __shared__ __align__(16) uint32_t smem[];
+    step_observe_body<RW, K, DO_STEP, WARPS, false>(p, smem, threadIdx.x);
+}
+
+// the same for a sized handle (per-environment agent count and side, mapf_env_enable_sizes): a separate instantiation, so
+// the uniform kernels above carry none of it
+template <int RW, int K, bool DO_STEP>
+__global__ void __launch_bounds__(128)
+step_observe_sized_kernel(const StepParams p, const uint8_t *__restrict__ sz_n, const uint8_t *__restrict__ sz_l)
+{
+    extern __shared__ __align__(16) uint32_t smem[];
+    step_observe_body<RW, K, DO_STEP, 4, true>(p, smem, threadIdx.x, sz_n, sz_l);
 }
 
 // ---- K1 alone: Environment.step without the observation.  The host-buffer steps launch it ahead of the observe kernel so
@@ -161,9 +180,32 @@ int launch_step_rwk(const mapf_env *env, StepParams &p, cudaStream_t st)
     return launch_step_cfg<RW, K, DO_STEP, 4, (K == 1 ? 12 : 1)>(env, p, st);
 }
 
+template <int RW, int K, bool DO_STEP>
+int launch_step_sized(const mapf_env *env, StepParams &p, cudaStream_t st)
+{
+    auto kern = step_observe_sized_kernel<RW, K, DO_STEP>;
+    const size_t smem = (size_t)p.warp_smem_words * 4 * 4;
+    if (smem > 227 * 1024) {
+        mapf_set_error("map too large for the step kernel's shared memory");
+        return MAPF_EINVAL;
+    }
+    if (smem > 48 * 1024) MAPF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<(p.env_end - p.env_begin + 3) / 4, 128, smem, st>>>(p, env->sz_n, env->sz_l);
+    MAPF_CUDA(cudaGetLastError());
+    return MAPF_OK;
+}
+
 template <int RW, bool DO_STEP>
 int launch_step_rw(const mapf_env *env, StepParams &p, cudaStream_t st)
 {
+    if (env->sz_n) {
+        switch (env->d.K) {
+            case 1: return launch_step_sized<RW, 1, DO_STEP>(env, p, st);
+            case 2: return launch_step_sized<RW, 2, DO_STEP>(env, p, st);
+            case 3: return launch_step_sized<RW, 3, DO_STEP>(env, p, st);
+            case 4: return launch_step_sized<RW, 4, DO_STEP>(env, p, st);
+        }
+    }
     switch (env->d.K) {
         case 1: return launch_step_rwk<RW, 1, DO_STEP>(env, p, st);
         case 2: return launch_step_rwk<RW, 2, DO_STEP>(env, p, st);

@@ -1,5 +1,5 @@
 """ReplayStore — device-resident mirror of the storage and sampling half of the reference's `GlobalBuffer`
-(worker.py:21-203, without Ray and without the curriculum statistics).
+(worker.py:21-203, without Ray; the curriculum statistics are `curriculum.Curriculum`).
 
 The buffers keep the reference's logical layout (worker.py:36-42) as CUDA tensors: episode slot g owns
 observation / comm-mask rows g*(max_steps+1)+f and action / reward / hidden rows g*max_steps+t, and the
