@@ -65,6 +65,17 @@ extern "C" {
 #define MAPF_FOV 9
 #define MAPF_OBS_CHANNELS 6
 #define MAPF_OBS_BYTES_PER_AGENT 486 /* 6*9*9, config.py:7 obs_shape */
+/* Packed observation (the compact replay store): one 64-byte row per agent.  Element k = c*81 + r*9 + col of the agent's
+ * flattened 6x9x9 bool observation is bit (k & 7) of byte (k >> 3), LSB first -- np.packbits(obs.reshape(N, 486), axis=-1,
+ * bitorder="little") padded to 64 bytes; bits 486..511 are always 0.  A frame is N*64 bytes.  This is the step kernel's own
+ * bit stream with agent a at bit 512*a instead of 486*a, so every agent starts on a word boundary. */
+#define MAPF_OBS_PACKED_BYTES_PER_AGENT 64
+/* Packed communication mask: agent i's row is CW = ceil(N/8) bytes, bit j (LSB first) = mask[i][j]; a frame is N*CW bytes. */
+
+/* element types of mapf_obs_unpack */
+#define MAPF_DTYPE_U8 0
+#define MAPF_DTYPE_F16 1
+#define MAPF_DTYPE_BF16 2
 #define MAPF_MAX_AGENTS 128
 #define MAPF_MAX_MAP_SIDE 120
 #define MAPF_DIST_UNREACHABLE 2147483647 /* environment.py:218 */
@@ -132,6 +143,20 @@ int mapf_env_observe(mapf_env *env, uint8_t *d_obs, uint8_t *d_pos, void *stream
 int mapf_env_step_observe_rows(mapf_env *env, const uint8_t *d_actions, uint8_t *d_obs_base, const int64_t *d_obs_rows,
                                float *d_rewards, uint8_t *d_done, int32_t *d_steps, void *stream);
 int mapf_env_observe_rows(mapf_env *env, uint8_t *d_obs_base, const int64_t *d_obs_rows, uint8_t *d_pos, void *stream);
+
+/* The same step and observe writing PACKED observations (MAPF_OBS_PACKED_BYTES_PER_AGENT): environment e writes its N*64-byte
+ * frame at d_bits_base + d_bits_rows[e] * N*64 (d_bits_rows i64[B]; NULL = row e).  d_bits_base must be 16-byte aligned.
+ * Positions, rewards, codes, done, steps and latched errors are those of mapf_env_step_observe_ex; the frame is
+ * np.packbits of what the dense call writes, pad bits 0.  Uniform and sized handles (an absent agent's 64 bytes are 0). */
+int mapf_env_step_observe_packed(mapf_env *env, const uint8_t *d_actions, uint8_t *d_bits_base, const int64_t *d_bits_rows,
+                                 float *d_rewards, uint8_t *d_codes, uint8_t *d_done, int32_t *d_steps, void *stream);
+int mapf_env_observe_packed(mapf_env *env, uint8_t *d_bits_base, const int64_t *d_bits_rows, uint8_t *d_pos, void *stream);
+
+/* Packed observation frames -> dense [count, N, 6, 9, 9] elements of `dtype` (MAPF_DTYPE_U8 0 / 1, MAPF_DTYPE_F16 or
+ * MAPF_DTYPE_BF16 0.0 / 1.0).  Frame i is read at d_bits_base + d_rows[i] * N*64 (d_rows i64[count]; NULL = row i).  Both
+ * pointers must be 16-byte aligned. */
+int mapf_obs_unpack(const uint8_t *d_bits_base, const int64_t *d_rows, int64_t count, int32_t num_agents, int32_t dtype,
+                    void *d_out, void *stream);
 
 /* T lockstep steps with the actions already resident on the device: the loop `for t: obs, r, done, _ = env.step(a[t])`
  * of test.py:120-130 / worker.py:383-395 when the actions do not depend on the observations (replaying planner paths,
@@ -252,6 +277,11 @@ int mapf_debug_step_host_mode(int32_t mode);
  *   distance, i itself included.  torch.topk's order among equal distances is unspecified; ties go to
  *   the lower agent id here. */
 int mapf_env_comm_mask(mapf_env *env, int32_t max_comm_agents, uint8_t *d_mask_out, void *stream);
+/* The same mask in one launch as the dense u8[B, N, N] (d_mask_out, optional: what the Q-network consumes) AND as packed rows
+ * (the comm-mask format above): environment e writes N*ceil(N/8) bytes at d_bits_base + d_bits_rows[e] * N*ceil(N/8)
+ * (d_bits_rows i64[B]; NULL = row e).  Uniform and sized handles. */
+int mapf_env_comm_mask_packed(mapf_env *env, int32_t max_comm_agents, uint8_t *d_mask_out, uint8_t *d_bits_base,
+                              const int64_t *d_bits_rows, void *stream);
 
 /* ---- state access (attributes read by worker.py:390,426 / test.py:46-48,130) --------------- */
 /* Any output pointer may be NULL.  d_map u8[B,L,L]; d_pos/d_goals u8[B,N,2]; d_steps i32[B];
@@ -419,6 +449,30 @@ typedef struct mapf_replay_batch {
  * leaf lies beyond its episode's size (the reference asserts, worker.py:120). */
 int mapf_replay_gather(const mapf_replay_view *view, const int64_t *d_idx, int64_t batch, const mapf_replay_batch *out,
                        int32_t *d_err, void *stream);
+
+/* The compact store: the same logical store with packed observations and comm masks (formats above) and ONE hidden vector per
+ * transition (the reference writes agent 0's hidden state into every agent's row, buffer.py:148).  About 12x fewer bytes per
+ * transition at 32 agents (DESIGN.md §3). */
+typedef struct mapf_replay_view_compact {
+    const uint8_t *obs_bits;   /* u8 [(max_steps+1)*capacity, num_agents, 64]                  */
+    const uint8_t *comm_bits;  /* u8 [(max_steps+1)*capacity, num_agents, ceil(num_agents/8)]  */
+    const uint16_t *hid_buf;   /* fp16 [max_steps*capacity, latent_dim]                        */
+    const uint8_t *act_buf;    /* u8  [max_steps*capacity]                                      */
+    const uint16_t *rew_buf;   /* fp16 [max_steps*capacity]                                     */
+    const uint8_t *done_buf;   /* u8 bool [capacity]                                            */
+    const int32_t *size_buf;   /* i32 [capacity]                                                */
+    int32_t num_agents;
+    int32_t max_steps;
+    int32_t bt_steps;
+    int32_t forward_steps;
+    int32_t latent_dim;
+} mapf_replay_view_compact;
+
+/* mapf_replay_gather from a compact store: fills the same mapf_replay_batch with the same contents the dense gather gives
+ * for the same logical store (fp16 observations, u8 comm masks, the sample's hidden vector in each of its N rows, scalars,
+ * zero padding, d_err).  view->obs_bits must be 16-byte aligned. */
+int mapf_replay_gather_compact(const mapf_replay_view_compact *view, const int64_t *d_idx, int64_t batch,
+                               const mapf_replay_batch *out, int32_t *d_err, void *stream);
 
 /* ---- CBS expert / solvable-instance generator (search.py:58-442, test.py:23-79; SURVEY 8(f)4) -- HOST code ------------------
  * Conflict-based search over space-time A*: a collision-free set of paths of minimal sum of costs (search.py:17-21), as the

@@ -12,6 +12,8 @@ _lib = None
 MAPF_OK, MAPF_EINVAL, MAPF_ECUDA, MAPF_EACTION, MAPF_EUNIQUE, MAPF_ENOMEM, MAPF_ENOSPACE = 0, -1, -2, -3, -4, -5, -6
 MAPF_ESTATE, MAPF_EINTERNAL, MAPF_EINDEX, MAPF_EPRIORITY = -7, -8, -9, -10
 ABI_VERSION = 2
+# element types of mapf_obs_unpack (MAPF_DTYPE_*)
+DTYPE_U8, DTYPE_F16, DTYPE_BF16 = 0, 1, 2
 # reward codes (MAPF_RCODE_*): index into reward_fn in config.REWARD_ORDER; 5 = reset step (reward 0), and on a sized
 # handle an absent agent slot
 RCODE_RESET = 5
@@ -24,6 +26,13 @@ class EnvConfig(C.Structure):
 
 class ReplayView(C.Structure):
     _fields_ = [("obs_buf", C.c_void_p), ("comm_buf", C.c_void_p), ("hid_buf", C.c_void_p), ("act_buf", C.c_void_p),
+                ("rew_buf", C.c_void_p), ("done_buf", C.c_void_p), ("size_buf", C.c_void_p),
+                ("num_agents", C.c_int32), ("max_steps", C.c_int32), ("bt_steps", C.c_int32),
+                ("forward_steps", C.c_int32), ("latent_dim", C.c_int32)]
+
+
+class ReplayViewCompact(C.Structure):
+    _fields_ = [("obs_bits", C.c_void_p), ("comm_bits", C.c_void_p), ("hid_buf", C.c_void_p), ("act_buf", C.c_void_p),
                 ("rew_buf", C.c_void_p), ("done_buf", C.c_void_p), ("size_buf", C.c_void_p),
                 ("num_agents", C.c_int32), ("max_steps", C.c_int32), ("bt_steps", C.c_int32),
                 ("forward_steps", C.c_int32), ("latent_dim", C.c_int32)]
@@ -65,6 +74,9 @@ SIGNATURES = {
     "mapf_env_observe": (C.c_int, [_vp, _vp, _vp, _vp]),
     "mapf_env_step_observe_rows": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mapf_env_observe_rows": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
+    "mapf_env_step_observe_packed": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "mapf_env_observe_packed": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
+    "mapf_obs_unpack": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _vp, _vp]),
     "mapf_env_rollout": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _i32, _vp, _vp, _vp, _i32, _i32, _vp]),
     "mapf_env_rollout_ex": (C.c_int, [_vp, C.POINTER(RolloutIO), _vp]),
     "mapf_env_set_autoreset": (C.c_int, [_vp, _i32, _u64, _u64, _u64, _f32, _vp]),
@@ -79,6 +91,7 @@ SIGNATURES = {
     "mapf_debug_rollout_pregen": (C.c_int, [_i32]),
     "mapf_debug_rollout_tasks": (C.c_int, [_i32]),
     "mapf_env_comm_mask": (C.c_int, [_vp, _i32, _vp, _vp]),
+    "mapf_env_comm_mask_packed": (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp]),
     "mapf_env_get_state": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mapf_env_set_state": (C.c_int, [_vp, _vp, _vp, _vp]),
     "mapf_env_status": (C.c_int, [_vp, _vp]),
@@ -95,6 +108,7 @@ SIGNATURES = {
     "mapf_per_td_update": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _f32, _f64, _i64, _i64, _i64,
                                      _vp, _vp, _vp]),
     "mapf_replay_gather": (C.c_int, [C.POINTER(ReplayView), _vp, _i64, C.POINTER(ReplayBatch), _vp, _vp]),
+    "mapf_replay_gather_compact": (C.c_int, [C.POINTER(ReplayViewCompact), _vp, _i64, C.POINTER(ReplayBatch), _vp, _vp]),
     "mapf_actor_td": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp]),
     "mapf_actor_td_n": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _f64, _vp, _vp]),
     "mapf_per_cycle": (C.c_int, [_vp, C.POINTER(PerCycleArgs), _vp]),

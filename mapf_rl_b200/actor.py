@@ -19,6 +19,9 @@ Every environment owns one episode slot of the store while its episode runs; a f
 (priorities inserted, size / done recorded) and the environment takes the next free slot of the ring, whose
 old leaves are zeroed first so a half-overwritten episode is never sampled.  The only host synchronisation
 per step is the read of the B-byte "episode finished" mask.
+With a compact store (`ReplayStore(compact=True)`) the step kernel and the comm-mask kernel write packed rows, the current
+frames are unpacked from the store for the Q-network (mapf_obs_unpack), and one hidden vector is kept per transition; the
+store then holds exactly what the dense store would.
 """
 from __future__ import annotations
 
@@ -29,6 +32,7 @@ import numpy as np
 from . import config
 from .batched import BatchedEnvironment
 from .buffer import actor_td_errors
+from .packed import unpack_obs
 from .replay import ReplayStore
 
 
@@ -121,7 +125,10 @@ class BatchedActor:
         self.t[idt] = 0
         # frame 0 of the new episodes (LocalBuffer.__init__: obs_buf[0] = init_obs, buffer.py:131); environments
         # in the middle of an episode rewrite the frame they already hold
-        self.env.observe(out_obs=self.store.obs_buf, obs_rows=self._rows())
+        if self.store.compact:
+            self.env.observe(out_bits=self.store.obs_bits, obs_rows=self._rows())
+        else:
+            self.env.observe(out_obs=self.store.obs_buf, obs_rows=self._rows())
         if self.on_begin is not None:
             self.on_begin(self, ids)
         return mask
@@ -137,9 +144,13 @@ class BatchedActor:
             self.net.reset()
             self._started = True
         rows = self._rows()
-        obs = st.obs_buf.index_select(0, rows)                                   # [B,N,6,9,9] current frames
-        comm = env.comm_mask()                                                   # model.py:196-208
-        st.comm_mask.index_copy_(0, rows, comm)                                  # comm_buf[size] = comm_mask, buffer.py:149
+        if st.compact:
+            obs = unpack_obs(st.obs_bits, rows)                                  # [B,N,6,9,9] current frames
+            comm = env.comm_mask(out_bits=st.comm_bits, rows=rows)               # + the packed row of comm_buf[size]
+        else:
+            obs = st.obs_buf.index_select(0, rows)                               # [B,N,6,9,9] current frames
+            comm = env.comm_mask()                                               # model.py:196-208
+            st.comm_mask.index_copy_(0, rows, comm)                              # comm_buf[size] = comm_mask, buffer.py:149
         actions, q, hidden = self.net.step(obs, comm, reset_mask=self._pending_reset)
         self._pending_reset = None
         # only agent 0 explores (worker.py:380-382)
@@ -148,12 +159,18 @@ class BatchedActor:
         actions = actions.clone()
         actions[:, 0] = torch.where(explore, rnd, actions[:, 0])
         a8 = actions.to(torch.uint8)
-        _, rewards, done = env.step(a8, out_obs=st.obs_buf, obs_rows=rows + 1)   # next_obs -> obs_buf[size + 1]
+        if st.compact:
+            _, rewards, done = env.step(a8, out_bits=st.obs_bits, obs_rows=rows + 1)
+        else:
+            _, rewards, done = env.step(a8, out_obs=st.obs_buf, obs_rows=rows + 1)   # next_obs -> obs_buf[size + 1]
         # local_buffer.add(q_val[0], actions[0], r[0], next_obs, hidden[0], comm_mask)  (worker.py:388, buffer.py:140-151)
         leaf = self.slot * S + self.t
         st.act_buf[leaf] = a8[:, 0]
         st.rew_buf[leaf] = rewards[:, 0].to(torch.float16)
-        st.hid_buf[leaf] = hidden[:, 0:1, :].to(torch.float16).expand(B, N, hidden.shape[-1])   # agent 0's vector, broadcast (SURVEY q8)
+        if st.compact:
+            st.hid_buf[leaf] = hidden[:, 0].to(torch.float16)                   # agent 0's vector, once
+        else:
+            st.hid_buf[leaf] = hidden[:, 0:1, :].to(torch.float16).expand(B, N, hidden.shape[-1])   # agent 0's vector, broadcast (SURVEY q8)
         self.q_buf[torch.arange(B, device=self.dev), self.t] = q[:, 0, :].float()
         self.t += 1
         self.transitions += B
@@ -182,7 +199,11 @@ class BatchedActor:
         # comm_buf[size]: the mask of the last model.step when the episode was cut at max_steps (worker.py:399-401; the
         # reference re-runs the model on the PREVIOUS observation there), zeros when it ended by done (buffer.py:124,155-156)
         last_rows = slots * (S + 1) + size
-        st.comm_mask[last_rows] = torch.where(done[:, None, None], torch.zeros_like(comm[idt]), comm[idt])
+        if st.compact:   # the packed row of this step's mask went to the row before (comm_mask(out_bits=...) in step)
+            prev = st.comm_bits[last_rows - 1]
+            st.comm_bits[last_rows] = torch.where(done[:, None, None], torch.zeros_like(prev), prev)
+        else:
+            st.comm_mask[last_rows] = torch.where(done[:, None, None], torch.zeros_like(comm[idt]), comm[idt])
         # initial priorities (buffer.py:170-177) and their insertion (worker.py:87-94)
         leaves = (slots[:, None] * S + torch.arange(S, device=self.dev)[None, :])
         rew = st.rew_buf[leaves].float()

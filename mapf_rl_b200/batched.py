@@ -192,13 +192,15 @@ class BatchedEnvironment:
                                                C.c_float(dens), self._stream()))
 
     # -- Environment.step + observe (environment.py:278-467) -------------------------------------
-    def step(self, actions, out_obs=None, out_rewards=None, out_done=None, obs_rows=None, out_codes=None):
+    def step(self, actions, out_obs=None, out_rewards=None, out_done=None, obs_rows=None, out_codes=None, out_bits=None):
         """actions: uint8 CUDA tensor [B,N] (anything else is converted).
         Returns (obs uint8[B,N,6,9,9], rewards float32[B,N], done uint8[B]); obs is written into
         `out_obs` when given (e.g. a slot of a device replay tensor).  With `obs_rows` (int64 CUDA tensor [B]),
         `out_obs` is the whole observation buffer of a replay store ([rows,N,6,9,9]) and environment e writes
         its block at row obs_rows[e] (returned obs is then `out_obs` itself).  `out_codes` (uint8 CUDA tensor [B,N])
-        additionally receives the reward codes (index into config.REWARD_ORDER)."""
+        additionally receives the reward codes (index into config.REWARD_ORDER).
+        `out_bits` (uint8 CUDA tensor [rows,N,64], instead of `out_obs`): the observation is written PACKED
+        (`mapf_rl_b200.packed`), at row obs_rows[e] or row e, and `out_bits` is returned in its place."""
         torch = _torch()
         B, N = self.num_envs, self.num_agents
         if not (isinstance(actions, torch.Tensor) and actions.dtype == torch.uint8 and actions.is_cuda
@@ -206,6 +208,15 @@ class BatchedEnvironment:
             actions = torch.as_tensor(np.asarray(actions) if not isinstance(actions, torch.Tensor) else actions)
             actions = actions.to(device=self.device, dtype=torch.uint8).contiguous()
         assert actions.shape == (B, N), "actions number"
+        if out_bits is not None:
+            assert out_obs is None, "out_bits replaces out_obs"
+            rewards = out_rewards if out_rewards is not None else self._rewards
+            done = out_done if out_done is not None else self._done
+            _native.check(self._lib.mapf_env_step_observe_packed(
+                self._h, C.c_void_p(actions.data_ptr()), C.c_void_p(out_bits.data_ptr()), self._bits_rows(out_bits, obs_rows),
+                C.c_void_p(rewards.data_ptr()), self._codes_ptr(out_codes), C.c_void_p(done.data_ptr()),
+                C.c_void_p(self._steps.data_ptr()), self._stream()))
+            return out_bits, rewards, done
         obs = out_obs if out_obs is not None else torch.empty((B, N, *self.OBS_SHAPE), dtype=torch.uint8, device=self.device)
         rewards = out_rewards if out_rewards is not None else self._rewards
         done = out_done if out_done is not None else self._done
@@ -216,14 +227,31 @@ class BatchedEnvironment:
             rows_ptr = C.c_void_p(obs_rows.data_ptr())
         else:
             assert obs.is_contiguous() and obs.dtype == torch.uint8 and obs.numel() == B * N * 486
-        codes_ptr = None
-        if out_codes is not None:
-            assert out_codes.is_cuda and out_codes.dtype == torch.uint8 and out_codes.is_contiguous() and out_codes.numel() == B * N
-            codes_ptr = C.c_void_p(out_codes.data_ptr())
+        codes_ptr = self._codes_ptr(out_codes)
         _native.check(self._lib.mapf_env_step_observe_ex(
             self._h, C.c_void_p(actions.data_ptr()), C.c_void_p(obs.data_ptr()), rows_ptr, C.c_void_p(rewards.data_ptr()),
             codes_ptr, C.c_void_p(done.data_ptr()), C.c_void_p(self._steps.data_ptr()), self._stream()))
         return obs, rewards, done
+
+    def _codes_ptr(self, out_codes):
+        if out_codes is None:
+            return None
+        torch = _torch()
+        assert (out_codes.is_cuda and out_codes.dtype == torch.uint8 and out_codes.is_contiguous()
+                and out_codes.numel() == self.num_envs * self.num_agents)
+        return C.c_void_p(out_codes.data_ptr())
+
+    def _bits_rows(self, bits, rows, row_bytes=64):
+        """Checks a packed output buffer [rows, N, row_bytes] and its optional int64 row tensor [B]; -> row pointer."""
+        torch = _torch()
+        B, N = self.num_envs, self.num_agents
+        assert (bits.is_cuda and bits.dtype == torch.uint8 and bits.is_contiguous() and bits.dim() == 3
+                and tuple(bits.shape[1:]) == (N, row_bytes)), f"packed buffer must be uint8 [rows, {N}, {row_bytes}]"
+        if rows is None:
+            assert bits.shape[0] >= B
+            return None
+        assert rows.dtype == torch.int64 and rows.is_cuda and rows.is_contiguous() and rows.numel() == B
+        return C.c_void_p(rows.data_ptr())
 
     def rollout(self, actions, num_steps: Optional[int] = None, out_obs=None, out_rewards=None, out_done=None,
                 out_steps=None, chains: int = 0, out_codes=None):
@@ -295,10 +323,18 @@ class BatchedEnvironment:
                                                      int(chains), *[C.byref(o) for o in out]))
         return tuple(o.value for o in out)
 
-    def observe(self, out_obs=None, obs_rows=None):
-        """-> (obs uint8[B,N,6,9,9], pos uint8[B,N,2])   (environment.py:433-467); `obs_rows` as in step()."""
+    def observe(self, out_obs=None, obs_rows=None, out_bits=None):
+        """-> (obs uint8[B,N,6,9,9], pos uint8[B,N,2])   (environment.py:433-467); `obs_rows` and `out_bits` (packed
+        observations, returned in the observation's place) as in step()."""
         torch = _torch()
         B, N = self.num_envs, self.num_agents
+        if out_bits is not None:
+            assert out_obs is None, "out_bits replaces out_obs"
+            pos = torch.empty((B, N, 2), dtype=torch.uint8, device=self.device)
+            _native.check(self._lib.mapf_env_observe_packed(self._h, C.c_void_p(out_bits.data_ptr()),
+                                                            self._bits_rows(out_bits, obs_rows), C.c_void_p(pos.data_ptr()),
+                                                            self._stream()))
+            return out_bits, pos
         obs = out_obs if out_obs is not None else torch.empty((B, N, *self.OBS_SHAPE), dtype=torch.uint8, device=self.device)
         pos = torch.empty((B, N, 2), dtype=torch.uint8, device=self.device)
         if obs_rows is not None:
@@ -310,13 +346,20 @@ class BatchedEnvironment:
                                                  self._stream()))
         return obs, pos
 
-    def comm_mask(self, max_comm_agents: int = config.max_comm_agents, out=None):
+    def comm_mask(self, max_comm_agents: int = config.max_comm_agents, out=None, out_bits=None, rows=None):
         """-> uint8[B,N,N] communication mask of Network.step (model.py:196-208) for the current positions:
-        in each other's field of view AND among the `max_comm_agents` nearest (self included; ties -> lower id)."""
+        in each other's field of view AND among the `max_comm_agents` nearest (self included; ties -> lower id).
+        `out_bits` (uint8 CUDA tensor [rows,N,ceil(N/8)]): the same launch also writes the mask as packed rows
+        (`mapf_rl_b200.packed`), at row rows[e] (int64 CUDA tensor [B]) or row e; the dense mask is still returned."""
         torch = _torch()
         B, N = self.num_envs, self.num_agents
         m = out if out is not None else torch.empty((B, N, N), dtype=torch.uint8, device=self.device)
         assert m.is_contiguous() and m.dtype == torch.uint8 and m.numel() == B * N * N
+        if out_bits is not None:
+            rows_ptr = self._bits_rows(out_bits, rows, row_bytes=(N + 7) // 8)
+            _native.check(self._lib.mapf_env_comm_mask_packed(self._h, int(max_comm_agents), C.c_void_p(m.data_ptr()),
+                                                              C.c_void_p(out_bits.data_ptr()), rows_ptr, self._stream()))
+            return m
         _native.check(self._lib.mapf_env_comm_mask(self._h, int(max_comm_agents), C.c_void_p(m.data_ptr()), self._stream()))
         return m
 

@@ -39,6 +39,12 @@ int mapf_launch_per_td_update(mapf_per *, PerScratch *, const float *, const flo
 int mapf_launch_per_cycle(mapf_per *, PerScratch *, const mapf_per_cycle_args *, cudaStream_t);
 int mapf_launch_actor_td(const float *, const float *, const uint8_t *, const int32_t *, int, int, int, double, double *, cudaStream_t);
 int mapf_launch_replay_gather(const mapf_replay_view *, const int64_t *, int64_t, const mapf_replay_batch *, int32_t *, cudaStream_t);
+int mapf_launch_step_packed(mapf_env *, const uint8_t *, uint8_t *, const int64_t *, const StepOut &, cudaStream_t);
+int mapf_launch_observe_packed(mapf_env *, uint8_t *, const int64_t *, uint8_t *, cudaStream_t);
+int mapf_launch_comm_mask_packed(mapf_env *, int, uint8_t *, uint8_t *, const int64_t *, cudaStream_t);
+int mapf_launch_obs_unpack(const uint8_t *, const int64_t *, int64_t, int, int, void *, cudaStream_t);
+int mapf_launch_replay_gather_compact(const mapf_replay_view_compact *, const int64_t *, int64_t, const mapf_replay_batch *, int32_t *,
+                                      cudaStream_t);
 
 static thread_local std::string g_last_error;
 
@@ -64,6 +70,8 @@ struct DeviceGuard {
         if (ok && prev >= 0) cudaSetDevice(prev);
     }
 };
+
+bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 bool host_is_pinned(const void *p)
 {
@@ -538,6 +546,31 @@ int mapf_env_observe(mapf_env *env, uint8_t *d_obs, uint8_t *d_pos, void *stream
         return MAPF_EINVAL;
     }
     return mapf_launch_observe(env, d_obs, nullptr, d_pos, nullptr, static_cast<cudaStream_t>(stream));
+}
+
+int mapf_env_step_observe_packed(mapf_env *env, const uint8_t *d_actions, uint8_t *d_bits_base, const int64_t *d_bits_rows,
+                                 float *d_rewards, uint8_t *d_codes, uint8_t *d_done, int32_t *d_steps, void *stream)
+{
+    REQUIRE_ENV(env);
+    MAPF_DRAIN(env, static_cast<cudaStream_t>(stream));
+    if (!d_actions || !d_bits_base || !d_done || !aligned16(d_bits_base)) {
+        mapf_set_error("mapf_env_step_observe_packed: NULL buffer or d_bits_base not 16-byte aligned");
+        return MAPF_EINVAL;
+    }
+    StepOut out;
+    out.rewards = d_rewards, out.codes = d_codes, out.done = d_done, out.steps = d_steps;
+    return mapf_launch_step_packed(env, d_actions, d_bits_base, d_bits_rows, out, static_cast<cudaStream_t>(stream));
+}
+
+int mapf_env_observe_packed(mapf_env *env, uint8_t *d_bits_base, const int64_t *d_bits_rows, uint8_t *d_pos, void *stream)
+{
+    REQUIRE_ENV(env);
+    MAPF_DRAIN(env, static_cast<cudaStream_t>(stream));
+    if (!d_bits_base || !aligned16(d_bits_base)) {
+        mapf_set_error("mapf_env_observe_packed: NULL buffer or d_bits_base not 16-byte aligned");
+        return MAPF_EINVAL;
+    }
+    return mapf_launch_observe_packed(env, d_bits_base, d_bits_rows, d_pos, static_cast<cudaStream_t>(stream));
 }
 
 namespace {
@@ -1101,6 +1134,18 @@ int mapf_env_comm_mask(mapf_env *env, int32_t max_comm_agents, uint8_t *d_mask_o
     return mapf_launch_comm_mask(env, max_comm_agents, d_mask_out, static_cast<cudaStream_t>(stream));
 }
 
+int mapf_env_comm_mask_packed(mapf_env *env, int32_t max_comm_agents, uint8_t *d_mask_out, uint8_t *d_bits_base,
+                              const int64_t *d_bits_rows, void *stream)
+{
+    REQUIRE_ENV(env);
+    MAPF_DRAIN(env, static_cast<cudaStream_t>(stream));
+    if (!d_bits_base || max_comm_agents < 1 || max_comm_agents > 3) {
+        mapf_set_error("mapf_env_comm_mask_packed: NULL buffer or max_comm_agents outside 1..3 (config.py:58)");
+        return MAPF_EINVAL;
+    }
+    return mapf_launch_comm_mask_packed(env, max_comm_agents, d_mask_out, d_bits_base, d_bits_rows, static_cast<cudaStream_t>(stream));
+}
+
 int mapf_env_get_state(mapf_env *env, uint8_t *d_map, uint8_t *d_pos, uint8_t *d_goals, int32_t *d_steps, uint8_t *d_navi,
                        void *stream)
 {
@@ -1372,6 +1417,53 @@ int mapf_replay_gather(const mapf_replay_view *view, const int64_t *d_idx, int64
     }
     if (batch == 0) return MAPF_OK;
     return mapf_launch_replay_gather(view, d_idx, batch, out, d_err, static_cast<cudaStream_t>(stream));
+}
+
+int mapf_obs_unpack(const uint8_t *d_bits_base, const int64_t *d_rows, int64_t count, int32_t num_agents, int32_t dtype,
+                    void *d_out, void *stream)
+{
+    if (count < 0 || (count > 0 && (!d_bits_base || !d_out)) || !aligned16(d_bits_base) || !aligned16(d_out)) {
+        mapf_set_error("mapf_obs_unpack: NULL buffer, negative count or a pointer not 16-byte aligned");
+        return MAPF_EINVAL;
+    }
+    if (num_agents < 1 || num_agents > MAPF_MAX_AGENTS || dtype < MAPF_DTYPE_U8 || dtype > MAPF_DTYPE_BF16 || count > 0x7fffffff) {
+        mapf_set_error("mapf_obs_unpack: num_agents outside 1..128, unknown dtype or count >= 2^31");
+        return MAPF_EINVAL;
+    }
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+        mapf_set_error("mapf_obs_unpack: no CUDA device (this library has no CPU fallback)");
+        return MAPF_ECUDA;
+    }
+    if (count == 0) return MAPF_OK;
+    return mapf_launch_obs_unpack(d_bits_base, d_rows, count, num_agents, dtype, d_out, static_cast<cudaStream_t>(stream));
+}
+
+int mapf_replay_gather_compact(const mapf_replay_view_compact *view, const int64_t *d_idx, int64_t batch,
+                               const mapf_replay_batch *out, int32_t *d_err, void *stream)
+{
+    if (!view || !out || batch < 0 || (batch > 0 && !d_idx)) {
+        mapf_set_error("mapf_replay_gather_compact: NULL argument");
+        return MAPF_EINVAL;
+    }
+    if (view->num_agents < 1 || view->num_agents > MAPF_MAX_AGENTS || view->max_steps < 1 || view->bt_steps < 1 ||
+        view->forward_steps < 1 || view->latent_dim < 1 || batch > 65535) {
+        mapf_set_error("mapf_replay_gather_compact: bad dimensions (batch <= 65535)");
+        return MAPF_EINVAL;
+    }
+    if (!view->obs_bits || !view->comm_bits || !view->hid_buf || !view->act_buf || !view->rew_buf || !view->done_buf ||
+        !view->size_buf || !out->obs || !out->comm_mask || !out->hidden || !out->action || !out->reward || !out->done ||
+        !out->steps || !out->bt_steps || !aligned16(view->obs_bits)) {
+        mapf_set_error("mapf_replay_gather_compact: NULL buffer or obs_bits not 16-byte aligned");
+        return MAPF_EINVAL;
+    }
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+        mapf_set_error("mapf_replay_gather_compact: no CUDA device (this library has no CPU fallback)");
+        return MAPF_ECUDA;
+    }
+    if (batch == 0) return MAPF_OK;
+    return mapf_launch_replay_gather_compact(view, d_idx, batch, out, d_err, static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

@@ -248,9 +248,11 @@ pregen_bfs_kernel(EnvDims d, const uint32_t *__restrict__ list, int min_count, u
 constexpr int kCommWarps = 4;
 
 // SIZED: only the n_e present agents take part; rows and columns of absent agents are 0
-template <bool SIZED>
+// PACKED: also writes the mask as packed rows (include/mapf_b200.h) at row bits_rows[e] (NULL: e) of `bits`; `out` is optional
+template <bool SIZED, bool PACKED = false>
 __device__ __forceinline__ void comm_mask_body(const EnvDims &d, const uint8_t *__restrict__ pos, int k_nearest, uint8_t *__restrict__ out,
-                                               const int tid, const uint8_t *sz_n = nullptr)
+                                               const int tid, const uint8_t *sz_n = nullptr, uint8_t *__restrict__ bits = nullptr,
+                                               const int64_t *__restrict__ bits_rows = nullptr)
 {
     __shared__ uint16_t s_pos[kCommWarps][MAPF_MAX_AGENTS];
     __shared__ uint32_t s_bits[kCommWarps][MAPF_MAX_AGENTS][MAPF_MAX_AGENTS / 32];
@@ -300,6 +302,16 @@ __device__ __forceinline__ void comm_mask_body(const EnvDims &d, const uint8_t *
         for (int w = 0; w < MAPF_MAX_AGENTS / 32; ++w) s_bits[warp][i][w] = row[w];
     }
     __syncwarp();
+    if constexpr (PACKED) {
+        // byte m of row i = bits 8m .. 8m+7 of the row (bits j >= N are 0)
+        const int CW = (N + 7) >> 3;
+        uint8_t *ob = bits + (size_t)(bits_rows ? bits_rows[e] : (int64_t)e) * N * CW;
+        for (int idx = lane; idx < N * CW; idx += 32) {
+            const int i = idx / CW, m = idx - i * CW;
+            ob[idx] = (uint8_t)(s_bits[warp][i][m >> 2] >> (8 * (m & 3)));
+        }
+        if (!out) return;
+    }
     uint8_t *o = out + (size_t)e * N * N;
     if ((N & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0) {
         // 16 mask bytes (16 consecutive j of one row) per lane and store: bits -> bool bytes as in the observation path
@@ -333,6 +345,14 @@ comm_mask_sized_kernel(EnvDims d, const uint8_t *__restrict__ pos, int k_nearest
                        const uint8_t *__restrict__ sz_n)
 {
     comm_mask_body<true>(d, pos, k_nearest, out, threadIdx.x, sz_n);
+}
+
+template <bool SIZED>
+__global__ void __launch_bounds__(kCommWarps * 32)
+comm_mask_packed_kernel(EnvDims d, const uint8_t *__restrict__ pos, int k_nearest, uint8_t *__restrict__ out,
+                        uint8_t *__restrict__ bits, const int64_t *__restrict__ bits_rows, const uint8_t *__restrict__ sz_n)
+{
+    comm_mask_body<SIZED, true>(d, pos, k_nearest, out, threadIdx.x, sz_n, bits, bits_rows);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -526,6 +546,15 @@ int mapf_launch_comm_mask(mapf_env *env, int k_nearest, uint8_t *d_out, cudaStre
     const int grid = (env->d.B + kCommWarps - 1) / kCommWarps;
     if (env->sz_n) comm_mask_sized_kernel<<<grid, kCommWarps * 32, 0, st>>>(env->d, env->pos, k_nearest, d_out, env->sz_n);
     else comm_mask_kernel<<<grid, kCommWarps * 32, 0, st>>>(env->d, env->pos, k_nearest, d_out);
+    MAPF_CUDA(cudaGetLastError());
+    return MAPF_OK;
+}
+
+int mapf_launch_comm_mask_packed(mapf_env *env, int k_nearest, uint8_t *d_out, uint8_t *d_bits, const int64_t *d_rows, cudaStream_t st)
+{
+    const int grid = (env->d.B + kCommWarps - 1) / kCommWarps;
+    if (env->sz_n) comm_mask_packed_kernel<true><<<grid, kCommWarps * 32, 0, st>>>(env->d, env->pos, k_nearest, d_out, d_bits, d_rows, env->sz_n);
+    else comm_mask_packed_kernel<false><<<grid, kCommWarps * 32, 0, st>>>(env->d, env->pos, k_nearest, d_out, d_bits, d_rows, nullptr);
     MAPF_CUDA(cudaGetLastError());
     return MAPF_OK;
 }

@@ -26,6 +26,20 @@ struct GatherParams {
 // two bool bytes (b0 at bits 0-7, b1 at bits 16-23) -> two fp16 (1.0 = 0x3C00)
 __device__ __forceinline__ uint32_t bools_to_half2(uint32_t spread) { return spread * 0x3C00u; }
 
+// the per-sample scalars of a gathered window (dense and compact views share these fields)
+template <typename View>
+__device__ __forceinline__ void gather_scalars(const View &v, const mapf_replay_batch &o, int32_t *err, const int64_t b,
+                                               const int64_t idx, const int64_t g, const int t, const int size, const int steps)
+{
+    if (t >= size && err) atomicOr(err, 1);  // the reference asserts local_idx < size (worker.py:120)
+    o.action[b] = v.act_buf[idx];                                               // :143
+    o.reward[b] = v.rew_buf[idx];                                               // :144
+    const bool done = (t == size - 1) && v.done_buf[g] != 0;                    // :145-148
+    o.done[b] = done ? 0x3C00 : 0;
+    o.steps[b] = __half_as_ushort(__int2half_rn(steps));                        // :171 HalfTensor(b_steps)
+    o.bt_steps[b] = min(t + 1, v.bt_steps);                                     // :150
+}
+
 __global__ void __launch_bounds__(256)
 replay_gather_kernel(const GatherParams p)
 {
@@ -54,15 +68,7 @@ replay_gather_kernel(const GatherParams p)
         } else {
             for (int k = threadIdx.x; k < HB; k += blockDim.x) dst[k] = src ? src[k] : (uint16_t)0;
         }
-        if (threadIdx.x == 0) {
-            if (t >= size && p.err) atomicOr(p.err, 1);  // the reference asserts local_idx < size (worker.py:120)
-            p.o.action[b] = v.act_buf[idx];                                               // :143
-            p.o.reward[b] = v.rew_buf[idx];                                               // :144
-            const bool done = (t == size - 1) && v.done_buf[g] != 0;                      // :145-148
-            p.o.done[b] = done ? 0x3C00 : 0;
-            p.o.steps[b] = __half_as_ushort(__int2half_rn(steps));                        // :171 HalfTensor(b_steps)
-            p.o.bt_steps[b] = min(t + 1, v.bt_steps);                                     // :150
-        }
+        if (threadIdx.x == 0) gather_scalars(v, p.o, p.err, b, idx, g, t, size, steps);
         return;
     }
 
@@ -114,7 +120,170 @@ replay_gather_kernel(const GatherParams p)
     }
 }
 
+// ---- packed observation frames (include/mapf_b200.h: 64-byte agent rows, element k = bit k) -> dense elements ----
+
+// one packed frame (N * 64 bytes, 16-byte aligned) into shared memory
+__device__ __forceinline__ void load_frame(uint8_t *s_frame, const uint8_t *src, const int N)
+{
+    for (int k = threadIdx.x; k < N * (MAPF_OBS_PACKED_BYTES_PER_AGENT / 16); k += blockDim.x)
+        reinterpret_cast<uint4 *>(s_frame)[k] = __ldg(reinterpret_cast<const uint4 *>(src) + k);
+}
+
+// elements e0 .. e0+7 of the frame's N * 486 (element e0 at bit 0); a group may run from one agent's row into the next
+__device__ __forceinline__ uint32_t frame_bits8(const uint8_t *s_frame, const int N, const int e0)
+{
+    const int a = e0 / MAPF_OBS_BYTES_PER_AGENT, k0 = e0 - a * MAPF_OBS_BYTES_PER_AGENT;
+    const uint8_t *r = s_frame + a * MAPF_OBS_PACKED_BYTES_PER_AGENT + (k0 >> 3);  // k0 <= 485: r[1] is byte 61 at most
+    uint32_t w = ((uint32_t)r[0] | ((uint32_t)r[1] << 8)) >> (k0 & 7);
+    const int n1 = MAPF_OBS_BYTES_PER_AGENT - k0;
+    if (n1 < 8) {
+        w &= (1u << n1) - 1u;  // the row's pad bits are no elements
+        if (a + 1 < N) w |= (uint32_t)s_frame[(a + 1) * MAPF_OBS_PACKED_BYTES_PER_AGENT] << n1;
+    }
+    return w & 0xffu;
+}
+
+// 4 bits -> 4 bool bytes (as the step kernel's expansion)
+__device__ __forceinline__ uint32_t expand4(uint32_t x) { return (x * 0x00204081u) & 0x01010101u; }
+
+// two bits (element 2q at bit 0) -> two 16-bit values ONE / 0, or two bytes 1 / 0 (ONE = 1)
+template <uint32_t ONE>
+__device__ __forceinline__ uint32_t bits2_to_pair(const uint32_t x)
+{
+    return ONE == 1 ? ((x & 1u) | ((x & 2u) << 7)) : ((x & 1u) | ((x & 2u) << 15)) * ONE;
+}
+
+// Expand a frame in shared memory (live) or zeros (!live) into FB = N * 486 consecutive output elements at dst.  ONE = 1:
+// u8 elements, else 16-bit elements whose 1.0 is ONE (fp16 0x3C00, bf16 0x3F80).  vec: dst is aligned for 8 elements per
+// store (FB % 8 == 0 and a 16-byte aligned base); else one store of two elements each (FB is even, an even element pair
+// never straddles two agents).
+template <uint32_t ONE>
+__device__ __forceinline__ void expand_frame(const uint8_t *s_frame, const int N, const bool live, void *dst, const bool vec)
+{
+    const int FB = N * MAPF_OBS_BYTES_PER_AGENT;
+    if (vec) {
+        for (int q = threadIdx.x; q < (FB >> 3); q += blockDim.x) {
+            const uint32_t w = live ? frame_bits8(s_frame, N, q << 3) : 0u;
+            if constexpr (ONE == 1) {
+                __stcs(reinterpret_cast<uint2 *>(dst) + q, make_uint2(expand4(w & 0xfu), expand4(w >> 4)));
+            } else {
+                __stcs(reinterpret_cast<uint4 *>(dst) + q, make_uint4(bits2_to_pair<ONE>(w), bits2_to_pair<ONE>(w >> 2),
+                                                                    bits2_to_pair<ONE>(w >> 4), bits2_to_pair<ONE>(w >> 6)));
+            }
+        }
+    } else {
+        for (int q = threadIdx.x; q < (FB >> 1); q += blockDim.x) {
+            uint32_t x = 0;
+            if (live) {
+                const int e0 = q << 1, a = e0 / MAPF_OBS_BYTES_PER_AGENT, k0 = e0 - a * MAPF_OBS_BYTES_PER_AGENT;
+                x = (s_frame[a * MAPF_OBS_PACKED_BYTES_PER_AGENT + (k0 >> 3)] >> (k0 & 7)) & 3u;
+            }
+            if constexpr (ONE == 1) reinterpret_cast<uint16_t *>(dst)[q] = (uint16_t)bits2_to_pair<1>(x);
+            else reinterpret_cast<uint32_t *>(dst)[q] = bits2_to_pair<ONE>(x);
+        }
+    }
+}
+
+template <uint32_t ONE>
+__global__ void __launch_bounds__(256)
+obs_unpack_kernel(const uint8_t *__restrict__ bits, const int64_t *__restrict__ rows, const int N, void *__restrict__ out)
+{
+    __shared__ __align__(16) uint8_t s_frame[MAPF_MAX_AGENTS * MAPF_OBS_PACKED_BYTES_PER_AGENT];
+    const int64_t f = blockIdx.x;
+    const int FB = N * MAPF_OBS_BYTES_PER_AGENT;
+    load_frame(s_frame, bits + (size_t)(rows ? rows[f] : f) * N * MAPF_OBS_PACKED_BYTES_PER_AGENT, N);
+    __syncthreads();
+    uint8_t *dst = reinterpret_cast<uint8_t *>(out) + (size_t)f * FB * (ONE == 1 ? 1 : 2);
+    expand_frame<ONE>(s_frame, N, true, dst, (FB & 7) == 0);
+}
+
+struct CompactGatherParams {
+    mapf_replay_view_compact v;
+    mapf_replay_batch o;
+    const int64_t *idx;
+    int32_t *err;
+};
+
+// replay_gather_kernel over a compact store: the same window, padding and scalars; the observation frame is expanded from
+// bits to fp16 (eight halves per 16-byte store), the comm mask from bits to bytes, and the one stored hidden vector of the
+// sample is written into each of its N rows
+__global__ void __launch_bounds__(256)
+replay_gather_compact_kernel(const CompactGatherParams p)
+{
+    __shared__ __align__(16) uint8_t s_frame[MAPF_MAX_AGENTS * MAPF_OBS_PACKED_BYTES_PER_AGENT];
+    const mapf_replay_view_compact &v = p.v;
+    const int W = v.bt_steps + v.forward_steps;
+    const int j = blockIdx.x;
+    const int64_t b = blockIdx.y;
+    const int64_t idx = p.idx[b];
+    const int64_t g = idx / v.max_steps;
+    const int t = (int)(idx - g * v.max_steps);
+    const int size = v.size_buf[g];
+    const int steps = min(v.forward_steps, size - t);
+    const int f0 = max(0, t + 1 - v.bt_steps);
+    const int len = t + 1 + steps - f0;
+    const int N = v.num_agents;
+
+    if (j == W) {
+        // the stored hidden vector of frame t - bt_steps in every agent's row, zeros while t < bt_steps
+        const int D = v.latent_dim;
+        uint16_t *dst = p.o.hidden + (size_t)b * N * D;
+        const uint16_t *src = t >= v.bt_steps ? v.hid_buf + (size_t)(idx - v.bt_steps) * D : nullptr;
+        if ((D & 7) == 0) {
+            const int D8 = D >> 3;
+            const uint4 *s4 = reinterpret_cast<const uint4 *>(src);
+            uint4 *d4 = reinterpret_cast<uint4 *>(dst);
+            for (int k = threadIdx.x; k < N * D8; k += blockDim.x) d4[k] = src ? __ldg(s4 + k % D8) : make_uint4(0, 0, 0, 0);
+        } else {
+            for (int k = threadIdx.x; k < N * D; k += blockDim.x) dst[k] = src ? src[k % D] : (uint16_t)0;
+        }
+        if (threadIdx.x == 0) gather_scalars(v, p.o, p.err, b, idx, g, t, size, steps);
+        return;
+    }
+
+    const bool live = j < len;
+    const int64_t row = g * (v.max_steps + 1) + f0 + j;
+    const int FB = N * MAPF_OBS_BYTES_PER_AGENT;
+    if (live) load_frame(s_frame, v.obs_bits + (size_t)row * N * MAPF_OBS_PACKED_BYTES_PER_AGENT, N);
+    __syncthreads();
+    expand_frame<0x3C00u>(s_frame, N, live, p.o.obs + ((size_t)b * W + j) * FB, (FB & 7) == 0);
+    // ---- communication mask frame: packed rows -> N * N bool bytes ----
+    const int CW = (N + 7) >> 3;
+    const uint8_t *src = v.comm_bits + (size_t)row * N * CW;
+    uint8_t *dst = p.o.comm_mask + ((size_t)b * W + j) * N * N;
+    for (int k = threadIdx.x; k < N * N; k += blockDim.x) {
+        const int i = k / N, c = k - i * N;
+        dst[k] = live ? (uint8_t)((__ldg(src + i * CW + (c >> 3)) >> (c & 7)) & 1u) : (uint8_t)0;
+    }
+}
+
 }  // namespace
+
+int mapf_launch_obs_unpack(const uint8_t *d_bits, const int64_t *d_rows, int64_t count, int N, int dtype, void *d_out,
+                           cudaStream_t st)
+{
+    switch (dtype) {
+        case MAPF_DTYPE_U8: obs_unpack_kernel<1u><<<(unsigned)count, 256, 0, st>>>(d_bits, d_rows, N, d_out); break;
+        case MAPF_DTYPE_F16: obs_unpack_kernel<0x3C00u><<<(unsigned)count, 256, 0, st>>>(d_bits, d_rows, N, d_out); break;
+        default: obs_unpack_kernel<0x3F80u><<<(unsigned)count, 256, 0, st>>>(d_bits, d_rows, N, d_out); break;
+    }
+    MAPF_CUDA(cudaGetLastError());
+    return MAPF_OK;
+}
+
+int mapf_launch_replay_gather_compact(const mapf_replay_view_compact *view, const int64_t *d_idx, int64_t batch,
+                                      const mapf_replay_batch *out, int32_t *d_err, cudaStream_t st)
+{
+    CompactGatherParams p;
+    p.v = *view;
+    p.o = *out;
+    p.idx = d_idx;
+    p.err = d_err;
+    const int W = view->bt_steps + view->forward_steps;
+    replay_gather_compact_kernel<<<dim3((unsigned)(W + 1), (unsigned)batch), 256, 0, st>>>(p);
+    MAPF_CUDA(cudaGetLastError());
+    return MAPF_OK;
+}
 
 int mapf_launch_replay_gather(const mapf_replay_view *view, const int64_t *d_idx, int64_t batch, const mapf_replay_batch *out,
                               int32_t *d_err, cudaStream_t st)

@@ -142,7 +142,9 @@ struct EnvRegs {
 // inside the handle's N x L layout.  Agents a >= n_e are absent: their actions are never read, they hold no cell, their
 // reward is 0 with code MAPF_RCODE_RESET and their 486-bit stream is zero.  A move outside l_e is a collision; the bitmap
 // and the heuristic maps are zero outside l_e, so the gather itself needs no clipping.
-template <int RW, int K, bool DO_STEP, bool DO_OBS = true, bool RESIDENT = false, bool SIZED = false>
+// PACKED (never RESIDENT): agent a's stream starts at bit 512 a (MAPF_OBS_PACKED_BYTES_PER_AGENT) and `head` is 0, so every
+// agent owns its 16 words: bits 486..511 are written as 0 and no word is shared with a neighbour.
+template <int RW, int K, bool DO_STEP, bool DO_OBS = true, bool RESIDENT = false, bool SIZED = false, bool PACKED = false>
 __device__ __forceinline__ void env_step_gather(const StepParams &p, const int e, const int lane, uint32_t *s_obst,
                                                 uint32_t *s_agent, uint32_t *s_bits, uint16_t *s_tgt, uint16_t *s_cell,
                                                 const int head, const uint64_t pol_keep, EnvRegs<K> &out,
@@ -514,8 +516,8 @@ __device__ __forceinline__ void env_step_gather(const StepParams &p, const int e
 #pragma unroll
         for (int k = 0; k < K; ++k) {
             const int a = k * 32 + lane;
-            // this agent's 486 bits start at stream bit (head + 486 a) = word f, bit o
-            const int gbit = head + MAPF_OBS_BYTES_PER_AGENT * a;
+            // this agent's 486 bits start at stream bit (head + 486 a) = word f, bit o  (512 a when PACKED)
+            const int gbit = PACKED ? 8 * MAPF_OBS_PACKED_BYTES_PER_AGENT * a : head + MAPF_OBS_BYTES_PER_AGENT * a;
             const int o = gbit & 31;
             uint32_t *S = s_bits + (gbit >> 5);
             uint32_t x0 = 0;
@@ -597,16 +599,16 @@ __device__ __forceinline__ void env_step_gather(const StepParams &p, const int e
                 // an absent agent's 486 bits are zero (words it shares with its neighbours: see below)
                 if (a < N) {
 #pragma unroll
-                    for (int m = 1; m < 16; ++m) S[m] = 0;
-                    if (((o + 485) >> 5) == 16) S[16] = 0;
+                    for (int m = PACKED ? 0 : 1; m < 16; ++m) S[m] = 0;
+                    if (!PACKED && ((o + 485) >> 5) == 16) S[16] = 0;
                 }
             }
             __syncwarp();
             // first word: shared with the previous agent's last word unless this agent starts a word
             bool streams = valid[k];
-            if constexpr (SIZED) streams = a < N;
+            if constexpr (SIZED && !PACKED) streams = a < N;
             if (streams) {
-                if (o == 0 || a == 0) S[0] = x0;
+                if (PACKED || o == 0 || a == 0) S[0] = x0;
                 else S[0] |= x0;
             }
             __syncwarp();
@@ -675,6 +677,20 @@ __device__ __forceinline__ void expand_store_block(const StepParams &p, uint8_t 
             const int g = (c << 4) + b;
             if (g >= head && g < total) obase[g] = (uint8_t)((s >> b) & 1u);
         }
+    }
+}
+
+// Store the env's packed frame (N * 64 bytes, already in stream order) with 16-byte streaming stores; obs_env is 16-byte
+// aligned.
+__device__ __forceinline__ void store_packed_block(uint8_t *obs_env, const int n_chunks, const uint32_t *s_bits, const int lane,
+                                                   const bool obs_policy, const uint64_t pol_stream)
+{
+    const uint4 *src = reinterpret_cast<const uint4 *>(s_bits);
+    uint4 *dst = reinterpret_cast<uint4 *>(obs_env);
+#pragma unroll 4
+    for (int c = lane; c < n_chunks; c += 32) {
+        if (obs_policy) stg_policy(dst + c, src[c], pol_stream);
+        else __stcs(dst + c, src[c]);
     }
 }
 

@@ -18,7 +18,8 @@ namespace {
 
 // ---- K1+K2: every warp steps an env, then expands and stores its own observation block.
 // (threadIdx.x is read by the kernel: the range its launch bounds give it is what lets the compiler form e with an OR)
-template <int RW, int K, bool DO_STEP, int WARPS, bool SIZED>
+// PACKED: the env's frame is N * 64 bytes of bits (MAPF_OBS_PACKED_BYTES_PER_AGENT), stored as it sits in shared memory.
+template <int RW, int K, bool DO_STEP, int WARPS, bool SIZED, bool PACKED = false>
 __device__ __forceinline__ void step_observe_body(const StepParams &p, uint32_t *smem, const int tid, const uint8_t *sz_n = nullptr,
                                                   const uint8_t *sz_l = nullptr)
 {
@@ -42,13 +43,14 @@ __device__ __forceinline__ void step_observe_body(const StepParams &p, uint32_t 
     __syncwarp();
 
     for (int e = p.env_begin + blockIdx.x * WARPS + warp; e < p.env_end; e += gridDim.x * WARPS) {
-        const size_t env_bytes = (size_t)N * MAPF_OBS_BYTES_PER_AGENT;
+        const size_t env_bytes = (size_t)N * (PACKED ? MAPF_OBS_PACKED_BYTES_PER_AGENT : MAPF_OBS_BYTES_PER_AGENT);
         uint8_t *obs_env = p.obs + (size_t)(p.obs_rows ? p.obs_rows[e] : (int64_t)e) * env_bytes;
-        const int head = (int)(reinterpret_cast<uintptr_t>(obs_env) & 15);  // bytes before the 16-B boundary
+        const int head = PACKED ? 0 : (int)(reinterpret_cast<uintptr_t>(obs_env) & 15);  // bytes before the 16-B boundary
         EnvRegs<K> r;
-        env_step_gather<RW, K, DO_STEP, true, false, SIZED>(p, e, lane, s_obst, s_agent, s_bits, s_tgt, s_cell, head, pol_keep, r,
-                                                            nullptr, nullptr, false, nullptr, sz_n, sz_l);
-        expand_store_block(p, obs_env, head, env_bytes, s_bits, lane, obs_policy, pol_stream);
+        env_step_gather<RW, K, DO_STEP, true, false, SIZED, PACKED>(p, e, lane, s_obst, s_agent, s_bits, s_tgt, s_cell, head, pol_keep,
+                                                                    r, nullptr, nullptr, false, nullptr, sz_n, sz_l);
+        if constexpr (PACKED) store_packed_block(obs_env, N * (MAPF_OBS_PACKED_BYTES_PER_AGENT / 16), s_bits, lane, obs_policy, pol_stream);
+        else expand_store_block(p, obs_env, head, env_bytes, s_bits, lane, obs_policy, pol_stream);
         __syncwarp();
         clear_agent_bits<RW, K>(s_agent, r);  // the agent bits this env set
     }
@@ -70,6 +72,16 @@ step_observe_sized_kernel(const StepParams p, const uint8_t *__restrict__ sz_n, 
 {
     extern __shared__ __align__(16) uint32_t smem[];
     step_observe_body<RW, K, DO_STEP, 4, true>(p, smem, threadIdx.x, sz_n, sz_l);
+}
+
+// the same writing packed frames (mapf_env_step_observe_packed / mapf_env_observe_packed), uniform and sized: separate
+// instantiations again, so the dense kernels above are unchanged
+template <int RW, int K, bool DO_STEP, int WARPS, int MINB, bool SIZED>
+__global__ void __launch_bounds__(WARPS * 32, MINB)
+step_observe_packed_kernel(const StepParams p, const uint8_t *__restrict__ sz_n, const uint8_t *__restrict__ sz_l)
+{
+    extern __shared__ __align__(16) uint32_t smem[];
+    step_observe_body<RW, K, DO_STEP, WARPS, SIZED, true>(p, smem, threadIdx.x, sz_n, sz_l);
 }
 
 // ---- K1 alone: Environment.step without the observation.  The host-buffer steps launch it ahead of the observe kernel so
@@ -216,6 +228,58 @@ int launch_step_rw(const mapf_env *env, StepParams &p, cudaStream_t st)
     return MAPF_EINVAL;
 }
 
+// Packed frames take the CTA shape the dense whole-batch launch takes for the same geometry (launch_step_rwk), so the two
+// compare at equal occupancy; a sized handle takes the shape of step_observe_sized_kernel.
+template <int RW, int K, bool DO_STEP, bool SIZED>
+int launch_packed_rwk(const mapf_env *env, StepParams &p, cudaStream_t st)
+{
+    constexpr bool hot1 = !SIZED && RW == 2 && K == 1, hot2 = !SIZED && K == 2 && DO_STEP && RW <= 2;
+    constexpr int WARPS = hot1 ? 8 : 4;
+    constexpr int MINB = hot1 ? 5 : (hot2 ? 8 : (SIZED || K > 1 ? 1 : 12));
+    auto kern = step_observe_packed_kernel<RW, K, DO_STEP, WARPS, MINB, SIZED>;
+    const size_t smem = (size_t)p.warp_smem_words * 4 * WARPS;
+    if (smem > 227 * 1024) {
+        mapf_set_error("map too large for the step kernel's shared memory");
+        return MAPF_EINVAL;
+    }
+    if (smem > 48 * 1024) MAPF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<(p.env_end - p.env_begin + WARPS - 1) / WARPS, WARPS * 32, smem, st>>>(p, env->sz_n, env->sz_l);
+    MAPF_CUDA(cudaGetLastError());
+    return MAPF_OK;
+}
+
+template <int RW, bool DO_STEP, bool SIZED>
+int launch_packed_rw(const mapf_env *env, StepParams &p, cudaStream_t st)
+{
+    switch (env->d.K) {
+        case 1: return launch_packed_rwk<RW, 1, DO_STEP, SIZED>(env, p, st);
+        case 2: return launch_packed_rwk<RW, 2, DO_STEP, SIZED>(env, p, st);
+        case 3: return launch_packed_rwk<RW, 3, DO_STEP, SIZED>(env, p, st);
+        case 4: return launch_packed_rwk<RW, 4, DO_STEP, SIZED>(env, p, st);
+    }
+    mapf_set_error("unsupported agent count");
+    return MAPF_EINVAL;
+}
+
+template <bool DO_STEP, bool SIZED>
+int launch_packed_sz(const mapf_env *env, StepParams &p, cudaStream_t st)
+{
+    switch (env->d.RW) {
+        case 1: return launch_packed_rw<1, DO_STEP, SIZED>(env, p, st);
+        case 2: return launch_packed_rw<2, DO_STEP, SIZED>(env, p, st);
+        case 3: return launch_packed_rw<3, DO_STEP, SIZED>(env, p, st);
+        case 4: return launch_packed_rw<4, DO_STEP, SIZED>(env, p, st);
+    }
+    mapf_set_error("unsupported map size");
+    return MAPF_EINVAL;
+}
+
+template <bool DO_STEP>
+int launch_packed(const mapf_env *env, StepParams &p, cudaStream_t st)
+{
+    return env->sz_n ? launch_packed_sz<DO_STEP, true>(env, p, st) : launch_packed_sz<DO_STEP, false>(env, p, st);
+}
+
 template <bool DO_STEP>
 int launch_step(const mapf_env *env, StepParams &p, cudaStream_t st)
 {
@@ -237,7 +301,7 @@ int mapf_step_tuning_generation() { return g_tuning_generation; }  // captured l
 int mapf_step_flags() { return tuning().flags | 0; }
 
 // Everything of StepParams that does not depend on the call: geometry, arena pointers, rewards, shared-memory layout.
-StepParams mapf_make_step_params(const mapf_env *env)
+StepParams mapf_make_step_params(const mapf_env *env, bool packed)
 {
     StepParams p{};
     const EnvDims &d = env->d;
@@ -252,9 +316,9 @@ StepParams mapf_make_step_params(const mapf_env *env)
     p.err = env->err;
     for (int i = 0; i < 5; ++i) p.r[i] = env->reward[i];
     p.obst_words = d.obst_stride;
-    // stream words: 15 head bits max + N*486 bits, +2 words of slack for the u16 tail read; the same
-    // buffer holds the L*L-byte occupancy grid of the step phase
-    const int stream_words = ((15 + d.N * MAPF_OBS_BYTES_PER_AGENT + 31) >> 5) + 2;
+    // stream words: 15 head bits max + N*486 bits, +2 words of slack for the u16 tail read (packed: 16 words per agent); the
+    // same buffer holds the L*L-byte occupancy grid of the step phase
+    const int stream_words = packed ? d.N * (MAPF_OBS_PACKED_BYTES_PER_AGENT / 4) : ((15 + d.N * MAPF_OBS_BYTES_PER_AGENT + 31) >> 5) + 2;
     // step-phase scratch in the same buffer: the L*L-byte occupancy grid, or (`RANKED` in mapf_step_device.cuh) the claim
     // bitmap + row ranks + rank -> agent table
     const int occ_words = MAPF_RANKED_LOOKUP(d.RW) ? ((((d.L * d.L + 127) >> 7) << 2) + ((d.R + 3) >> 2) + ((d.N + 3) >> 2)) : ((d.L * d.L + 3) >> 2);
@@ -362,4 +426,25 @@ int mapf_launch_observe(mapf_env *env, uint8_t *d_obs, const int64_t *d_obs_rows
     p.obs_rows = d_obs_rows;
     p.pos_out = d_pos;
     return launch_step<false>(env, p, st);
+}
+
+// packed frames (mapf_env_step_observe_packed / mapf_env_observe_packed): d_bits_base is 16-byte aligned, rows optional
+int mapf_launch_step_packed(mapf_env *env, const uint8_t *d_actions, uint8_t *d_bits, const int64_t *d_rows, const StepOut &out,
+                            cudaStream_t st)
+{
+    StepParams p = mapf_make_step_params(env, true);
+    p.actions = d_actions;
+    p.obs = d_bits;
+    p.obs_rows = d_rows;
+    fill_out(p, out);
+    return launch_packed<true>(env, p, st);
+}
+
+int mapf_launch_observe_packed(mapf_env *env, uint8_t *d_bits, const int64_t *d_rows, uint8_t *d_pos, cudaStream_t st)
+{
+    StepParams p = mapf_make_step_params(env, true);
+    p.obs = d_bits;
+    p.obs_rows = d_rows;
+    p.pos_out = d_pos;
+    return launch_packed<false>(env, p, st);
 }

@@ -9,6 +9,11 @@ of `obs_buf`.  `sample_batch` is two launches: the sum-tree descent (mapf_per_sa
 gather with bool->fp16 conversion (mapf_replay_gather); `update_priorities` is the fused stale-mask +
 tree update.  Return values follow the reference's tuple (worker.py:168-182) with CUDA tensors in
 place of CPU ones.
+
+`compact=True` keeps the same logical store in about a twelfth of the memory at 32 agents (DESIGN.md §3): observations
+and comm masks as packed bits (`obs_bits`, `comm_bits`, formats in `mapf_rl_b200.packed`) and one hidden vector per
+transition (`hid_buf` [max_steps*capacity, latent]; the reference writes agent 0's vector into every agent's row,
+buffer.py:148).  `gather` / `sample_batch` return exactly what the dense store returns for the same contents.
 """
 from __future__ import annotations
 
@@ -17,7 +22,7 @@ from typing import List, Optional
 
 import numpy as np
 
-from . import _native, config
+from . import _native, config, packed
 from .buffer import SumTree
 
 
@@ -30,7 +35,7 @@ class ReplayStore:
     def __init__(self, capacity: int, alpha=config.prioritized_replay_alpha, beta=config.prioritized_replay_beta,
                  max_num_agents: int = config.max_num_agents, device=None, max_steps: int = config.max_steps,
                  bt_steps: int = config.bt_steps, forward_steps: int = config.forward_steps,
-                 latent_dim: int = config.latent_dim):
+                 latent_dim: int = config.latent_dim, compact: bool = False):
         torch = _torch()
         if not torch.cuda.is_available():
             raise RuntimeError("mapf_rl_b200 needs a CUDA device: the replay kernels have no CPU fallback")
@@ -47,18 +52,42 @@ class ReplayStore:
         self.priority_tree = SumTree(self.capacity * self.max_steps, device=self.device)   # worker.py:27
         n, S, dev = self.max_num_agents, self.max_steps, self.device
         z = lambda shape, dt: torch.zeros(shape, dtype=dt, device=dev)
-        self.obs_buf = z(((S + 1) * capacity, n, *config.obs_shape), torch.uint8)          # worker.py:36
+        self.compact = bool(compact)
+        if self.compact:
+            self.obs_bits = z(((S + 1) * capacity, n, packed.OBS_BYTES), torch.uint8)
+            self.comm_bits = z(((S + 1) * capacity, n, packed.comm_bytes(n)), torch.uint8)
+            self.hid_buf = z((S * capacity, self.latent_dim), torch.float16)
+        else:
+            self.obs_buf = z(((S + 1) * capacity, n, *config.obs_shape), torch.uint8)      # worker.py:36
+            self.hid_buf = z((S * capacity, n, self.latent_dim), torch.float16)            # worker.py:39
+            self.comm_mask = z(((S + 1) * capacity, n, n), torch.uint8)                    # worker.py:42
         self.act_buf = z((S * capacity,), torch.uint8)                                     # worker.py:37
         self.rew_buf = z((S * capacity,), torch.float16)                                   # worker.py:38
-        self.hid_buf = z((S * capacity, n, self.latent_dim), torch.float16)                # worker.py:39
         self.done_buf = z((capacity,), torch.uint8)                                        # worker.py:40
         self.size_buf = z((capacity,), torch.int32)                                        # worker.py:41
-        self.comm_mask = z(((S + 1) * capacity, n, n), torch.uint8)                        # worker.py:42
         self._size_host = np.zeros(capacity, dtype=np.int64)
         self._err = z((1,), torch.int32)
 
     def __len__(self):
         return self.size
+
+    @staticmethod
+    def bytes_per_transition(num_agents: int, latent_dim: int = config.latent_dim, compact: bool = False) -> int:
+        """Device bytes one stored transition takes: its observation and comm-mask frame, hidden state, action and reward
+        (without the extra frame per episode slot, the per-slot done / size and the sum tree)."""
+        n = int(num_agents)
+        if compact:
+            frame = n * packed.OBS_BYTES + n * packed.comm_bytes(n) + 2 * int(latent_dim)
+        else:
+            frame = n * packed.OBS_ELEMS + n * n + 2 * n * int(latent_dim)
+        return frame + 1 + 2
+
+    @property
+    def nbytes(self) -> int:
+        """Device bytes of the store's buffers (without the sum tree, which is the same for both layouts)."""
+        bufs = ((self.obs_bits, self.comm_bits) if self.compact else (self.obs_buf, self.comm_mask)) + (
+            self.hid_buf, self.act_buf, self.rew_buf, self.done_buf, self.size_buf)
+        return sum(b.numel() * b.element_size() for b in bufs)
 
     def _stream(self):
         return C.c_void_p(_torch().cuda.current_stream(self.device).cuda_stream)
@@ -66,7 +95,10 @@ class ReplayStore:
     # -- GlobalBuffer.add (worker.py:68-104) ------------------------------------------------------
     def add(self, buffer_list: List):
         """buffer_list: tuples as returned by LocalBuffer.finish — actor_id 0, num_agents 1, map_len 2, obs_buf 3,
-        act_buf 4, rew_buf 5, hid_buf 6, td_errors 7, done 8, size 9, comm_mask 10 (worker.py:72)."""
+        act_buf 4, rew_buf 5, hid_buf 6, td_errors 7, done 8, size 9, comm_mask 10 (worker.py:72).
+        A compact store packs observations and comm masks on the host (agents >= num_agents get zero rows) and keeps one
+        hidden vector per transition: it raises ValueError if a transition's hidden rows differ, which the reference never
+        writes (buffer.py:148)."""
         torch = _torch()
         S = self.max_steps
         dev = self.device
@@ -74,7 +106,9 @@ class ReplayStore:
         def up(x, dt):
             return torch.as_tensor(np.ascontiguousarray(x)).to(device=dev, dtype=dt, non_blocking=True)
 
-        for buffer in buffer_list:
+        if self.compact:   # check every tuple before anything is written
+            hids = [packed.single_hidden(np.asarray(b[6], dtype=np.float16)[:int(b[9])]) for b in buffer_list]
+        for k, buffer in enumerate(buffer_list):
             n, size = int(buffer[1]), int(buffer[9])
             idxes = np.arange(self.ptr * S, (self.ptr + 1) * S, dtype=np.int64)            # worker.py:88
             start_idx = self.ptr * S
@@ -83,25 +117,41 @@ class ReplayStore:
             self.counter += size
             self.priority_tree.batch_update(idxes, np.asarray(buffer[7], dtype=np.float64) ** self.alpha)   # worker.py:94
             row0 = start_idx + self.ptr                                                    # = ptr * (S + 1)
-            self.obs_buf[row0:row0 + size + 1, :n] = up(buffer[3], torch.uint8)            # worker.py:96
+            if self.compact:
+                N = self.max_num_agents
+                obs = np.zeros((size + 1, N, *config.obs_shape), dtype=np.uint8)
+                obs[:, :n] = np.asarray(buffer[3])[:size + 1]
+                comm = np.zeros((size + 1, N, N), dtype=np.uint8)
+                comm[:, :n, :n] = np.asarray(buffer[10])[:size + 1]
+                self.obs_bits[row0:row0 + size + 1] = up(packed.pack_obs(obs), torch.uint8)
+                self.comm_bits[row0:row0 + size + 1] = up(packed.pack_comm(comm), torch.uint8)
+                self.hid_buf[start_idx:start_idx + size] = up(hids[k], torch.float16)
+            else:
+                self.obs_buf[row0:row0 + size + 1, :n] = up(buffer[3], torch.uint8)        # worker.py:96
+                self.hid_buf[start_idx:start_idx + size, :n] = up(np.asarray(buffer[6], dtype=np.float16), torch.float16)
+                self.comm_mask[row0:row0 + size + 1, :n, :n] = up(buffer[10], torch.uint8)  # worker.py:102
             self.act_buf[start_idx:start_idx + size] = up(buffer[4], torch.uint8)
             self.rew_buf[start_idx:start_idx + size] = up(np.asarray(buffer[5], dtype=np.float16), torch.float16)
-            self.hid_buf[start_idx:start_idx + size, :n] = up(np.asarray(buffer[6], dtype=np.float16), torch.float16)
             self.done_buf[self.ptr] = int(bool(buffer[8]))
             self.size_buf[self.ptr] = size
             self._size_host[self.ptr] = size
-            self.comm_mask[row0:row0 + size + 1, :n, :n] = up(buffer[10], torch.uint8)     # worker.py:102
             self.ptr = (self.ptr + 1) % self.capacity
 
     # -- direct-write path of a batched actor -------------------------------------------------------
     def obs_rows(self, slot: int, first_frame: int, count: int):
         """View of `count` consecutive observation frames of episode slot `slot` — the tensor a batched actor
-        passes as `out_obs` so the step kernel writes into the replay store with no copy."""
+        passes as `out_obs` (`out_bits`: packed rows of a compact store) so the step kernel writes into the replay store
+        with no copy."""
         row0 = slot * (self.max_steps + 1) + first_frame
-        return self.obs_buf[row0:row0 + count]
+        return (self.obs_bits if self.compact else self.obs_buf)[row0:row0 + count]
 
     # -- GlobalBuffer.sample_batch (worker.py:106-184) ------------------------------------------------
     def _view(self):
+        if self.compact:
+            return _native.ReplayViewCompact(self.obs_bits.data_ptr(), self.comm_bits.data_ptr(), self.hid_buf.data_ptr(),
+                                             self.act_buf.data_ptr(), self.rew_buf.data_ptr(), self.done_buf.data_ptr(),
+                                             self.size_buf.data_ptr(), self.max_num_agents, self.max_steps, self.bt_steps,
+                                             self.forward_steps, self.latent_dim)
         return _native.ReplayView(self.obs_buf.data_ptr(), self.comm_mask.data_ptr(), self.hid_buf.data_ptr(),
                                   self.act_buf.data_ptr(), self.rew_buf.data_ptr(), self.done_buf.data_ptr(),
                                   self.size_buf.data_ptr(), self.max_num_agents, self.max_steps, self.bt_steps,
@@ -120,8 +170,9 @@ class ReplayStore:
         view = self._view()
         batch = _native.ReplayBatch(*[out[k].data_ptr() for k in ("obs", "comm_mask", "hidden", "action", "reward", "done",
                                                                    "steps", "bt_steps")])
-        _native.check(self._lib.mapf_replay_gather(C.byref(view), C.c_void_p(idx.data_ptr()), B, C.byref(batch),
-                                                   C.c_void_p(self._err.data_ptr()), self._stream()))
+        gather = self._lib.mapf_replay_gather_compact if self.compact else self._lib.mapf_replay_gather
+        _native.check(gather(C.byref(view), C.c_void_p(idx.data_ptr()), B, C.byref(batch), C.c_void_p(self._err.data_ptr()),
+                             self._stream()))
         return out
 
     def sample_batch(self, batch_size: int, uniforms=None, check: bool = True):
