@@ -158,6 +158,14 @@ int mapf_env_observe_packed(mapf_env *env, uint8_t *d_bits_base, const int64_t *
 int mapf_obs_unpack(const uint8_t *d_bits_base, const int64_t *d_rows, int64_t count, int32_t num_agents, int32_t dtype,
                     void *d_out, void *stream);
 
+/* Packed frames -> the observations of PRESENT agents only, one row each (mapf_rl_b200/present.py): output row d_first[f] + a
+ * holds agent a < min(d_n[f], num_agents) of frame f (read at d_bits_base + d_rows[f] * N*64); every other row of
+ * [0, out_rows) is zeros.  d_rows i64[count], d_n u8[count], d_first i32[count] nondecreasing with
+ * d_first[f] + min(d_n[f], N) <= d_first[f + 1].  Output [out_rows, 6, 9, 9] of `dtype` as mapf_obs_unpack; d_bits_base and
+ * d_out must be 16-byte aligned. */
+int mapf_obs_unpack_present(const uint8_t *d_bits_base, const int64_t *d_rows, const uint8_t *d_n, const int32_t *d_first,
+                            int64_t count, int32_t num_agents, int64_t out_rows, int32_t dtype, void *d_out, void *stream);
+
 /* T lockstep steps with the actions already resident on the device: the loop `for t: obs, r, done, _ = env.step(a[t])`
  * of test.py:120-130 / worker.py:383-395 when the actions do not depend on the observations (replaying planner paths,
  * random-policy data generation, benchmarking).  Step t reads action slot t % action_slots, writes observation slot
@@ -473,6 +481,17 @@ typedef struct mapf_replay_view_compact {
  * zero padding, d_err).  view->obs_bits must be 16-byte aligned. */
 int mapf_replay_gather_compact(const mapf_replay_view_compact *view, const int64_t *d_idx, int64_t batch,
                                const mapf_replay_batch *out, int32_t *d_err, void *stream);
+
+/* mapf_replay_gather_compact with observations and hidden vectors in PRESENT-agent rows (mapf_rl_b200/present.py): sample b
+ * has n_b = min(d_agents[slot of b], num_agents) agents (d_agents u8[capacity], the store's per-slot agent count), and row
+ * d_first[b] + a (d_first i32[batch] nondecreasing, d_first[b] + n_b <= d_first[b + 1]) holds its agent a:
+ *   out->obs     fp16 [out_rows, W, 6, 9, 9]   the agent's window frames, zero padded as the compact gather pads them
+ *   out->hidden  fp16 [out_rows, latent_dim]    the sample's stored vector, zeros while t < bt_steps
+ * Rows of [0, out_rows) that hold no agent are zeros.  comm_mask, the scalars and d_err are those of
+ * mapf_replay_gather_compact.  W = bt_steps + forward_steps <= 64; obs_bits and out->obs must be 16-byte aligned. */
+int mapf_replay_gather_present(const mapf_replay_view_compact *view, const uint8_t *d_agents, const int64_t *d_idx,
+                               const int32_t *d_first, int64_t batch, int64_t out_rows, const mapf_replay_batch *out,
+                               int32_t *d_err, void *stream);
 
 /* ---- CBS expert / solvable-instance generator (search.py:58-442, test.py:23-79; SURVEY 8(f)4) -- HOST code ------------------
  * Conflict-based search over space-time A*: a collision-free set of paths of minimal sum of costs (search.py:17-21), as the

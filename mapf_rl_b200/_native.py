@@ -77,6 +77,7 @@ SIGNATURES = {
     "mapf_env_step_observe_packed": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mapf_env_observe_packed": (C.c_int, [_vp, _vp, _vp, _vp, _vp]),
     "mapf_obs_unpack": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _vp, _vp]),
+    "mapf_obs_unpack_present": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i32, _i64, _i32, _vp, _vp]),
     "mapf_env_rollout": (C.c_int, [_vp, _i32, _vp, _i32, _vp, _i32, _vp, _vp, _vp, _i32, _i32, _vp]),
     "mapf_env_rollout_ex": (C.c_int, [_vp, C.POINTER(RolloutIO), _vp]),
     "mapf_env_set_autoreset": (C.c_int, [_vp, _i32, _u64, _u64, _u64, _f32, _vp]),
@@ -109,6 +110,8 @@ SIGNATURES = {
                                      _vp, _vp, _vp]),
     "mapf_replay_gather": (C.c_int, [C.POINTER(ReplayView), _vp, _i64, C.POINTER(ReplayBatch), _vp, _vp]),
     "mapf_replay_gather_compact": (C.c_int, [C.POINTER(ReplayViewCompact), _vp, _i64, C.POINTER(ReplayBatch), _vp, _vp]),
+    "mapf_replay_gather_present": (C.c_int, [C.POINTER(ReplayViewCompact), _vp, _vp, _vp, _i64, _i64, C.POINTER(ReplayBatch),
+                                             _vp, _vp]),
     "mapf_actor_td": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _vp, _vp]),
     "mapf_actor_td_n": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i32, _i32, _f64, _vp, _vp]),
     "mapf_per_cycle": (C.c_int, [_vp, C.POINTER(PerCycleArgs), _vp]),

@@ -22,6 +22,10 @@ per step is the read of the B-byte "episode finished" mask.
 With a compact store (`ReplayStore(compact=True)`) the step kernel and the comm-mask kernel write packed rows, the current
 frames are unpacked from the store for the Q-network (mapf_obs_unpack), and one hidden vector is kept per transition; the
 store then holds exactly what the dense store would.
+With `present_only=True` the Q-network's encoder and input GRU run on present agents only (`present.py`): the present rows
+are rebuilt at every episode start (agent counts change only at resets), the current frames come in that layout
+(mapf_obs_unpack_present with a compact store, indexing obs_buf with a dense one), and the store receives what it receives
+without.  The results equal the padded path's up to floating-point reordering, not bit for bit.
 """
 from __future__ import annotations
 
@@ -33,6 +37,7 @@ from . import config
 from .batched import BatchedEnvironment
 from .buffer import actor_td_errors
 from .packed import unpack_obs
+from .present import PresentRows, unpack_obs_present
 from .replay import ReplayStore
 
 
@@ -45,10 +50,11 @@ class BatchedActor:
     def __init__(self, env: BatchedEnvironment, net, store: ReplayStore, epsilon=0.1, seed: int = 0,
                  density: Optional[float] = None, max_steps: int = config.max_steps,
                  on_step: Optional[Callable] = None, on_episode: Optional[Callable] = None,
-                 on_begin: Optional[Callable] = None, curriculum=None, curriculum_envs=None):
+                 on_begin: Optional[Callable] = None, curriculum=None, curriculum_envs=None, present_only: bool = False):
         """curriculum: a `Curriculum` whose levels the resets draw from (needs `BatchedEnvironment(..., sized=True)`);
         curriculum_envs: the environments whose finished episodes it counts (default: all; the reference counts its
-        low-epsilon actors, ids 10-15, only)."""
+        low-epsilon actors, ids 10-15, only); present_only: run the network's encoder on present agents only (`net.step`
+        takes `present=`)."""
         torch = _torch()
         assert curriculum is None or env.sized, "a curriculum needs a sized environment batch"
         self.curriculum = curriculum
@@ -76,6 +82,8 @@ class BatchedActor:
         self.transitions = 0
         self.resets = 0
         self._started = False
+        self.present_only = bool(present_only)
+        self.present = None
 
     # -- slots ---------------------------------------------------------------------------------------
     def _take_slots(self, count: int) -> np.ndarray:
@@ -122,6 +130,10 @@ class BatchedActor:
         slots = self._take_slots(len(ids))
         self._slot_host[ids] = slots
         self.slot[idt] = torch.as_tensor(slots, device=self.dev)
+        counts = self.env.sizes[0] if self.env.sized else torch.full((self.B,), self.N, dtype=torch.uint8, device=self.dev)
+        self.store.agents_buf[self.slot[idt]] = counts[idt]                     # num_agents of the slot's episode
+        if self.present_only:
+            self.present = PresentRows(counts, int(counts.sum(dtype=torch.int64).item()), self.N)
         self.t[idt] = 0
         # frame 0 of the new episodes (LocalBuffer.__init__: obs_buf[0] = init_obs, buffer.py:131); environments
         # in the middle of an episode rewrite the frame they already hold
@@ -144,14 +156,23 @@ class BatchedActor:
             self.net.reset()
             self._started = True
         rows = self._rows()
+        pr = self.present
         if st.compact:
-            obs = unpack_obs(st.obs_bits, rows)                                  # [B,N,6,9,9] current frames
+            if pr is not None:
+                obs = unpack_obs_present(st.obs_bits, rows, pr)                  # [M_pad,6,9,9] present agents' frames
+            else:
+                obs = unpack_obs(st.obs_bits, rows)                              # [B,N,6,9,9] current frames
             comm = env.comm_mask(out_bits=st.comm_bits, rows=rows)               # + the packed row of comm_buf[size]
         else:
             obs = st.obs_buf.index_select(0, rows)                               # [B,N,6,9,9] current frames
+            if pr is not None:
+                obs = pr.select(obs.flatten(0, 1))
             comm = env.comm_mask()                                               # model.py:196-208
             st.comm_mask.index_copy_(0, rows, comm)                              # comm_buf[size] = comm_mask, buffer.py:149
-        actions, q, hidden = self.net.step(obs, comm, reset_mask=self._pending_reset)
+        if pr is not None:
+            actions, q, hidden = self.net.step(obs, comm, reset_mask=self._pending_reset, present=pr)
+        else:
+            actions, q, hidden = self.net.step(obs, comm, reset_mask=self._pending_reset)
         self._pending_reset = None
         # only agent 0 explores (worker.py:380-382)
         explore = torch.rand(B, device=self.dev, generator=self.gen) < self.epsilon

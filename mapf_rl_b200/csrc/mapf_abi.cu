@@ -45,6 +45,10 @@ int mapf_launch_comm_mask_packed(mapf_env *, int, uint8_t *, uint8_t *, const in
 int mapf_launch_obs_unpack(const uint8_t *, const int64_t *, int64_t, int, int, void *, cudaStream_t);
 int mapf_launch_replay_gather_compact(const mapf_replay_view_compact *, const int64_t *, int64_t, const mapf_replay_batch *, int32_t *,
                                       cudaStream_t);
+int mapf_launch_obs_unpack_present(const uint8_t *, const int64_t *, const uint8_t *, const int32_t *, int64_t, int, int64_t, int,
+                                   void *, cudaStream_t);
+int mapf_launch_replay_gather_present(const mapf_replay_view_compact *, const uint8_t *, const int64_t *, const int32_t *, int64_t,
+                                      int64_t, const mapf_replay_batch *, int32_t *, cudaStream_t);
 
 static thread_local std::string g_last_error;
 
@@ -1464,6 +1468,59 @@ int mapf_replay_gather_compact(const mapf_replay_view_compact *view, const int64
     }
     if (batch == 0) return MAPF_OK;
     return mapf_launch_replay_gather_compact(view, d_idx, batch, out, d_err, static_cast<cudaStream_t>(stream));
+}
+
+int mapf_obs_unpack_present(const uint8_t *d_bits_base, const int64_t *d_rows, const uint8_t *d_n, const int32_t *d_first,
+                            int64_t count, int32_t num_agents, int64_t out_rows, int32_t dtype, void *d_out, void *stream)
+{
+    if (count < 0 || out_rows < 0 || (count > 0 && (!d_bits_base || !d_rows || !d_n || !d_first)) || (out_rows > 0 && !d_out) ||
+        !aligned16(d_bits_base) || !aligned16(d_out)) {
+        mapf_set_error("mapf_obs_unpack_present: NULL buffer, negative count or a pointer not 16-byte aligned");
+        return MAPF_EINVAL;
+    }
+    if (num_agents < 1 || num_agents > MAPF_MAX_AGENTS || dtype < MAPF_DTYPE_U8 || dtype > MAPF_DTYPE_BF16 || count > 0x7fffffff ||
+        out_rows > 0x7fffffff) {
+        mapf_set_error("mapf_obs_unpack_present: num_agents outside 1..128, unknown dtype, or count or out_rows >= 2^31");
+        return MAPF_EINVAL;
+    }
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+        mapf_set_error("mapf_obs_unpack_present: no CUDA device (this library has no CPU fallback)");
+        return MAPF_ECUDA;
+    }
+    if (out_rows == 0) return MAPF_OK;
+    return mapf_launch_obs_unpack_present(d_bits_base, d_rows, d_n, d_first, count, num_agents, out_rows, dtype, d_out,
+                                          static_cast<cudaStream_t>(stream));
+}
+
+int mapf_replay_gather_present(const mapf_replay_view_compact *view, const uint8_t *d_agents, const int64_t *d_idx,
+                               const int32_t *d_first, int64_t batch, int64_t out_rows, const mapf_replay_batch *out,
+                               int32_t *d_err, void *stream)
+{
+    if (!view || !out || batch < 0 || out_rows < 0 || (batch > 0 && (!d_idx || !d_first || !d_agents))) {
+        mapf_set_error("mapf_replay_gather_present: NULL argument");
+        return MAPF_EINVAL;
+    }
+    if (view->num_agents < 1 || view->num_agents > MAPF_MAX_AGENTS || view->max_steps < 1 || view->bt_steps < 1 ||
+        view->forward_steps < 1 || view->latent_dim < 1 || view->bt_steps + view->forward_steps > 64 || batch > 65535 ||
+        out_rows > 0x7fffffff) {
+        mapf_set_error("mapf_replay_gather_present: bad dimensions (bt_steps + forward_steps <= 64, batch <= 65535)");
+        return MAPF_EINVAL;
+    }
+    if (!view->obs_bits || !view->comm_bits || !view->hid_buf || !view->act_buf || !view->rew_buf || !view->done_buf ||
+        !view->size_buf || !out->obs || !out->comm_mask || !out->hidden || !out->action || !out->reward || !out->done ||
+        !out->steps || !out->bt_steps || !aligned16(view->obs_bits) || !aligned16(out->obs)) {
+        mapf_set_error("mapf_replay_gather_present: NULL buffer, or obs_bits or the obs output not 16-byte aligned");
+        return MAPF_EINVAL;
+    }
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+        mapf_set_error("mapf_replay_gather_present: no CUDA device (this library has no CPU fallback)");
+        return MAPF_ECUDA;
+    }
+    if (batch == 0 && out_rows == 0) return MAPF_OK;
+    return mapf_launch_replay_gather_present(view, d_agents, d_idx, d_first, batch, out_rows, out, d_err,
+                                             static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

@@ -257,7 +257,223 @@ replay_gather_compact_kernel(const CompactGatherParams p)
     }
 }
 
+// ---- present-agent rows (mapf_rl_b200/present.py): output row first[f] + a holds agent a < min(n[f], N) of frame f; first is
+// nondecreasing with first[f] + min(n[f], N) <= first[f + 1]; every other row up to out_rows is zeros ----
+
+// frame f of output row m (-1 if m lies before first[0]): the last f with first[f] <= m
+__device__ __forceinline__ int present_frame(const int32_t *__restrict__ first, const int count, const int64_t m)
+{
+    int lo = 0, hi = count;  // invariant: first[f] <= m for f < lo, first[f] > m for f >= hi
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (__ldg(first + mid) <= m) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo - 1;
+}
+
+// Output rows are 486 elements, so one row does not start on a 16-byte boundary, but eight consecutive rows do (8 * 486
+// elements, u8 or 16-bit).  A CTA therefore owns a run of rows (a multiple of 8), stages their packed 64-byte rows in shared
+// memory -- laid out like one frame of that many agents, so frame_bits8 reads across row ends -- and writes 16-byte streaming
+// stores that straddle rows.  Only the last run may be cut short by out_rows; its tail past the last whole 16 bytes is
+// written element by element.
+template <uint32_t ONE>
+__device__ __forceinline__ void expand_run(const uint8_t *s_rows, const int nrows, const int64_t elems, void *dst)
+{
+    constexpr int G = ONE == 1 ? 16 : 8;  // elements per 16-byte store
+    const int64_t groups = elems / G;
+    for (int64_t q = threadIdx.x; q < groups; q += blockDim.x) {
+        const int e0 = (int)q * G;
+        const uint32_t w = frame_bits8(s_rows, nrows, e0);
+        if constexpr (ONE == 1) {
+            const uint32_t w2 = frame_bits8(s_rows, nrows, e0 + 8);
+            __stcs(reinterpret_cast<uint4 *>(dst) + q,
+                   make_uint4(expand4(w & 0xfu), expand4(w >> 4), expand4(w2 & 0xfu), expand4(w2 >> 4)));
+        } else {
+            __stcs(reinterpret_cast<uint4 *>(dst) + q, make_uint4(bits2_to_pair<ONE>(w), bits2_to_pair<ONE>(w >> 2),
+                                                                bits2_to_pair<ONE>(w >> 4), bits2_to_pair<ONE>(w >> 6)));
+        }
+    }
+    if (threadIdx.x == 0) {
+        for (int64_t e = groups * G; e < elems; ++e) {
+            const int a = (int)(e / MAPF_OBS_BYTES_PER_AGENT), k = (int)(e - (int64_t)a * MAPF_OBS_BYTES_PER_AGENT);
+            const uint32_t bit = (s_rows[a * MAPF_OBS_PACKED_BYTES_PER_AGENT + (k >> 3)] >> (k & 7)) & 1u;
+            if constexpr (ONE == 1) reinterpret_cast<uint8_t *>(dst)[e] = (uint8_t)bit;
+            else reinterpret_cast<uint16_t *>(dst)[e] = (uint16_t)(bit * ONE);
+        }
+    }
+}
+
+constexpr int kUnpackRunRows = 32;  // output rows per CTA of obs_unpack_present_kernel
+
+template <uint32_t ONE>
+__global__ void __launch_bounds__(256)
+obs_unpack_present_kernel(const uint8_t *__restrict__ bits, const int64_t *__restrict__ rows, const uint8_t *__restrict__ n,
+                          const int32_t *__restrict__ first, const int count, const int N, const int64_t out_rows,
+                          void *__restrict__ out)
+{
+    __shared__ __align__(16) uint8_t s_rows[kUnpackRunRows * MAPF_OBS_PACKED_BYTES_PER_AGENT];
+    const int64_t r0 = (int64_t)blockIdx.x * kUnpackRunRows;
+    const int nrows = (int)min((int64_t)kUnpackRunRows, out_rows - r0);
+    // four threads per row, one 16-byte quarter each
+    for (int k = threadIdx.x; k < kUnpackRunRows * 4; k += blockDim.x) {
+        const int i = k >> 2;
+        uint4 x = make_uint4(0, 0, 0, 0);
+        if (i < nrows) {
+            const int64_t m = r0 + i;
+            const int f = present_frame(first, count, m);
+            if (f >= 0) {
+                const int64_t a = m - first[f];
+                if (a < min((int)n[f], N))
+                    x = __ldg(reinterpret_cast<const uint4 *>(bits + ((size_t)rows[f] * N + a) * MAPF_OBS_PACKED_BYTES_PER_AGENT) + (k & 3));
+            }
+        }
+        reinterpret_cast<uint4 *>(s_rows)[k] = x;
+    }
+    __syncthreads();
+    uint8_t *dst = reinterpret_cast<uint8_t *>(out) + (size_t)r0 * MAPF_OBS_BYTES_PER_AGENT * (ONE == 1 ? 1 : 2);
+    expand_run<ONE>(s_rows, kUnpackRunRows, (int64_t)nrows * MAPF_OBS_BYTES_PER_AGENT, dst);
+}
+
+constexpr int kGatherRunRows = 8;  // output rows per observation CTA of replay_gather_present_kernel
+constexpr int kGatherMaxW = 64;    // window frames the staging buffer holds (bt_steps + forward_steps, checked on the host)
+
+struct PresentGatherParams {
+    mapf_replay_view_compact v;
+    mapf_replay_batch o;  // obs [out_rows, W, 6, 9, 9] and hidden [out_rows, latent] in present rows
+    const uint8_t *agents;
+    const int64_t *idx;
+    const int32_t *first;
+    int32_t *err;
+    int batch;
+    int64_t out_rows;
+    int runs;  // CTAs [0, runs) write observation and hidden rows, CTA runs + b the comm mask and scalars of sample b
+};
+
+// replay_gather_compact_kernel's window, padding, error latch and scalars, with observations and hidden vectors in present
+// rows: row first[b] + a is agent a < n_b of sample b, n_b = agents[slot of b] (clamped to N)
+__global__ void __launch_bounds__(256)
+replay_gather_present_kernel(const PresentGatherParams p)
+{
+    __shared__ __align__(16) uint8_t s_rows[kGatherRunRows * kGatherMaxW * MAPF_OBS_PACKED_BYTES_PER_AGENT];
+    __shared__ int64_t s_src[kGatherRunRows];  // leaf of the row's sample, -1: zero row
+    __shared__ int s_a[kGatherRunRows], s_f0[kGatherRunRows], s_len[kGatherRunRows];
+    const mapf_replay_view_compact &v = p.v;
+    const int W = v.bt_steps + v.forward_steps;
+    const int N = v.num_agents;
+
+    if ((int)blockIdx.x >= p.runs) {
+        const int64_t b = blockIdx.x - p.runs;
+        const int64_t idx = p.idx[b];
+        const int64_t g = idx / v.max_steps;
+        const int t = (int)(idx - g * v.max_steps);
+        const int size = v.size_buf[g];
+        const int steps = min(v.forward_steps, size - t);
+        const int f0 = max(0, t + 1 - v.bt_steps);
+        const int len = t + 1 + steps - f0;
+        if (threadIdx.x == 0) gather_scalars(v, p.o, p.err, b, idx, g, t, size, steps);
+        const int CW = (N + 7) >> 3;
+        for (int j = 0; j < W; ++j) {
+            const bool live = j < len;
+            const uint8_t *src = v.comm_bits + (size_t)(g * (v.max_steps + 1) + f0 + j) * N * CW;
+            uint8_t *dst = p.o.comm_mask + ((size_t)b * W + j) * N * N;
+            for (int k = threadIdx.x; k < N * N; k += blockDim.x) {
+                const int i = k / N, c = k - i * N;
+                dst[k] = live ? (uint8_t)((__ldg(src + i * CW + (c >> 3)) >> (c & 7)) & 1u) : (uint8_t)0;
+            }
+        }
+        return;
+    }
+
+    const int64_t r0 = (int64_t)blockIdx.x * kGatherRunRows;
+    const int nrows = (int)min((int64_t)kGatherRunRows, p.out_rows - r0);
+    if (threadIdx.x < kGatherRunRows) {
+        const int i = threadIdx.x;
+        int64_t src = -1;
+        int a = 0, f0 = 0, len = 0;
+        if (i < nrows) {
+            const int64_t m = r0 + i;
+            const int b = present_frame(p.first, p.batch, m);
+            if (b >= 0) {
+                const int64_t idx = p.idx[b];
+                const int64_t g = idx / v.max_steps;
+                a = (int)(m - p.first[b]);
+                if (a < min((int)p.agents[g], N)) {
+                    const int t = (int)(idx - g * v.max_steps);
+                    const int steps = min(v.forward_steps, v.size_buf[g] - t);
+                    f0 = max(0, t + 1 - v.bt_steps);
+                    len = t + 1 + steps - f0;
+                    src = idx;
+                }
+            }
+        }
+        s_src[i] = src;
+        s_a[i] = a;
+        s_f0[i] = f0;
+        s_len[i] = len;
+    }
+    __syncthreads();
+    // packed rows [row][frame][64], four threads per 64 bytes
+    for (int k = threadIdx.x; k < kGatherRunRows * W * 4; k += blockDim.x) {
+        const int i = k / (W * 4), j = (k >> 2) - i * W;
+        uint4 x = make_uint4(0, 0, 0, 0);
+        const int64_t idx = s_src[i];
+        if (idx >= 0 && j < s_len[i]) {
+            const int64_t g = idx / v.max_steps;
+            const int64_t row = g * (v.max_steps + 1) + s_f0[i] + j;
+            x = __ldg(reinterpret_cast<const uint4 *>(v.obs_bits + ((size_t)row * N + s_a[i]) * MAPF_OBS_PACKED_BYTES_PER_AGENT) + (k & 3));
+        }
+        reinterpret_cast<uint4 *>(s_rows)[k] = x;
+    }
+    __syncthreads();
+    expand_run<0x3C00u>(s_rows, kGatherRunRows * W, (int64_t)nrows * W * MAPF_OBS_BYTES_PER_AGENT,
+                        p.o.obs + (size_t)r0 * W * MAPF_OBS_BYTES_PER_AGENT);
+    // hidden: the sample's stored vector of frame t - bt_steps, zeros while t < bt_steps and in zero rows
+    const int D = v.latent_dim;
+    for (int k = threadIdx.x; k < nrows * D; k += blockDim.x) {
+        const int i = k / D, c = k - i * D;
+        const int64_t idx = s_src[i];
+        const bool has = idx >= 0 && idx - (idx / v.max_steps) * v.max_steps >= v.bt_steps;
+        p.o.hidden[(size_t)(r0 + i) * D + c] = has ? v.hid_buf[(size_t)(idx - v.bt_steps) * D + c] : (uint16_t)0;
+    }
+}
+
 }  // namespace
+
+int mapf_launch_obs_unpack_present(const uint8_t *d_bits, const int64_t *d_rows, const uint8_t *d_n, const int32_t *d_first,
+                                   int64_t count, int N, int64_t out_rows, int dtype, void *d_out, cudaStream_t st)
+{
+    const unsigned grid = (unsigned)((out_rows + kUnpackRunRows - 1) / kUnpackRunRows);
+    const int c = (int)count;
+    switch (dtype) {
+        case MAPF_DTYPE_U8: obs_unpack_present_kernel<1u><<<grid, 256, 0, st>>>(d_bits, d_rows, d_n, d_first, c, N, out_rows, d_out); break;
+        case MAPF_DTYPE_F16:
+            obs_unpack_present_kernel<0x3C00u><<<grid, 256, 0, st>>>(d_bits, d_rows, d_n, d_first, c, N, out_rows, d_out);
+            break;
+        default: obs_unpack_present_kernel<0x3F80u><<<grid, 256, 0, st>>>(d_bits, d_rows, d_n, d_first, c, N, out_rows, d_out); break;
+    }
+    MAPF_CUDA(cudaGetLastError());
+    return MAPF_OK;
+}
+
+int mapf_launch_replay_gather_present(const mapf_replay_view_compact *view, const uint8_t *d_agents, const int64_t *d_idx,
+                                      const int32_t *d_first, int64_t batch, int64_t out_rows, const mapf_replay_batch *out,
+                                      int32_t *d_err, cudaStream_t st)
+{
+    PresentGatherParams p;
+    p.v = *view;
+    p.o = *out;
+    p.agents = d_agents;
+    p.idx = d_idx;
+    p.first = d_first;
+    p.err = d_err;
+    p.batch = (int)batch;
+    p.out_rows = out_rows;
+    p.runs = (int)((out_rows + kGatherRunRows - 1) / kGatherRunRows);
+    replay_gather_present_kernel<<<(unsigned)(p.runs + batch), 256, 0, st>>>(p);
+    MAPF_CUDA(cudaGetLastError());
+    return MAPF_OK;
+}
 
 int mapf_launch_obs_unpack(const uint8_t *d_bits, const int64_t *d_rows, int64_t count, int N, int dtype, void *d_out,
                            cudaStream_t st)

@@ -14,6 +14,10 @@ the device and the cycle has no host synchronisation (the only `.item()` calls a
 precision: the reference runs fp16 autocast with a GradScaler (worker.py:283,316-323); on a B200 the same region runs under
 bf16 autocast, which needs no loss scaling.  With more than one rank the gradients are averaged with ONE NCCL all-reduce of
 the flattened 2.05 M fp32 gradients (8.2 MB) per update -- the only collective of the whole package.
+
+`present_only=True` gathers each batch in present-agent rows (`ReplayStore.gather(idx, present=True)`) and runs both
+bootstraps with the encoder on those rows only.  Sizing that batch reads its row count on the host when it is gathered, so the
+host waits for update k's sampling before it can enqueue update k + 1 (DESIGN.md §4 measures what that costs).
 """
 from __future__ import annotations
 
@@ -32,7 +36,7 @@ def _torch():
 class BatchedLearner:
     def __init__(self, model, store: ReplayStore, batch_size: int = config.batch_size, lr: float = 1e-4, gamma: float = 0.99,
                  grad_clip: float = 40.0, target_update_freq: int = 2500, autocast_dtype=None, allreduce: bool = False,
-                 seed: int = 0):
+                 seed: int = 0, present_only: bool = False):
         torch = _torch()
         self.model, self.store, self.batch_size = model, store, int(batch_size)
         self.dev = store.device
@@ -48,6 +52,7 @@ class BatchedLearner:
         self.gen.manual_seed(seed)
         self.counter = 0
         self.loss = None
+        self.present_only = bool(present_only)
         # (idx int64[B], weights f32[B], old_ptr, gathered batch) drawn by the previous cycle.  The window gather runs right
         # after the draw -- the reference's sample_batch assembles the batch under the buffer lock at sampling time,
         # worker.py:112-184 -- so an episode slot the actor evicts between two updates cannot tear the batch; its priorities
@@ -59,7 +64,7 @@ class BatchedLearner:
         torch = _torch()
         u = torch.rand(self.batch_size, dtype=torch.float64, device=self.dev, generator=self.gen)
         out = self.store.priority_tree.cycle(sample_size=self.batch_size, uniforms=u, beta=self.store.beta)
-        self._next = (out["idx"], out["weights"], self.store.ptr, self.store.gather(out["idx"]))
+        self._next = (out["idx"], out["weights"], self.store.ptr, self.store.gather(out["idx"], present=self.present_only))
 
     @staticmethod
     def huber(td, kappa: float = 1.0):   # worker.py:341-344
@@ -86,15 +91,15 @@ class BatchedLearner:
         if self._next is None:
             self._first_sample()
         idx, weights, old_ptr, b = self._next                               # batch assembled at sampling time (worker.py:118-162)
-        obs, comm, hidden = b["obs"], b["comm_mask"], b["hidden"]
+        obs, comm, hidden, pr = b["obs"], b["comm_mask"], b["hidden"], b.get("present")
         action = b["action"].unsqueeze(1)
         reward, done, steps = b["reward"].float().unsqueeze(1), b["done"].float().unsqueeze(1), b["steps"].float().unsqueeze(1)
         bt = b["bt_steps"]
         next_bt = bt + b["steps"].long()                                    # worker.py:296-297
         with torch.autocast("cuda", dtype=self.autocast_dtype):
             with torch.no_grad():
-                q_tgt_all = self.tar_model.bootstrap(obs, next_bt, hidden, comm).float()                      # :302
-            q_all = self.model.bootstrap(obs[:, :-fwd], bt, hidden, comm[:, :-fwd]).float()                  # :304
+                q_tgt_all = self.tar_model.bootstrap(obs, next_bt, hidden, comm, present=pr).float()          # :302
+            q_all = self.model.bootstrap(obs[:, :-fwd], bt, hidden, comm[:, :-fwd], present=pr).float()      # :304
         q_ = (1.0 - done) * q_tgt_all.max(1, keepdim=True)[0]
         td = q_all.gather(1, action) - (reward + torch.pow(self.gamma, steps) * q_)                           # :306
         loss = (weights.unsqueeze(1) * self.huber(td)).mean()                                                # :310
@@ -112,7 +117,7 @@ class BatchedLearner:
                         steps=steps.reshape(-1).contiguous(), idx=idx),
             sample_size=B, uniforms=u, beta=st.beta, old_ptr=old_ptr, ptr=st.ptr, slot_steps=st.max_steps, gamma=self.gamma,
             alpha=st.alpha)
-        self._next = (out["idx"], out["weights"], st.ptr, st.gather(out["idx"]))
+        self._next = (out["idx"], out["weights"], st.ptr, st.gather(out["idx"], present=self.present_only))
         self.counter += 1
         if self.counter % self.target_update_freq == 0:                                                      # :336-337
             self.tar_model.load_state_dict(self.model.state_dict())

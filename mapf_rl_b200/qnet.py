@@ -103,41 +103,62 @@ class Network(nn.Module):
         return self.state(hidden) + adv - adv.mean(-1, keepdim=True)   # model.py:216-219
 
     @torch.no_grad()
-    def step(self, obs, comm_mask, reset_mask=None):
+    def step(self, obs, comm_mask, reset_mask=None, present=None):
         """obs uint8/float [B,N,6,9,9], comm_mask uint8/bool [B,N,N] (BatchedEnvironment.comm_mask),
         reset_mask bool [B] (optional): environments whose recurrent state restarts (Network.reset, model.py:224).
-        -> (actions int64[B,N], q [B,N,5], hidden [B,N,256]); the recurrent state is kept in self.hidden."""
-        B, N = obs.shape[:2]
+        -> (actions int64[B,N], q [B,N,5], hidden [B,N,256]); the recurrent state is kept in self.hidden.
+        present (`present.PresentRows`): obs is [M_pad,6,9,9] in present rows; the encoder and the input GRU run on those rows
+        only, the comm block and the head on the padded [B,N] layout, and absent agents' hidden state, q and actions are 0."""
+        B, N = comm_mask.shape[:2]
         p = next(self.parameters())
-        latent = self.obs_encoder(obs.reshape(B * N, *obs.shape[2:]).to(p.dtype))
+        x = obs if present is not None else obs.reshape(B * N, *obs.shape[2:])
+        latent = self.obs_encoder(x.to(p.dtype))
         if self.hidden is None or self.hidden.shape[0] != B * N:
             self.hidden = torch.zeros(B * N, self.latent_dim, dtype=p.dtype, device=p.device)   # GRUCell(x) == GRUCell(x, 0)
         elif reset_mask is not None:
             keep = (~reset_mask.bool()).to(p.dtype).repeat_interleave(N).unsqueeze(1)
             self.hidden = self.hidden * keep
-        hidden = self.recurrent(latent, self.hidden).view(B, N, self.latent_dim)
+        if present is None:
+            hidden = self.recurrent(latent, self.hidden).view(B, N, self.latent_dim)
+        else:
+            h = self.recurrent(latent[:present.M], present.gather(self.hidden))
+            hidden = present.scatter(h).view(B, N, self.latent_dim)
         hidden = self.comm(hidden, comm_mask.bool())
         self.hidden = hidden.reshape(B * N, self.latent_dim)
         q = self._q(hidden)
+        if present is not None:
+            q = torch.where(present.mask.unsqueeze(-1), q, torch.zeros_like(q))
         return q.argmax(-1), q, hidden
 
     def reset(self):
         self.hidden = None
 
-    def bootstrap(self, obs, steps, hidden, comm_mask):
+    def bootstrap(self, obs, steps, hidden, comm_mask, present=None):
         """model.py:227-263 for any batch size: obs [B,T,N,6,9,9], steps int64[B] (1-based frame whose hidden is
-        read out), hidden [B*N,256], comm_mask bool [B,T,N,N] -> q of agent 0, [B,5]."""
-        B, T, N = obs.shape[:3]
+        read out), hidden [B*N,256], comm_mask bool [B,T,N,N] -> q of agent 0, [B,5].
+        present (`present.PresentRows`): obs [M_pad,T,6,9,9] and hidden [M_pad,256] in present rows
+        (`ReplayStore.gather(idx, present=True)`); the encoder and the input GRU run on those rows, the comm block on the
+        padded layout of each frame."""
+        B, T, N = comm_mask.shape[:3]
         p = next(self.parameters())
-        x = obs.transpose(1, 2).contiguous().view(-1, *obs.shape[3:]).to(p.dtype)
-        latent = self.obs_encoder(x).view(B * N, T, 16 * 7 * 7).transpose(0, 1)
-        hidden = hidden.to(p.dtype)
+        if present is None:
+            x = obs.transpose(1, 2).contiguous().view(-1, *obs.shape[3:]).to(p.dtype)
+            latent = self.obs_encoder(x).view(B * N, T, 16 * 7 * 7).transpose(0, 1)
+            hidden = hidden.to(p.dtype)
+        else:
+            latent = self.obs_encoder(obs.reshape(-1, *obs.shape[2:]).to(p.dtype)).view(-1, T, 16 * 7 * 7)
+            latent = latent[:present.M].transpose(0, 1)
+            hidden = hidden[:present.M].to(p.dtype)
         buf = []
         for i in range(T):
-            hidden = self.recurrent(latent[i].to(hidden.dtype), hidden).view(B, N, self.latent_dim)
-            hidden = self.comm(hidden, comm_mask[:, i].bool())
+            hidden = self.recurrent(latent[i].to(hidden.dtype), hidden)
+            if present is not None:
+                hidden = present.scatter(hidden)
+            hidden = self.comm(hidden.view(B, N, self.latent_dim), comm_mask[:, i].bool())
             buf.append(hidden[:, 0])
             hidden = hidden.reshape(B * N, self.latent_dim)
+            if present is not None:
+                hidden = present.gather(hidden)
         buf = torch.stack(buf).transpose(0, 1)
         h = buf[torch.arange(B, device=buf.device), steps - 1]
         return self._q(h)

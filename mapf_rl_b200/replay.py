@@ -23,6 +23,7 @@ from typing import List, Optional
 import numpy as np
 
 from . import _native, config, packed
+from .present import PresentRows
 from .buffer import SumTree
 
 
@@ -65,6 +66,9 @@ class ReplayStore:
         self.rew_buf = z((S * capacity,), torch.float16)                                   # worker.py:38
         self.done_buf = z((capacity,), torch.uint8)                                        # worker.py:40
         self.size_buf = z((capacity,), torch.int32)                                        # worker.py:41
+        # agents of each slot's episode (the tuple's num_agents, worker.py:72); N until written, so an unannotated slot reads as
+        # padded.  gather(present=True) lays its rows out by it.
+        self.agents_buf = torch.full((capacity,), n, dtype=torch.uint8, device=dev)
         self._size_host = np.zeros(capacity, dtype=np.int64)
         self._err = z((1,), torch.int32)
 
@@ -86,7 +90,7 @@ class ReplayStore:
     def nbytes(self) -> int:
         """Device bytes of the store's buffers (without the sum tree, which is the same for both layouts)."""
         bufs = ((self.obs_bits, self.comm_bits) if self.compact else (self.obs_buf, self.comm_mask)) + (
-            self.hid_buf, self.act_buf, self.rew_buf, self.done_buf, self.size_buf)
+            self.hid_buf, self.act_buf, self.rew_buf, self.done_buf, self.size_buf, self.agents_buf)
         return sum(b.numel() * b.element_size() for b in bufs)
 
     def _stream(self):
@@ -98,10 +102,13 @@ class ReplayStore:
         act_buf 4, rew_buf 5, hid_buf 6, td_errors 7, done 8, size 9, comm_mask 10 (worker.py:72).
         A compact store packs observations and comm masks on the host (agents >= num_agents get zero rows) and keeps one
         hidden vector per transition: it raises ValueError if a transition's hidden rows differ, which the reference never
-        writes (buffer.py:148)."""
+        writes (buffer.py:148).  num_agents goes to `agents_buf`; it raises ValueError outside 1..max_num_agents."""
         torch = _torch()
         S = self.max_steps
         dev = self.device
+        for b in buffer_list:
+            if not 1 <= int(b[1]) <= self.max_num_agents:
+                raise ValueError(f"num_agents {int(b[1])} outside 1..{self.max_num_agents}")
 
         def up(x, dt):
             return torch.as_tensor(np.ascontiguousarray(x)).to(device=dev, dtype=dt, non_blocking=True)
@@ -134,6 +141,7 @@ class ReplayStore:
             self.rew_buf[start_idx:start_idx + size] = up(np.asarray(buffer[5], dtype=np.float16), torch.float16)
             self.done_buf[self.ptr] = int(bool(buffer[8]))
             self.size_buf[self.ptr] = size
+            self.agents_buf[self.ptr] = n
             self._size_host[self.ptr] = size
             self.ptr = (self.ptr + 1) % self.capacity
 
@@ -157,10 +165,15 @@ class ReplayStore:
                                   self.size_buf.data_ptr(), self.max_num_agents, self.max_steps, self.bt_steps,
                                   self.forward_steps, self.latent_dim)
 
-    def gather(self, idxes):
-        """Window gather for the given leaf indices (int64 CUDA tensor [B]) -> dict of CUDA tensors."""
+    def gather(self, idxes, present: bool = False):
+        """Window gather for the given leaf indices (int64 CUDA tensor [B]) -> dict of CUDA tensors.
+        present=True: observations [M_pad, W, 6, 9, 9] and hidden [M_pad, latent] in present-agent rows (`present.py`, one
+        row per agent a < agents_buf[slot] of each sample), under "present" the `PresentRows` of the batch; comm_mask and the
+        scalars as without.  Sizing the output reads M on the host (one small device-to-host copy)."""
         torch = _torch()
         idx = torch.as_tensor(idxes, dtype=torch.int64).to(self.device).contiguous()
+        if present:
+            return self._gather_present(idx)
         B, n, W, dev = int(idx.numel()), self.max_num_agents, self.bt_steps + self.forward_steps, self.device
         e = lambda shape, dt: torch.empty(shape, dtype=dt, device=dev)
         out = dict(obs=e((B, W, n, *config.obs_shape), torch.float16), comm_mask=e((B, W, n, n), torch.uint8),
@@ -173,6 +186,32 @@ class ReplayStore:
         gather = self._lib.mapf_replay_gather_compact if self.compact else self._lib.mapf_replay_gather
         _native.check(gather(C.byref(view), C.c_void_p(idx.data_ptr()), B, C.byref(batch), C.c_void_p(self._err.data_ptr()),
                              self._stream()))
+        return out
+
+    def _gather_present(self, idx):
+        torch = _torch()
+        counts = self.agents_buf[idx // self.max_steps]
+        pr = PresentRows(counts, int(counts.sum(dtype=torch.int64).item()), self.max_num_agents)
+        if not self.compact:   # the padded gather, indexed: also the reference the kernel is tested against
+            out = self.gather(idx)
+            B, W = pr.B, self.bt_steps + self.forward_steps
+            out["obs"] = pr.select(out["obs"].transpose(1, 2).reshape(B * pr.N, W, *config.obs_shape))
+            out["hidden"] = pr.select(out["hidden"])
+            out["present"] = pr
+            return out
+        B, n, W, dev = pr.B, self.max_num_agents, self.bt_steps + self.forward_steps, self.device
+        e = lambda shape, dt: torch.empty(shape, dtype=dt, device=dev)
+        out = dict(obs=e((pr.M_pad, W, *config.obs_shape), torch.float16), comm_mask=e((B, W, n, n), torch.uint8),
+                   hidden=e((pr.M_pad, self.latent_dim), torch.float16), action=e((B,), torch.int64),
+                   reward=e((B,), torch.float16), done=e((B,), torch.float16), steps=e((B,), torch.float16),
+                   bt_steps=e((B,), torch.int64))
+        view = self._view()
+        batch = _native.ReplayBatch(*[out[k].data_ptr() for k in ("obs", "comm_mask", "hidden", "action", "reward", "done",
+                                                                   "steps", "bt_steps")])
+        _native.check(self._lib.mapf_replay_gather_present(
+            C.byref(view), C.c_void_p(self.agents_buf.data_ptr()), C.c_void_p(idx.data_ptr()), C.c_void_p(pr.first.data_ptr()),
+            B, pr.M_pad, C.byref(batch), C.c_void_p(self._err.data_ptr()), self._stream()))
+        out["present"] = pr
         return out
 
     def sample_batch(self, batch_size: int, uniforms=None, check: bool = True):
