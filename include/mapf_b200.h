@@ -493,6 +493,23 @@ int mapf_replay_gather_present(const mapf_replay_view_compact *view, const uint8
                                const int32_t *d_first, int64_t batch, int64_t out_rows, const mapf_replay_batch *out,
                                int32_t *d_err, void *stream);
 
+/* ---- prioritized planning on the device (DESIGN.md §8 (f)5) --------------------------------------------------------------
+ * A collision-free plan for every environment of the batch from its current state (map, positions as starts, goals), in one
+ * launch.  Agents a = 0 .. n_e - 1 (n_e = N on a uniform handle) are planned in index order; agent a takes the
+ * earliest-arrival space-time path, waits included, that neither enters a cell a higher-priority agent occupies at that time
+ * nor swaps cells with one, and then parks on its goal until the horizon.  Its arrival is the first t <= horizon at which it
+ * stands on its goal and no higher-priority agent enters the goal at t or later.  Ties between paths go to the lowest action id
+ * when the path is read back from the goal.
+ *   d_actions  u8[horizon, B, N]  action ids of environment.py:12; 0 from an agent's arrival on, for absent agents and for a
+ *                                 failed environment -- the [T, B, N] layout mapf_env_rollout replays
+ *   d_arrival  i32[B, N]          each agent's arrival step; 0 for absent agents; the whole row -1 where some agent finds no
+ *                                 path within the horizon (the agents after it are not planned)
+ * MAPF_EINVAL for a horizon outside 1 .. MAPF_PLAN_MAX_HORIZON or a NULL buffer, MAPF_ENOMEM if the planner's scratch (per
+ * resident warp: six bit tables of horizon + 1 map slices, added to mapf_env_arena_bytes) cannot be allocated.  Reads the
+ * handle's state and writes nothing in it; asynchronous on `stream`. */
+#define MAPF_PLAN_MAX_HORIZON 1024
+int mapf_env_plan_prioritized(mapf_env *env, int32_t horizon, uint8_t *d_actions, int32_t *d_arrival, void *stream);
+
 /* ---- CBS expert / solvable-instance generator (search.py:58-442, test.py:23-79; SURVEY 8(f)4) -- HOST code ------------------
  * Conflict-based search over space-time A*: a collision-free set of paths of minimal sum of costs (search.py:17-21), as the
  * action script search.find_path returns (search.py:396-442).  All pointers are HOST memory; no kernel is launched.

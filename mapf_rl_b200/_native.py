@@ -69,6 +69,7 @@ SIGNATURES = {
     "mapf_env_arena_bytes": (_i64, [_vp]),
     "mapf_env_load": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _vp, _vp]),
     "mapf_env_bfs_navi": (C.c_int, [_vp, _vp, _i32, _vp, _vp]),
+    "mapf_env_plan_prioritized": (C.c_int, [_vp, _i32, _vp, _vp, _vp]),
     "mapf_env_step_observe": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mapf_env_step_observe_ex": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mapf_env_observe": (C.c_int, [_vp, _vp, _vp, _vp]),

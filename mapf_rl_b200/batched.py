@@ -292,6 +292,25 @@ class BatchedEnvironment:
         _native.check(self._lib.mapf_env_rollout_ex(self._h, C.byref(io), self._stream()))
         return obs, rewards, done, steps
 
+    def plan(self, horizon: int = config.max_steps):
+        """Prioritized planning on the device (mapf_env_plan_prioritized) from the current state: agents in index order,
+        each on its earliest-arrival path that avoids the paths of the agents before it (no shared cell, no swap), parked
+        on its goal afterwards.  Returns (actions uint8[H,B,N], arrival int32[B,N], makespan int32[B], soc int32[B]) CUDA
+        tensors on the current stream.  `actions` is the [T, B, N] script `rollout` replays as it is.  arrival: each
+        agent's arrival step, 0 for absent agents; makespan / soc are the maximum / sum of an environment's arrivals.  An
+        environment where some agent finds no path within `horizon` steps has arrival row, makespan and soc -1 and all
+        actions 0.  The handle's state is not changed."""
+        torch = _torch()
+        B, N, H = self.num_envs, self.num_agents, int(horizon)
+        actions = torch.empty((max(H, 1), B, N), dtype=torch.uint8, device=self.device)
+        arrival = torch.empty((B, N), dtype=torch.int32, device=self.device)
+        _native.check(self._lib.mapf_env_plan_prioritized(self._h, H, C.c_void_p(actions.data_ptr()),
+                                                          C.c_void_p(arrival.data_ptr()), self._stream()))
+        failed = (arrival < 0).any(1)
+        makespan = torch.where(failed, -1, arrival.max(1).values).to(torch.int32)
+        soc = torch.where(failed, -1, arrival.sum(1)).to(torch.int32)
+        return actions, arrival, makespan, soc
+
     def set_autoreset(self, max_steps: int = config.max_steps, seed: int = 0, env_offset: int = 0, stride: Optional[int] = None,
                       density: Optional[float] = None):
         """Episode handling inside `rollout` (worker.py:390,422-428): a step that finds its environment finished (done, or

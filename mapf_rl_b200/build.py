@@ -20,7 +20,7 @@ LIB_PATH = LIB_OVERRIDE or os.path.join(_HERE, "libmapf_b200.so")
 DIAG_LIB_PATH = os.path.join(_HERE, "libmapf_b200_diag.so")
 SOURCES = ["mapf_rollout_occ8.cu", "mapf_rollout_occ10.cu", "mapf_rollout_occ12.cu", "mapf_rollout_occ16.cu", "mapf_step_kernels.cu", "mapf_abi.cu",
            "mapf_env_kernels.cu", "mapf_rollout_kernels.cu", "mapf_reset_kernels.cu", "mapf_per_kernels.cu", "mapf_replay_kernels.cu",
-           "mapf_cbs.cu"]
+           "mapf_cbs.cu", "mapf_plan_kernels.cu"]
 HEADERS = ["mapf_common.cuh", "mapf_step_device.cuh", "mapf_bfs_device.cuh", "mapf_reset_device.cuh", "mapf_rollout_device.cuh",
            os.path.join("..", "..", "include", "mapf_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"]

@@ -15,6 +15,7 @@ int mapf_launch_pack_load_sized(mapf_env *, const int32_t *, int, const uint8_t 
 int mapf_launch_reset_levels(mapf_env *, const uint8_t *, uint64_t, uint64_t, float, const uint8_t *, int, cudaStream_t);
 int mapf_launch_validate_state(mapf_env *, const int32_t *, int, cudaStream_t);
 int mapf_launch_bfs(mapf_env *, const int32_t *, int, int32_t *, cudaStream_t);
+int mapf_launch_plan(mapf_env *, int, uint8_t *, int32_t *, cudaStream_t);
 int mapf_launch_step(mapf_env *, const uint8_t *, uint8_t *, const int64_t *, const StepOut &, cudaStream_t);
 int mapf_launch_observe(mapf_env *, uint8_t *, const int64_t *, uint8_t *, const uint8_t *, cudaStream_t);
 int mapf_launch_step_only(mapf_env *, const uint8_t *, const StepOut &, uint8_t *, cudaStream_t);
@@ -277,6 +278,7 @@ int mapf_env_destroy(mapf_env *env)
     cudaFree(env->sz_n);
     cudaFree(env->sz_l);
     cudaFree(env->sz_full);
+    cudaFree(env->pp_scratch);
     cudaFree(env->ro_work);
     cudaFree(env->ro_progress);
     cudaFree(env->ro_episode);
@@ -494,6 +496,18 @@ int mapf_env_bfs_navi(mapf_env *env, const int32_t *d_env_ids, int32_t n, int32_
     }
     if (n == 0) return MAPF_OK;
     return mapf_launch_bfs(env, d_env_ids, n, d_dist_out, static_cast<cudaStream_t>(stream));
+}
+
+int mapf_env_plan_prioritized(mapf_env *env, int32_t horizon, uint8_t *d_actions, int32_t *d_arrival, void *stream)
+{
+    REQUIRE_ENV(env);
+    if (horizon < 1 || horizon > MAPF_PLAN_MAX_HORIZON || !d_actions || !d_arrival) {
+        mapf_set_error("mapf_env_plan_prioritized: 1 <= horizon <= 1024 and non-NULL d_actions, d_arrival required");
+        return MAPF_EINVAL;
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    MAPF_DRAIN(env, st);
+    return mapf_launch_plan(env, horizon, d_actions, d_arrival, st);
 }
 
 int mapf_env_step_observe_ex(mapf_env *env, const uint8_t *d_actions, uint8_t *d_obs, const int64_t *d_obs_rows, float *d_rewards,

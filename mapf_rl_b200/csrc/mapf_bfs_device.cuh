@@ -85,10 +85,27 @@ __device__ __forceinline__ void bfs_init(const EnvDims &d, const BfsFree<RW, RPL
     }
 }
 
-// One wave: nw = (frontier shifted to the four neighbours) & free-and-unvisited; returns the OR of this lane's words.
+// Word w of the rows of the neighbouring lanes that touch this lane's block: the last row of the lane above and the first
+// row of the lane below, 0 past the group's ends.
 // WRAP: the group's last row is past the map (L < LW * RPL), so the neighbour rows can come from a rotating shuffle with
 // nothing to zero at the group's ends -- the first lane receives the last lane's (empty) last row, and what the last lane
 // receives lands on that empty row, where free-and-unvisited is 0.
+template <int RW, int RPL, int LW, bool WRAP>
+__device__ __forceinline__ void bfs_rows_around(const uint32_t (&f)[RPL][RW], const int w, const int lane, uint32_t &above,
+                                                uint32_t &below)
+{
+    if constexpr (WRAP) {
+        above = __shfl_sync(MAPF_FULL_MASK, f[RPL - 1][w], (lane + LW - 1) & (LW - 1), LW);
+        below = __shfl_sync(MAPF_FULL_MASK, f[0][w], (lane + 1) & (LW - 1), LW);
+    } else {
+        above = __shfl_up_sync(MAPF_FULL_MASK, f[RPL - 1][w], 1, LW);
+        below = __shfl_down_sync(MAPF_FULL_MASK, f[0][w], 1, LW);
+        if (lane == 0) above = 0;
+        if (lane == LW - 1) below = 0;
+    }
+}
+
+// One wave: nw = (frontier shifted to the four neighbours) & free-and-unvisited; returns the OR of this lane's words.
 template <int RW, int RPL, int APW, bool WRAP>
 __device__ __forceinline__ uint32_t bfs_wave(const BfsState<RW, RPL> &S, uint32_t (&nw)[RPL][RW])
 {
@@ -97,17 +114,8 @@ __device__ __forceinline__ uint32_t bfs_wave(const BfsState<RW, RPL> &S, uint32_
     uint32_t any = 0;
 #pragma unroll
     for (int w = 0; w < RW; ++w) {
-        // rows of the neighbouring lanes that touch this lane's block
         uint32_t above, below;
-        if constexpr (WRAP) {
-            above = __shfl_sync(MAPF_FULL_MASK, S.fro[RPL - 1][w], (lane + LW - 1) & (LW - 1), LW);
-            below = __shfl_sync(MAPF_FULL_MASK, S.fro[0][w], (lane + 1) & (LW - 1), LW);
-        } else {
-            above = __shfl_up_sync(MAPF_FULL_MASK, S.fro[RPL - 1][w], 1, LW);
-            below = __shfl_down_sync(MAPF_FULL_MASK, S.fro[0][w], 1, LW);
-            if (lane == 0) above = 0;
-            if (lane == LW - 1) below = 0;
-        }
+        bfs_rows_around<RW, RPL, LW, WRAP>(S.fro, w, lane, above, below);
 #pragma unroll
         for (int q = 0; q < RPL; ++q) {
             const uint32_t f = S.fro[q][w];
