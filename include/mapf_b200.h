@@ -510,6 +510,24 @@ int mapf_replay_gather_present(const mapf_replay_view_compact *view, const uint8
 #define MAPF_PLAN_MAX_HORIZON 1024
 int mapf_env_plan_prioritized(mapf_env *env, int32_t horizon, uint8_t *d_actions, int32_t *d_arrival, void *stream);
 
+/* The best of `orders` priority orders per environment.  Order 0 is index order; order r >= 1 sorts the present agents a by
+ * (k_a, a), k_a = word 0 of Philox4x32-10 with counter (g_lo, g_hi, 4 | r << 8, a) and key (seed_lo, seed_hi), where
+ * g = env_offset + e is the environment's global index -- so a batch sharded over handles plans what one handle would.  Each
+ * order is planned as mapf_env_plan_prioritized plans index order, with the agents taken in that order; the environment's
+ * result is its solved order of smallest sum of costs, ties to the smallest r.
+ *   d_actions  u8[horizon, B, N]  that order's actions, as mapf_env_plan_prioritized writes them
+ *   d_arrival  i32[B, N]          that order's arrivals, indexed by agent; 0 for absent agents; the whole row -1 where every
+ *                                 order fails (actions 0 there)
+ *   d_order    i32[B]             the winning r, -1 where every order fails
+ *   d_rank     u8[B, N]           agent a's position in the winning order; 255 for absent agents and failed environments
+ * MAPF_EINVAL for a horizon outside 1 .. MAPF_PLAN_MAX_HORIZON, orders outside 1 .. MAPF_PLAN_MAX_ORDERS or a NULL buffer,
+ * MAPF_ENOMEM if the planner's scratch (mapf_env_plan_prioritized's, plus 8 bytes per environment) cannot be allocated.
+ * Every order is planned once, and the winning one once more to write its results.  Reads the handle's state and writes
+ * nothing in it; asynchronous on `stream`. */
+#define MAPF_PLAN_MAX_ORDERS 256
+int mapf_env_plan_prioritized_orders(mapf_env *env, int32_t horizon, int32_t orders, uint64_t seed, uint64_t env_offset,
+                                     uint8_t *d_actions, int32_t *d_arrival, int32_t *d_order, uint8_t *d_rank, void *stream);
+
 /* ---- CBS expert / solvable-instance generator (search.py:58-442, test.py:23-79; SURVEY 8(f)4) -- HOST code ------------------
  * Conflict-based search over space-time A*: a collision-free set of paths of minimal sum of costs (search.py:17-21), as the
  * action script search.find_path returns (search.py:396-442).  All pointers are HOST memory; no kernel is launched.

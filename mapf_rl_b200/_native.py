@@ -70,6 +70,7 @@ SIGNATURES = {
     "mapf_env_load": (C.c_int, [_vp, _vp, _i32, _vp, _vp, _vp, _vp]),
     "mapf_env_bfs_navi": (C.c_int, [_vp, _vp, _i32, _vp, _vp]),
     "mapf_env_plan_prioritized": (C.c_int, [_vp, _i32, _vp, _vp, _vp]),
+    "mapf_env_plan_prioritized_orders": (C.c_int, [_vp, _i32, _i32, _u64, _u64, _vp, _vp, _vp, _vp, _vp]),
     "mapf_env_step_observe": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mapf_env_step_observe_ex": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mapf_env_observe": (C.c_int, [_vp, _vp, _vp, _vp]),

@@ -311,6 +311,28 @@ class BatchedEnvironment:
         soc = torch.where(failed, -1, arrival.sum(1)).to(torch.int32)
         return actions, arrival, makespan, soc
 
+    def plan_orders(self, horizon: int = config.max_steps, orders: int = 8, seed: int = 0, env_offset: int = 0):
+        """Prioritized planning over `orders` priority orders per environment (mapf_env_plan_prioritized_orders): order 0 is
+        index order, order r >= 1 a Philox permutation of the agents drawn from (seed, env_offset + e, r), each planned as
+        `plan` plans index order; an environment keeps its solved order of smallest sum of costs, ties to the smallest r.
+        Returns (actions uint8[H,B,N], arrival int32[B,N], makespan int32[B], soc int32[B], order int32[B], rank
+        uint8[B,N]) CUDA tensors on the current stream: the first four as `plan` returns them, for the winning order;
+        order: the winning r, -1 where every order fails; rank: each agent's position in the winning order, 255 for absent
+        agents and failed environments.  With orders=1 the first four equal `plan`'s.  The handle's state is not changed."""
+        torch = _torch()
+        B, N, H = self.num_envs, self.num_agents, int(horizon)
+        actions = torch.empty((max(H, 1), B, N), dtype=torch.uint8, device=self.device)
+        arrival = torch.empty((B, N), dtype=torch.int32, device=self.device)
+        order = torch.empty(B, dtype=torch.int32, device=self.device)
+        rank = torch.empty((B, N), dtype=torch.uint8, device=self.device)
+        _native.check(self._lib.mapf_env_plan_prioritized_orders(
+            self._h, H, int(orders), int(seed), int(env_offset), C.c_void_p(actions.data_ptr()),
+            C.c_void_p(arrival.data_ptr()), C.c_void_p(order.data_ptr()), C.c_void_p(rank.data_ptr()), self._stream()))
+        failed = (arrival < 0).any(1)
+        makespan = torch.where(failed, -1, arrival.max(1).values).to(torch.int32)
+        soc = torch.where(failed, -1, arrival.sum(1)).to(torch.int32)
+        return actions, arrival, makespan, soc, order, rank
+
     def set_autoreset(self, max_steps: int = config.max_steps, seed: int = 0, env_offset: int = 0, stride: Optional[int] = None,
                       density: Optional[float] = None):
         """Episode handling inside `rollout` (worker.py:390,422-428): a step that finds its environment finished (done, or

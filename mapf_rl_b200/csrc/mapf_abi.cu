@@ -16,6 +16,7 @@ int mapf_launch_reset_levels(mapf_env *, const uint8_t *, uint64_t, uint64_t, fl
 int mapf_launch_validate_state(mapf_env *, const int32_t *, int, cudaStream_t);
 int mapf_launch_bfs(mapf_env *, const int32_t *, int, int32_t *, cudaStream_t);
 int mapf_launch_plan(mapf_env *, int, uint8_t *, int32_t *, cudaStream_t);
+int mapf_launch_plan_orders(mapf_env *, int, int, uint64_t, uint64_t, uint8_t *, int32_t *, int32_t *, uint8_t *, cudaStream_t);
 int mapf_launch_step(mapf_env *, const uint8_t *, uint8_t *, const int64_t *, const StepOut &, cudaStream_t);
 int mapf_launch_observe(mapf_env *, uint8_t *, const int64_t *, uint8_t *, const uint8_t *, cudaStream_t);
 int mapf_launch_step_only(mapf_env *, const uint8_t *, const StepOut &, uint8_t *, cudaStream_t);
@@ -508,6 +509,21 @@ int mapf_env_plan_prioritized(mapf_env *env, int32_t horizon, uint8_t *d_actions
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     MAPF_DRAIN(env, st);
     return mapf_launch_plan(env, horizon, d_actions, d_arrival, st);
+}
+
+int mapf_env_plan_prioritized_orders(mapf_env *env, int32_t horizon, int32_t orders, uint64_t seed, uint64_t env_offset,
+                                     uint8_t *d_actions, int32_t *d_arrival, int32_t *d_order, uint8_t *d_rank, void *stream)
+{
+    REQUIRE_ENV(env);
+    if (horizon < 1 || horizon > MAPF_PLAN_MAX_HORIZON || orders < 1 || orders > MAPF_PLAN_MAX_ORDERS || !d_actions || !d_arrival ||
+        !d_order || !d_rank) {
+        mapf_set_error("mapf_env_plan_prioritized_orders: 1 <= horizon <= 1024, 1 <= orders <= 256 and non-NULL d_actions, "
+                       "d_arrival, d_order, d_rank required");
+        return MAPF_EINVAL;
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    MAPF_DRAIN(env, st);
+    return mapf_launch_plan_orders(env, horizon, orders, seed, env_offset, d_actions, d_arrival, d_order, d_rank, st);
 }
 
 int mapf_env_step_observe_ex(mapf_env *env, const uint8_t *d_actions, uint8_t *d_obs, const int64_t *d_obs_rows, float *d_rewards,

@@ -1,5 +1,6 @@
 // mapf_plan_kernels.cu — prioritized planning (PP) on the device: a collision-free plan for every environment of a batch in
-// one launch (mapf_env_plan_prioritized, DESIGN.md §8 (f)5).
+// one launch (mapf_env_plan_prioritized, DESIGN.md §8 (f)5), and the best of R priority orders per environment
+// (mapf_env_plan_prioritized_orders).
 //
 // Agents a = 0 .. n-1 are planned in index order.  Agent a takes the earliest-arrival space-time path that avoids the paths
 // of agents 0 .. a-1, which are reserved in three tables over t = 0 .. H:
@@ -17,10 +18,16 @@
 // of padded column bits per row.  The tables and the frontier history live in per-warp global scratch owned by the handle;
 // environments are handed out through a work counter, and a warp clears its tables before each environment, so a result
 // does not depend on which warp planned it or what that warp planned before.
+//
+// Several orders: order 0 is index order, order r >= 1 sorts the agents by (Philox key of (g, PURPOSE_ORDER | r << 8, a), a).
+// Pass 1 plans every (environment, order) pair as a work item without writing actions and folds (sum of costs, r) of a
+// solved order into the environment's selection word with atomicMin, so the smallest sum of costs wins and ties go to the
+// smallest r whatever the schedule.  Pass 2 re-plans each environment's winning order and writes its results.
 #include <algorithm>
 
 #include "mapf_bfs_device.cuh"
 #include "mapf_common.cuh"
+#include "mapf_reset_device.cuh"
 
 namespace {
 
@@ -34,6 +41,7 @@ constexpr size_t kPlanCounterWords = 64;                // the work counter, ahe
 #define MAPF_PLAN_SCRATCH_MB 4096
 #endif
 constexpr int64_t kPlanScratchCap = (int64_t)MAPF_PLAN_SCRATCH_MB << 20;
+constexpr unsigned long long kNoOrder = ~0ull;  // selection word of an environment no order has solved
 
 struct PlanArgs {
     EnvDims d;
@@ -47,12 +55,29 @@ struct PlanArgs {
     int32_t *arrival;            // i32[B, N]
 };
 
+struct OrderArgs {
+    int R;                       // priority orders per environment
+    uint2 key;                   // Philox key (seed)
+    uint64_t env_offset;         // global index of environment 0
+    unsigned long long *sel;     // u64[B]: (sum of costs << 32 | r) of the best solved order, kNoOrder before pass 1
+    int32_t *order;              // i32[B]: the winning r, -1
+    uint8_t *rank;               // u8[B, N]: agent a's position in the winning order, 255
+};
+
 // offsets of action k (environment.py:12): 0 stay, 1 x-1, 2 x+1, 3 y-1, 4 y+1
 __device__ __forceinline__ int act_dx(int k) { return k == 1 ? -1 : (k == 2 ? 1 : 0); }
 __device__ __forceinline__ int act_dy(int k) { return k == 3 ? -1 : (k == 4 ? 1 : 0); }
 
-template <int RW, int RPL>
-__global__ void __launch_bounds__(kPlanWarps * 32) plan_pp_kernel(const PlanArgs p)
+// The planner of one warp, all three kernels' code:
+//   kPlanIndex        plan_pp_kernel: environment e is a work item, its agents planned in index order, results written
+//   kPlanOrders       pass 1 of plan_orders_kernel: item i = (e, r) = (i / R, i % R), agents in order r, nothing written but
+//                     (sum of costs << 32 | r) of a solved order, folded into the selection word ord.sel[e] with atomicMin
+//   kPlanOrdersFinal  pass 2: environment e is a work item, its winning order re-planned with results, rank and order
+//                     written, or the failure rows where no order solved it
+enum : int { kPlanIndex = 0, kPlanOrders = 1, kPlanOrdersFinal = 2 };
+
+template <int RW, int RPL, int MODE>
+__device__ __forceinline__ void plan_body(const PlanArgs &p, const OrderArgs &ord)
 {
     __shared__ uint16_t s_path[kPlanWarps][MAPF_PLAN_MAX_HORIZON + 1];  // x << 8 | y of the current agent at t = 0 .. t*
     constexpr int WPT = 32 * RPL * RW;  // words of one time slice of a table: [q][w][lane]
@@ -67,11 +92,39 @@ __global__ void __launch_bounds__(kPlanWarps * 32) plan_pp_kernel(const PlanArgs
     auto cell = [](int x, int y) -> size_t { return (size_t)((x % RPL) * RW + ((y + 4) >> 5)) * 32 + x / RPL; };
     auto bit = [](int y) -> uint32_t { return 1u << ((y + 4) & 31); };
 
+    uint8_t *agent = nullptr;  // the agent at each position of the order
+    uint32_t *key = nullptr;
+    if constexpr (MODE != kPlanIndex) {
+        __shared__ uint8_t s_agent[kPlanWarps][MAPF_MAX_AGENTS];
+        __shared__ uint32_t s_key[kPlanWarps][MAPF_MAX_AGENTS];
+        agent = s_agent[wid], key = s_key[wid];
+    }
+
     for (;;) {
         unsigned e = 0;
-        if (lane == 0) e = atomicAdd(p.scratch, 1u);
-        e = __shfl_sync(MAPF_FULL_MASK, e, 0);
-        if (e >= (unsigned)d.B) break;
+        int oi = 0;  // the order
+        if constexpr (MODE == kPlanIndex) {
+            if (lane == 0) e = atomicAdd(p.scratch, 1u);
+            e = __shfl_sync(MAPF_FULL_MASK, e, 0);
+            if (e >= (unsigned)d.B) break;
+        } else {
+            // 64-bit counters (B * R items): words 0 .. 1 for pass 1, 2 .. 3 for pass 2
+            unsigned long long i = 0;
+            if (lane == 0) i = atomicAdd(reinterpret_cast<unsigned long long *>(p.scratch) + (MODE == kPlanOrdersFinal), 1ull);
+            i = __shfl_sync(MAPF_FULL_MASK, i, 0);
+            if (i >= (unsigned long long)d.B * (MODE == kPlanOrders ? ord.R : 1)) break;
+            e = MODE == kPlanOrders ? (unsigned)(i / ord.R) : (unsigned)i;
+            oi = MODE == kPlanOrders ? (int)(i % ord.R) : 0;
+            if constexpr (MODE == kPlanOrdersFinal) {
+                const unsigned long long sel = __ldcg(ord.sel + e);
+                if (sel == kNoOrder) {  // every order failed: arrival row -1, rank 255, actions 0 (zeroed before the launch)
+                    for (int b = lane; b < d.N; b += 32) p.arrival[(size_t)e * d.N + b] = -1, ord.rank[(size_t)e * d.N + b] = 255;
+                    if (lane == 0) ord.order[e] = -1;
+                    continue;
+                }
+                oi = (int)(uint32_t)sel;
+            }
+        }
 
         // clean reservation tables: Occ and SB_1 .. SB_4 over t = 0 .. H
         {
@@ -85,10 +138,31 @@ __global__ void __launch_bounds__(kPlanWarps * 32) plan_pp_kernel(const PlanArgs
         BfsFree<RW, RPL> F;
         bfs_load_free<RW, RPL, 1>(df, p.obst + (size_t)e * d.obst_stride, F);
         int32_t *const arr = p.arrival + (size_t)e * d.N;
-        for (int a = n + lane; a < d.N; a += 32) arr[a] = 0;  // absent agents
+        if constexpr (MODE != kPlanOrders)
+            for (int a = n + lane; a < d.N; a += 32) arr[a] = 0;  // absent agents
+        if constexpr (MODE != kPlanIndex) {
+            // order oi: agent a goes to position #{b < n : (k_b, b) < (k_a, a)}; order 0 has every key 0, i.e. index order
+            const uint64_t ge = ord.env_offset + e;  // the environment's global index
+            for (int a = lane; a < n; a += 32)
+                key[a] = oi ? philox4x32_10(make_uint4((uint32_t)ge, (uint32_t)(ge >> 32), PURPOSE_ORDER | ((uint32_t)oi << 8), (uint32_t)a), ord.key).x
+                           : 0u;
+            __syncwarp();
+            for (int a = lane; a < n; a += 32) {
+                const uint32_t ka = key[a];
+                int pos = 0;
+                for (int b = 0; b < n; ++b) pos += key[b] < ka || (key[b] == ka && b < a);
+                agent[pos] = (uint8_t)a;
+                if constexpr (MODE == kPlanOrdersFinal) ord.rank[(size_t)e * d.N + a] = (uint8_t)pos;
+            }
+            if constexpr (MODE == kPlanOrdersFinal)
+                for (int a = n + lane; a < d.N; a += 32) ord.rank[(size_t)e * d.N + a] = 255;
+        }
         __syncwarp();
 
-        for (int a = 0; a < n; ++a) {
+        int soc = 0;
+        bool solved = true;
+        for (int j = 0; j < n; ++j) {  // an order stops at its first failing agent
+            const int a = MODE == kPlanIndex ? j : agent[j];
             const uchar2 s = __ldcg(reinterpret_cast<const uchar2 *>(p.pos) + (size_t)e * d.N + a);
             const uchar2 g = __ldcg(reinterpret_cast<const uchar2 *>(p.goal) + (size_t)e * d.N + a);
             const size_t gi = cell(g.x, g.y);
@@ -169,10 +243,13 @@ __global__ void __launch_bounds__(kPlanWarps * 32) plan_pp_kernel(const PlanArgs
             }
             __syncwarp();
 
-            if (tstar < 0) {  // the environment fails: no plan, no actions, arrival row -1
-                for (int t = lane; t < H; t += 32)
-                    for (int b = 0; b < a; ++b) p.actions[((size_t)t * d.B + e) * d.N + b] = 0;
-                for (int b = lane; b < d.N; b += 32) arr[b] = -1;
+            if (tstar < 0) {  // the environment (the order) fails: no plan, no actions, arrival row -1
+                if constexpr (MODE == kPlanIndex) {
+                    for (int t = lane; t < H; t += 32)
+                        for (int b = 0; b < a; ++b) p.actions[((size_t)t * d.B + e) * d.N + b] = 0;
+                    for (int b = lane; b < d.N; b += 32) arr[b] = -1;
+                }
+                solved = false;
                 break;
             }
 
@@ -205,16 +282,81 @@ __global__ void __launch_bounds__(kPlanWarps * 32) plan_pp_kernel(const PlanArgs
                     const int x2 = path[t + 1] >> 8, y2 = path[t + 1] & 255;
                     const int k = x2 < x ? 1 : (x2 > x ? 2 : (y2 < y ? 3 : (y2 > y ? 4 : 0)));
                     if (k) {
-                        p.actions[((size_t)t * d.B + e) * d.N + a] = (uint8_t)k;
+                        if constexpr (MODE != kPlanOrders) p.actions[((size_t)t * d.B + e) * d.N + a] = (uint8_t)k;
                         uint32_t *r = sb + (k & 1 ? k + 1 : k - 1) * tbl + (size_t)t * WPT + cell(x, y);
                         __stcg(r, __ldcg(r) | bit(y));
                     }
                 }
             }
-            if (lane == 0) arr[a] = tstar;
+            if (MODE != kPlanOrders && lane == 0) arr[a] = tstar;
+            soc += tstar;
+            __syncwarp();
+        }
+        if constexpr (MODE != kPlanIndex) {
+            if (lane == 0) {
+                if (MODE == kPlanOrdersFinal) ord.order[e] = oi;
+                else if (solved) atomicMin(ord.sel + e, (unsigned long long)soc << 32 | (unsigned)oi);
+            }
             __syncwarp();
         }
     }
+}
+
+template <int RW, int RPL>
+__global__ void __launch_bounds__(kPlanWarps * 32) plan_pp_kernel(const PlanArgs p)
+{
+    plan_body<RW, RPL, kPlanIndex>(p, OrderArgs{});
+}
+
+template <int RW, int RPL, int MODE>
+__global__ void __launch_bounds__(kPlanWarps * 32) plan_orders_kernel(const PlanArgs p, const OrderArgs o)
+{
+    plan_body<RW, RPL, MODE>(p, o);
+}
+
+// The handle's planner scratch: at least `bytes`, allocated on first use and grown when a call needs more
+int reserve_plan_scratch(mapf_env *env, int64_t bytes, cudaStream_t st, const char *what)
+{
+    if (bytes <= env->pp_bytes) return MAPF_OK;
+    if (env->pp_scratch) {
+        MAPF_CUDA(cudaStreamSynchronize(st));
+        cudaFree(env->pp_scratch);
+        env->arena_bytes -= env->pp_bytes;
+        env->pp_scratch = nullptr, env->pp_bytes = 0;
+    }
+    const cudaError_t e = cudaMalloc(reinterpret_cast<void **>(&env->pp_scratch), (size_t)bytes);
+    if (e != cudaSuccess) {
+        mapf_cuda_fail(e, what);
+        env->pp_scratch = nullptr;
+        return MAPF_ENOMEM;
+    }
+    env->pp_bytes = bytes;
+    env->arena_bytes += bytes;
+    return MAPF_OK;
+}
+
+// blocks of a planner launch over `items` warp work items: the resident blocks, at most the scratch cap
+template <typename Kernel>
+int plan_blocks(mapf_env *env, Kernel kernel, int64_t items, int64_t block_bytes, int64_t &blocks)
+{
+    int per_sm = 0;
+    MAPF_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kPlanWarps * 32, 0));
+    blocks = std::min<int64_t>((int64_t)std::max(per_sm, 1) * env->num_sms, (items + kPlanWarps - 1) / kPlanWarps);
+    blocks = std::max<int64_t>(1, std::min<int64_t>(blocks, kPlanScratchCap / block_bytes));
+    return MAPF_OK;
+}
+
+PlanArgs plan_args(mapf_env *env, int H, size_t warp_words, uint8_t *d_actions, int32_t *d_arrival)
+{
+    PlanArgs p;
+    p.d = env->d;
+    p.obst = env->obst, p.pos = env->pos, p.goal = env->goal;
+    p.sz_n = env->sz_n, p.sz_l = env->sz_l;
+    p.H = H;
+    p.warp_words = warp_words;
+    p.scratch = env->pp_scratch;
+    p.actions = d_actions, p.arrival = d_arrival;
+    return p;
 }
 
 template <int RW, int RPL>
@@ -222,39 +364,49 @@ int launch_plan(mapf_env *env, int H, uint8_t *d_actions, int32_t *d_arrival, cu
 {
     const EnvDims &d = env->d;
     const size_t warp_words = (size_t)kPlanTables * (H + 1) * 32 * RPL * RW;
-    int per_sm = 0;
-    MAPF_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, plan_pp_kernel<RW, RPL>, kPlanWarps * 32, 0));
     const int64_t block_bytes = (int64_t)kPlanWarps * warp_words * 4;
-    int64_t blocks = std::min<int64_t>((int64_t)std::max(per_sm, 1) * env->num_sms, (d.B + kPlanWarps - 1) / kPlanWarps);
-    blocks = std::max<int64_t>(1, std::min<int64_t>(blocks, kPlanScratchCap / block_bytes));
-    const int64_t bytes = (int64_t)kPlanCounterWords * 4 + blocks * block_bytes;
-    if (bytes > env->pp_bytes) {  // first use, or a larger horizon / grid than before
-        if (env->pp_scratch) {
-            MAPF_CUDA(cudaStreamSynchronize(st));
-            cudaFree(env->pp_scratch);
-            env->arena_bytes -= env->pp_bytes;
-            env->pp_scratch = nullptr, env->pp_bytes = 0;
-        }
-        const cudaError_t e = cudaMalloc(reinterpret_cast<void **>(&env->pp_scratch), (size_t)bytes);
-        if (e != cudaSuccess) {
-            mapf_cuda_fail(e, "mapf_env_plan_prioritized: scratch");
-            env->pp_scratch = nullptr;
-            return MAPF_ENOMEM;
-        }
-        env->pp_bytes = bytes;
-        env->arena_bytes += bytes;
-    }
+    int64_t blocks = 0;
+    int rc = plan_blocks(env, plan_pp_kernel<RW, RPL>, d.B, block_bytes, blocks);
+    if (rc != MAPF_OK) return rc;
+    rc = reserve_plan_scratch(env, (int64_t)kPlanCounterWords * 4 + blocks * block_bytes, st,
+                                        "mapf_env_plan_prioritized: scratch");
+    if (rc != MAPF_OK) return rc;
     MAPF_CUDA(cudaMemsetAsync(env->pp_scratch, 0, 4, st));
     MAPF_CUDA(cudaMemsetAsync(d_actions, 0, (size_t)H * d.B * d.N, st));
-    PlanArgs p;
-    p.d = d;
-    p.obst = env->obst, p.pos = env->pos, p.goal = env->goal;
-    p.sz_n = env->sz_n, p.sz_l = env->sz_l;
-    p.H = H;
-    p.warp_words = warp_words;
-    p.scratch = env->pp_scratch;
-    p.actions = d_actions, p.arrival = d_arrival;
-    plan_pp_kernel<RW, RPL><<<(unsigned)blocks, kPlanWarps * 32, 0, st>>>(p);
+    plan_pp_kernel<RW, RPL><<<(unsigned)blocks, kPlanWarps * 32, 0, st>>>(plan_args(env, H, warp_words, d_actions, d_arrival));
+    MAPF_CUDA(cudaGetLastError());
+    return MAPF_OK;
+}
+
+template <int RW, int RPL>
+int launch_plan_orders(mapf_env *env, int H, int R, uint64_t seed, uint64_t env_offset, uint8_t *d_actions, int32_t *d_arrival,
+                       int32_t *d_order, uint8_t *d_rank, cudaStream_t st)
+{
+    const EnvDims &d = env->d;
+    const size_t warp_words = (size_t)kPlanTables * (H + 1) * 32 * RPL * RW;
+    const int64_t block_bytes = (int64_t)kPlanWarps * warp_words * 4;
+    int64_t blocks = 0, blocks2 = 0;
+    int rc = plan_blocks(env, plan_orders_kernel<RW, RPL, kPlanOrders>, (int64_t)d.B * R, block_bytes, blocks);
+    if (rc == MAPF_OK) rc = plan_blocks(env, plan_orders_kernel<RW, RPL, kPlanOrdersFinal>, d.B, block_bytes, blocks2);
+    if (rc != MAPF_OK) return rc;
+    // the selection words follow the warps' tables
+    const int64_t sel_off = (int64_t)kPlanCounterWords * 4 + blocks * block_bytes;
+    rc = reserve_plan_scratch(env, sel_off + (int64_t)d.B * 8, st, "mapf_env_plan_prioritized_orders: scratch");
+    if (rc != MAPF_OK) return rc;
+    OrderArgs o;
+    o.R = R;
+    o.key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
+    o.env_offset = env_offset;
+    o.sel = reinterpret_cast<unsigned long long *>(reinterpret_cast<char *>(env->pp_scratch) + sel_off);
+    o.order = d_order, o.rank = d_rank;
+    MAPF_CUDA(cudaMemsetAsync(env->pp_scratch, 0, 16, st));
+    MAPF_CUDA(cudaMemsetAsync(o.sel, 0xff, (size_t)d.B * 8, st));
+    MAPF_CUDA(cudaMemsetAsync(d_actions, 0, (size_t)H * d.B * d.N, st));
+    const PlanArgs p = plan_args(env, H, warp_words, d_actions, d_arrival);
+    plan_orders_kernel<RW, RPL, kPlanOrders><<<(unsigned)blocks, kPlanWarps * 32, 0, st>>>(p, o);
+    MAPF_CUDA(cudaGetLastError());
+    // pass 2 uses the tables of the first blocks2 <= blocks blocks of pass 1
+    plan_orders_kernel<RW, RPL, kPlanOrdersFinal><<<(unsigned)std::min(blocks, blocks2), kPlanWarps * 32, 0, st>>>(p, o);
     MAPF_CUDA(cudaGetLastError());
     return MAPF_OK;
 }
@@ -275,5 +427,25 @@ int mapf_launch_plan(mapf_env *env, int H, uint8_t *d_actions, int32_t *d_arriva
         case 4 * 8 + 4: return launch_plan<4, 4>(env, H, d_actions, d_arrival, st);
     }
     mapf_set_error("mapf_env_plan_prioritized: unsupported map size");
+    return MAPF_EINVAL;
+}
+
+int mapf_launch_plan_orders(mapf_env *env, int H, int R, uint64_t seed, uint64_t env_offset, uint8_t *d_actions, int32_t *d_arrival,
+                            int32_t *d_order, uint8_t *d_rank, cudaStream_t st)
+{
+    const int rpl = (env->d.L + 31) / 32;
+#define MAPF_PLAN_ORDERS_CASE(rw, r) \
+    case rw * 8 + r: return launch_plan_orders<rw, r>(env, H, R, seed, env_offset, d_actions, d_arrival, d_order, d_rank, st)
+    switch (env->d.RW * 8 + rpl) {
+        MAPF_PLAN_ORDERS_CASE(1, 1);
+        MAPF_PLAN_ORDERS_CASE(2, 1);
+        MAPF_PLAN_ORDERS_CASE(2, 2);
+        MAPF_PLAN_ORDERS_CASE(3, 2);
+        MAPF_PLAN_ORDERS_CASE(3, 3);
+        MAPF_PLAN_ORDERS_CASE(4, 3);
+        MAPF_PLAN_ORDERS_CASE(4, 4);
+    }
+#undef MAPF_PLAN_ORDERS_CASE
+    mapf_set_error("mapf_env_plan_prioritized_orders: unsupported map size");
     return MAPF_EINVAL;
 }
