@@ -190,7 +190,8 @@ class ReplayStore:
 
     def _gather_present(self, idx):
         torch = _torch()
-        counts = self.agents_buf[idx // self.max_steps]
+        # an entry above N reads as N, as mapf_replay_gather_present reads it
+        counts = self.agents_buf[idx // self.max_steps].clamp(max=self.max_num_agents)
         pr = PresentRows(counts, int(counts.sum(dtype=torch.int64).item()), self.max_num_agents)
         if not self.compact:   # the padded gather, indexed: also the reference the kernel is tested against
             out = self.gather(idx)

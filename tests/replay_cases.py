@@ -18,3 +18,26 @@ def make_episode(rng, actor_id, num_agents, size, done, latent=256, cap=256):
 EPISODES = [(6, 5, True), (3, 16, False), (6, 17, True), (2, 40, False), (4, 256, False), (6, 1, True)]
 CAPACITY = 4
 BATCH = 48
+
+
+def ring_plan(geo, rng):
+    """Episodes for a store at window geometry `geo` (replay_window_ref.Geometry) -> (capacity, [(num_agents, size, done)]
+    in the order they are added).  Sizes 1, 2, bt - 1, bt, bt + 1, S - 1 and S (those in 1..S) each end up in two slots:
+    once in a slot written once, once over a full episode (stale frames past its size); agent counts are random in 1..N and
+    `done` alternates."""
+    S, bt = geo.S, geo.bt
+    sizes = sorted({s for s in (1, 2, bt - 1, bt, bt + 1, S - 1, S) if 1 <= s <= S})
+    k = len(sizes)
+    order = [S] * k + sizes + sizes      # the ring wraps after 2k: the last k overwrite the full episodes of slots 0..k-1
+    return 2 * k, [(int(rng.integers(1, geo.N + 1)), s, i % 2 == 1) for i, s in enumerate(order)]
+
+
+def ring_episodes(geo, rng):
+    """ring_plan's episodes as LocalBuffer.finish tuples, the hidden rows of a transition equal (buffer.py:148)."""
+    cap, plan = ring_plan(geo, rng)
+    eps = []
+    for k, (n, size, done) in enumerate(plan):
+        ep = list(make_episode(rng, k, n, size, done, latent=geo.latent, cap=geo.S))
+        ep[6] = np.repeat(ep[6][:, :1], n, axis=1)
+        eps.append(tuple(ep))
+    return cap, eps
