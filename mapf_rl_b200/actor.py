@@ -36,8 +36,7 @@ import numpy as np
 from . import config
 from .batched import BatchedEnvironment
 from .buffer import actor_td_errors
-from .packed import unpack_obs
-from .present import PresentRows, unpack_obs_present
+from .present import PresentRows
 from .replay import ReplayStore
 
 
@@ -137,10 +136,7 @@ class BatchedActor:
         self.t[idt] = 0
         # frame 0 of the new episodes (LocalBuffer.__init__: obs_buf[0] = init_obs, buffer.py:131); environments
         # in the middle of an episode rewrite the frame they already hold
-        if self.store.compact:
-            self.env.observe(out_bits=self.store.obs_bits, obs_rows=self._rows())
-        else:
-            self.env.observe(out_obs=self.store.obs_buf, obs_rows=self._rows())
+        self.env.observe(**self.store.frame_out(), obs_rows=self._rows())
         if self.on_begin is not None:
             self.on_begin(self, ids)
         return mask
@@ -148,7 +144,7 @@ class BatchedActor:
     # -- one lockstep step -----------------------------------------------------------------------------
     def step(self):
         torch = _torch()
-        st, env, B, N = self.store, self.env, self.B, self.N
+        st, env, B = self.store, self.env, self.B
         S = st.max_steps
         reset_mask = None
         if not self._started:
@@ -157,18 +153,8 @@ class BatchedActor:
             self._started = True
         rows = self._rows()
         pr = self.present
-        if st.compact:
-            if pr is not None:
-                obs = unpack_obs_present(st.obs_bits, rows, pr)                  # [M_pad,6,9,9] present agents' frames
-            else:
-                obs = unpack_obs(st.obs_bits, rows)                              # [B,N,6,9,9] current frames
-            comm = env.comm_mask(out_bits=st.comm_bits, rows=rows)               # + the packed row of comm_buf[size]
-        else:
-            obs = st.obs_buf.index_select(0, rows)                               # [B,N,6,9,9] current frames
-            if pr is not None:
-                obs = pr.select(obs.flatten(0, 1))
-            comm = env.comm_mask()                                               # model.py:196-208
-            st.comm_mask.index_copy_(0, rows, comm)                              # comm_buf[size] = comm_mask, buffer.py:149
+        obs = st.current_frames(rows, pr)                                        # [B,N,6,9,9] or [M_pad,6,9,9]
+        comm = st.record_comm(env, rows)                                         # model.py:196-208, -> comm_buf[size]
         if pr is not None:
             actions, q, hidden = self.net.step(obs, comm, reset_mask=self._pending_reset, present=pr)
         else:
@@ -180,18 +166,12 @@ class BatchedActor:
         actions = actions.clone()
         actions[:, 0] = torch.where(explore, rnd, actions[:, 0])
         a8 = actions.to(torch.uint8)
-        if st.compact:
-            _, rewards, done = env.step(a8, out_bits=st.obs_bits, obs_rows=rows + 1)
-        else:
-            _, rewards, done = env.step(a8, out_obs=st.obs_buf, obs_rows=rows + 1)   # next_obs -> obs_buf[size + 1]
+        _, rewards, done = env.step(a8, **st.frame_out(), obs_rows=rows + 1)     # next_obs -> obs_buf[size + 1]
         # local_buffer.add(q_val[0], actions[0], r[0], next_obs, hidden[0], comm_mask)  (worker.py:388, buffer.py:140-151)
         leaf = self.slot * S + self.t
         st.act_buf[leaf] = a8[:, 0]
         st.rew_buf[leaf] = rewards[:, 0].to(torch.float16)
-        if st.compact:
-            st.hid_buf[leaf] = hidden[:, 0].to(torch.float16)                   # agent 0's vector, once
-        else:
-            st.hid_buf[leaf] = hidden[:, 0:1, :].to(torch.float16).expand(B, N, hidden.shape[-1])   # agent 0's vector, broadcast (SURVEY q8)
+        st.write_hidden(leaf, hidden[:, 0])                                      # agent 0's vector
         self.q_buf[torch.arange(B, device=self.dev), self.t] = q[:, 0, :].float()
         self.t += 1
         self.transitions += B
@@ -202,7 +182,7 @@ class BatchedActor:
         fin = fin_dev.cpu().numpy()                                              # the one host sync of the step
         ids = np.flatnonzero(fin)
         if ids.size:
-            self._finish(ids, comm)
+            self._finish(ids)
             self._begin(ids, first=False)
             self._pending_reset = fin_dev                                        # model.reset() for those envs (worker.py:423)
         return rewards, done
@@ -210,21 +190,14 @@ class BatchedActor:
     _pending_reset = None
 
     # -- LocalBuffer.finish + GlobalBuffer.add for the envs in `ids` -------------------------------------
-    def _finish(self, ids: np.ndarray, comm):
+    def _finish(self, ids: np.ndarray):
         torch = _torch()
         st = self.store
         S = st.max_steps
         idt = torch.as_tensor(ids, device=self.dev)
         slots, size = self.slot[idt], self.t[idt]
         done = self.env._done[idt] != 0
-        # comm_buf[size]: the mask of the last model.step when the episode was cut at max_steps (worker.py:399-401; the
-        # reference re-runs the model on the PREVIOUS observation there), zeros when it ended by done (buffer.py:124,155-156)
-        last_rows = slots * (S + 1) + size
-        if st.compact:   # the packed row of this step's mask went to the row before (comm_mask(out_bits=...) in step)
-            prev = st.comm_bits[last_rows - 1]
-            st.comm_bits[last_rows] = torch.where(done[:, None, None], torch.zeros_like(prev), prev)
-        else:
-            st.comm_mask[last_rows] = torch.where(done[:, None, None], torch.zeros_like(comm[idt]), comm[idt])
+        st.close_comm(slots * (S + 1) + size, done)                             # comm_buf[size]
         # initial priorities (buffer.py:170-177) and their insertion (worker.py:87-94)
         leaves = (slots[:, None] * S + torch.arange(S, device=self.dev)[None, :])
         rew = st.rew_buf[leaves].float()

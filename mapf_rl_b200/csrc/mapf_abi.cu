@@ -5,6 +5,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <new>
+#include <type_traits>
 
 #include "mapf_common.cuh"
 
@@ -78,6 +79,58 @@ struct DeviceGuard {
 };
 
 bool aligned16(const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+// MAPF_ECUDA with `fn`'s message when the process sees no device
+int require_device(const char *fn)
+{
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
+        mapf_set_error(std::string(fn) + ": no CUDA device (this library has no CPU fallback)");
+        return MAPF_ECUDA;
+    }
+    return MAPF_OK;
+}
+
+// the arguments only mapf_replay_gather_present takes
+struct PresentRowArgs {
+    const uint8_t *agents;
+    const int32_t *first;
+    int64_t out_rows;
+};
+
+// The checks of the three window gathers, every MAPF_EINVAL before MAPF_ECUDA.  A compact store's obs_bits must be 16-byte
+// aligned (the gathers load packed frames 16 bytes at a time); the present gather (pr != nullptr) stages at most 64 window
+// frames and writes its observations 16 bytes at a time.
+template <typename View>
+int check_window_gather(const char *fn, const View *view, const int64_t *d_idx, int64_t batch, const mapf_replay_batch *out,
+                        const PresentRowArgs *pr = nullptr)
+{
+    constexpr bool compact = std::is_same_v<View, mapf_replay_view_compact>;
+    if (!view || !out || batch < 0 || (batch > 0 && !d_idx) ||
+        (pr && (pr->out_rows < 0 || (batch > 0 && (!pr->first || !pr->agents))))) {
+        mapf_set_error(std::string(fn) + ": NULL argument");
+        return MAPF_EINVAL;
+    }
+    if (view->num_agents < 1 || view->num_agents > MAPF_MAX_AGENTS || view->max_steps < 1 || view->bt_steps < 1 ||
+        view->forward_steps < 1 || view->latent_dim < 1 || batch > 65535 ||
+        (pr && ((int64_t)view->bt_steps + view->forward_steps > 64 || pr->out_rows > 0x7fffffff))) {
+        mapf_set_error(std::string(fn) + (pr ? ": bad dimensions (bt_steps + forward_steps <= 64, batch <= 65535)"
+                                             : ": bad dimensions (batch <= 65535)"));
+        return MAPF_EINVAL;
+    }
+    const void *obs, *comm;
+    if constexpr (compact) obs = view->obs_bits, comm = view->comm_bits;
+    else obs = view->obs_buf, comm = view->comm_buf;
+    if (!obs || !comm || !view->hid_buf || !view->act_buf || !view->rew_buf || !view->done_buf || !view->size_buf || !out->obs ||
+        !out->comm_mask || !out->hidden || !out->action || !out->reward || !out->done || !out->steps || !out->bt_steps ||
+        (compact && !aligned16(obs)) || (pr && !aligned16(out->obs))) {
+        mapf_set_error(std::string(fn) + (pr        ? ": NULL buffer, or obs_bits or the obs output not 16-byte aligned"
+                                          : compact ? ": NULL buffer or obs_bits not 16-byte aligned"
+                                                    : ": NULL buffer"));
+        return MAPF_EINVAL;
+    }
+    return require_device(fn);
+}
 
 bool host_is_pinned(const void *p)
 {
@@ -1429,27 +1482,8 @@ int mapf_actor_td(const float *d_rew, const float *d_q, const uint8_t *d_act, co
 int mapf_replay_gather(const mapf_replay_view *view, const int64_t *d_idx, int64_t batch, const mapf_replay_batch *out,
                        int32_t *d_err, void *stream)
 {
-    if (!view || !out || batch < 0 || (batch > 0 && !d_idx)) {
-        mapf_set_error("mapf_replay_gather: NULL argument");
-        return MAPF_EINVAL;
-    }
-    if (view->num_agents < 1 || view->num_agents > MAPF_MAX_AGENTS || view->max_steps < 1 || view->bt_steps < 1 ||
-        view->forward_steps < 1 || view->latent_dim < 1 || batch > 65535) {
-        mapf_set_error("mapf_replay_gather: bad dimensions (batch <= 65535)");
-        return MAPF_EINVAL;
-    }
-    if (!view->obs_buf || !view->comm_buf || !view->hid_buf || !view->act_buf || !view->rew_buf || !view->done_buf ||
-        !view->size_buf || !out->obs || !out->comm_mask || !out->hidden || !out->action || !out->reward || !out->done ||
-        !out->steps || !out->bt_steps) {
-        mapf_set_error("mapf_replay_gather: NULL buffer");
-        return MAPF_EINVAL;
-    }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        mapf_set_error("mapf_replay_gather: no CUDA device (this library has no CPU fallback)");
-        return MAPF_ECUDA;
-    }
-    if (batch == 0) return MAPF_OK;
+    const int rc = check_window_gather("mapf_replay_gather", view, d_idx, batch, out);
+    if (rc != MAPF_OK || batch == 0) return rc;
     return mapf_launch_replay_gather(view, d_idx, batch, out, d_err, static_cast<cudaStream_t>(stream));
 }
 
@@ -1464,39 +1498,16 @@ int mapf_obs_unpack(const uint8_t *d_bits_base, const int64_t *d_rows, int64_t c
         mapf_set_error("mapf_obs_unpack: num_agents outside 1..128, unknown dtype or count >= 2^31");
         return MAPF_EINVAL;
     }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        mapf_set_error("mapf_obs_unpack: no CUDA device (this library has no CPU fallback)");
-        return MAPF_ECUDA;
-    }
-    if (count == 0) return MAPF_OK;
+    const int rc = require_device("mapf_obs_unpack");
+    if (rc != MAPF_OK || count == 0) return rc;
     return mapf_launch_obs_unpack(d_bits_base, d_rows, count, num_agents, dtype, d_out, static_cast<cudaStream_t>(stream));
 }
 
 int mapf_replay_gather_compact(const mapf_replay_view_compact *view, const int64_t *d_idx, int64_t batch,
                                const mapf_replay_batch *out, int32_t *d_err, void *stream)
 {
-    if (!view || !out || batch < 0 || (batch > 0 && !d_idx)) {
-        mapf_set_error("mapf_replay_gather_compact: NULL argument");
-        return MAPF_EINVAL;
-    }
-    if (view->num_agents < 1 || view->num_agents > MAPF_MAX_AGENTS || view->max_steps < 1 || view->bt_steps < 1 ||
-        view->forward_steps < 1 || view->latent_dim < 1 || batch > 65535) {
-        mapf_set_error("mapf_replay_gather_compact: bad dimensions (batch <= 65535)");
-        return MAPF_EINVAL;
-    }
-    if (!view->obs_bits || !view->comm_bits || !view->hid_buf || !view->act_buf || !view->rew_buf || !view->done_buf ||
-        !view->size_buf || !out->obs || !out->comm_mask || !out->hidden || !out->action || !out->reward || !out->done ||
-        !out->steps || !out->bt_steps || !aligned16(view->obs_bits)) {
-        mapf_set_error("mapf_replay_gather_compact: NULL buffer or obs_bits not 16-byte aligned");
-        return MAPF_EINVAL;
-    }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        mapf_set_error("mapf_replay_gather_compact: no CUDA device (this library has no CPU fallback)");
-        return MAPF_ECUDA;
-    }
-    if (batch == 0) return MAPF_OK;
+    const int rc = check_window_gather("mapf_replay_gather_compact", view, d_idx, batch, out);
+    if (rc != MAPF_OK || batch == 0) return rc;
     return mapf_launch_replay_gather_compact(view, d_idx, batch, out, d_err, static_cast<cudaStream_t>(stream));
 }
 
@@ -1513,12 +1524,8 @@ int mapf_obs_unpack_present(const uint8_t *d_bits_base, const int64_t *d_rows, c
         mapf_set_error("mapf_obs_unpack_present: num_agents outside 1..128, unknown dtype, or count or out_rows >= 2^31");
         return MAPF_EINVAL;
     }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        mapf_set_error("mapf_obs_unpack_present: no CUDA device (this library has no CPU fallback)");
-        return MAPF_ECUDA;
-    }
-    if (out_rows == 0) return MAPF_OK;
+    const int rc = require_device("mapf_obs_unpack_present");
+    if (rc != MAPF_OK || out_rows == 0) return rc;
     return mapf_launch_obs_unpack_present(d_bits_base, d_rows, d_n, d_first, count, num_agents, out_rows, dtype, d_out,
                                           static_cast<cudaStream_t>(stream));
 }
@@ -1527,28 +1534,9 @@ int mapf_replay_gather_present(const mapf_replay_view_compact *view, const uint8
                                const int32_t *d_first, int64_t batch, int64_t out_rows, const mapf_replay_batch *out,
                                int32_t *d_err, void *stream)
 {
-    if (!view || !out || batch < 0 || out_rows < 0 || (batch > 0 && (!d_idx || !d_first || !d_agents))) {
-        mapf_set_error("mapf_replay_gather_present: NULL argument");
-        return MAPF_EINVAL;
-    }
-    if (view->num_agents < 1 || view->num_agents > MAPF_MAX_AGENTS || view->max_steps < 1 || view->bt_steps < 1 ||
-        view->forward_steps < 1 || view->latent_dim < 1 || view->bt_steps + view->forward_steps > 64 || batch > 65535 ||
-        out_rows > 0x7fffffff) {
-        mapf_set_error("mapf_replay_gather_present: bad dimensions (bt_steps + forward_steps <= 64, batch <= 65535)");
-        return MAPF_EINVAL;
-    }
-    if (!view->obs_bits || !view->comm_bits || !view->hid_buf || !view->act_buf || !view->rew_buf || !view->done_buf ||
-        !view->size_buf || !out->obs || !out->comm_mask || !out->hidden || !out->action || !out->reward || !out->done ||
-        !out->steps || !out->bt_steps || !aligned16(view->obs_bits) || !aligned16(out->obs)) {
-        mapf_set_error("mapf_replay_gather_present: NULL buffer, or obs_bits or the obs output not 16-byte aligned");
-        return MAPF_EINVAL;
-    }
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        mapf_set_error("mapf_replay_gather_present: no CUDA device (this library has no CPU fallback)");
-        return MAPF_ECUDA;
-    }
-    if (batch == 0 && out_rows == 0) return MAPF_OK;
+    const PresentRowArgs pr{d_agents, d_first, out_rows};
+    const int rc = check_window_gather("mapf_replay_gather_present", view, d_idx, batch, out, &pr);
+    if (rc != MAPF_OK || (batch == 0 && out_rows == 0)) return rc;
     return mapf_launch_replay_gather_present(view, d_agents, d_idx, d_first, batch, out_rows, out, d_err,
                                              static_cast<cudaStream_t>(stream));
 }

@@ -15,52 +15,77 @@
 
 namespace {
 
+// parameters of the (W + 1, batch) grid kernels over a dense or a compact store
+template <typename View>
 struct GatherParams {
-    mapf_replay_view v;
+    View v;
     mapf_replay_batch o;
     const int64_t *idx;
-    int64_t batch;
     int32_t *err;
 };
 
 // two bool bytes (b0 at bits 0-7, b1 at bits 16-23) -> two fp16 (1.0 = 0x3C00)
 __device__ __forceinline__ uint32_t bools_to_half2(uint32_t spread) { return spread * 0x3C00u; }
 
-// the per-sample scalars of a gathered window (dense and compact views share these fields)
+// the sampled window of one leaf (worker.py:115-137)
+struct Window {
+    int64_t idx, g;  // leaf and its episode slot (worker.py:115)
+    int t, size;     // step of the leaf in the episode (:116) and the episode's size
+    int steps;       // forward steps, min(forward_steps, size - t) (:122)
+    int f0, len;     // the window starts at the episode start until bt_steps frames of history exist (:124-137);
+                     // frames j >= len are zero padding (:139-142)
+    int64_t row0;    // store row of window frame 0
+    __device__ __forceinline__ int64_t row(const int j) const { return row0 + j; }
+    // leaf of the stored hidden state, t - bt_steps (:137); -1 (zeros) while t < bt_steps (:127,:132)
+    __device__ __forceinline__ int64_t hidden_leaf(const int bt_steps) const { return t >= bt_steps ? idx - bt_steps : -1; }
+};
+
+// dense and compact views share these fields
+template <typename View>
+__device__ __forceinline__ Window leaf_window(const View &v, const int64_t idx)
+{
+    Window w;
+    w.idx = idx;
+    w.g = idx / v.max_steps;
+    w.t = (int)(idx - w.g * v.max_steps);
+    w.size = v.size_buf[w.g];
+    w.steps = min(v.forward_steps, w.size - w.t);
+    w.f0 = max(0, w.t + 1 - v.bt_steps);
+    w.len = w.t + 1 + w.steps - w.f0;
+    w.row0 = w.g * (v.max_steps + 1) + w.f0;
+    return w;
+}
+
+// the per-sample scalars of a gathered window
 template <typename View>
 __device__ __forceinline__ void gather_scalars(const View &v, const mapf_replay_batch &o, int32_t *err, const int64_t b,
-                                               const int64_t idx, const int64_t g, const int t, const int size, const int steps)
+                                               const Window &w)
 {
-    if (t >= size && err) atomicOr(err, 1);  // the reference asserts local_idx < size (worker.py:120)
-    o.action[b] = v.act_buf[idx];                                               // :143
-    o.reward[b] = v.rew_buf[idx];                                               // :144
-    const bool done = (t == size - 1) && v.done_buf[g] != 0;                    // :145-148
+    if (w.t >= w.size && err) atomicOr(err, 1);  // the reference asserts local_idx < size (worker.py:120)
+    o.action[b] = v.act_buf[w.idx];                                             // :143
+    o.reward[b] = v.rew_buf[w.idx];                                             // :144
+    const bool done = (w.t == w.size - 1) && v.done_buf[w.g] != 0;              // :145-148
     o.done[b] = done ? 0x3C00 : 0;
-    o.steps[b] = __half_as_ushort(__int2half_rn(steps));                        // :171 HalfTensor(b_steps)
-    o.bt_steps[b] = min(t + 1, v.bt_steps);                                     // :150
+    o.steps[b] = __half_as_ushort(__int2half_rn(w.steps));                      // :171 HalfTensor(b_steps)
+    o.bt_steps[b] = min(w.t + 1, v.bt_steps);                                   // :150
 }
 
 __global__ void __launch_bounds__(256)
-replay_gather_kernel(const GatherParams p)
+replay_gather_kernel(const GatherParams<mapf_replay_view> p)
 {
     const mapf_replay_view &v = p.v;
     const int W = v.bt_steps + v.forward_steps;
     const int j = blockIdx.x;  // frame of the window, or W = the hidden-state / scalar block
     const int64_t b = blockIdx.y;
-    const int64_t idx = p.idx[b];
-    const int64_t g = idx / v.max_steps;             // worker.py:115
-    const int t = (int)(idx - g * v.max_steps);      // worker.py:116
-    const int size = v.size_buf[g];
-    const int steps = min(v.forward_steps, size - t);  // worker.py:122
-    const int f0 = max(0, t + 1 - v.bt_steps);         // worker.py:124-137: the window starts at the episode start
-    const int len = t + 1 + steps - f0;                //                   until bt_steps frames of history exist
+    const Window w = leaf_window(v, p.idx[b]);
     const int N = v.num_agents;
 
     if (j == W) {
-        // stored hidden state of frame t - bt_steps (worker.py:137), zeros while t < bt_steps (:127,:132)
+        // the window's stored hidden state, zeros while t < bt_steps
         const int HB = N * v.latent_dim;  // halfs
         uint16_t *dst = p.o.hidden + (size_t)b * HB;
-        const uint16_t *src = t >= v.bt_steps ? v.hid_buf + (size_t)(idx - v.bt_steps) * HB : nullptr;
+        const int64_t hid = w.hidden_leaf(v.bt_steps);
+        const uint16_t *src = hid >= 0 ? v.hid_buf + (size_t)hid * HB : nullptr;
         if ((HB & 7) == 0) {
             const uint4 *s4 = reinterpret_cast<const uint4 *>(src);
             uint4 *d4 = reinterpret_cast<uint4 *>(dst);
@@ -68,12 +93,12 @@ replay_gather_kernel(const GatherParams p)
         } else {
             for (int k = threadIdx.x; k < HB; k += blockDim.x) dst[k] = src ? src[k] : (uint16_t)0;
         }
-        if (threadIdx.x == 0) gather_scalars(v, p.o, p.err, b, idx, g, t, size, steps);
+        if (threadIdx.x == 0) gather_scalars(v, p.o, p.err, b, w);
         return;
     }
 
-    const bool live = j < len;  // frames past the window are zero padding (worker.py:139-142)
-    const int64_t row = g * (v.max_steps + 1) + f0 + j;
+    const bool live = j < w.len;
+    const int64_t row = w.row(j);
     // ---- observation frame: N * 486 bool bytes -> fp16 ----
     {
         const int FB = N * MAPF_OBS_BYTES_PER_AGENT;
@@ -197,38 +222,38 @@ obs_unpack_kernel(const uint8_t *__restrict__ bits, const int64_t *__restrict__ 
     expand_frame<ONE>(s_frame, N, true, dst, (FB & 7) == 0);
 }
 
-struct CompactGatherParams {
-    mapf_replay_view_compact v;
-    mapf_replay_batch o;
-    const int64_t *idx;
-    int32_t *err;
-};
+// comm mask frame `row` of a compact store: packed rows (N rows of ceil(N / 8) bytes) -> N * N bool bytes, zeros if !live
+__device__ __forceinline__ void expand_comm_frame(const uint8_t *comm_bits, const int64_t row, const int N, const bool live,
+                                                  uint8_t *dst)
+{
+    const int CW = (N + 7) >> 3;
+    const uint8_t *src = comm_bits + (size_t)row * N * CW;
+    for (int k = threadIdx.x; k < N * N; k += blockDim.x) {
+        const int i = k / N, c = k - i * N;
+        dst[k] = live ? (uint8_t)((__ldg(src + i * CW + (c >> 3)) >> (c & 7)) & 1u) : (uint8_t)0;
+    }
+}
 
 // replay_gather_kernel over a compact store: the same window, padding and scalars; the observation frame is expanded from
 // bits to fp16 (eight halves per 16-byte store), the comm mask from bits to bytes, and the one stored hidden vector of the
 // sample is written into each of its N rows
 __global__ void __launch_bounds__(256)
-replay_gather_compact_kernel(const CompactGatherParams p)
+replay_gather_compact_kernel(const GatherParams<mapf_replay_view_compact> p)
 {
     __shared__ __align__(16) uint8_t s_frame[MAPF_MAX_AGENTS * MAPF_OBS_PACKED_BYTES_PER_AGENT];
     const mapf_replay_view_compact &v = p.v;
     const int W = v.bt_steps + v.forward_steps;
     const int j = blockIdx.x;
     const int64_t b = blockIdx.y;
-    const int64_t idx = p.idx[b];
-    const int64_t g = idx / v.max_steps;
-    const int t = (int)(idx - g * v.max_steps);
-    const int size = v.size_buf[g];
-    const int steps = min(v.forward_steps, size - t);
-    const int f0 = max(0, t + 1 - v.bt_steps);
-    const int len = t + 1 + steps - f0;
+    const Window w = leaf_window(v, p.idx[b]);
     const int N = v.num_agents;
 
     if (j == W) {
-        // the stored hidden vector of frame t - bt_steps in every agent's row, zeros while t < bt_steps
+        // the window's stored hidden vector in every agent's row, zeros while t < bt_steps
         const int D = v.latent_dim;
         uint16_t *dst = p.o.hidden + (size_t)b * N * D;
-        const uint16_t *src = t >= v.bt_steps ? v.hid_buf + (size_t)(idx - v.bt_steps) * D : nullptr;
+        const int64_t hid = w.hidden_leaf(v.bt_steps);
+        const uint16_t *src = hid >= 0 ? v.hid_buf + (size_t)hid * D : nullptr;
         if ((D & 7) == 0) {
             const int D8 = D >> 3;
             const uint4 *s4 = reinterpret_cast<const uint4 *>(src);
@@ -237,24 +262,17 @@ replay_gather_compact_kernel(const CompactGatherParams p)
         } else {
             for (int k = threadIdx.x; k < N * D; k += blockDim.x) dst[k] = src ? src[k % D] : (uint16_t)0;
         }
-        if (threadIdx.x == 0) gather_scalars(v, p.o, p.err, b, idx, g, t, size, steps);
+        if (threadIdx.x == 0) gather_scalars(v, p.o, p.err, b, w);
         return;
     }
 
-    const bool live = j < len;
-    const int64_t row = g * (v.max_steps + 1) + f0 + j;
+    const bool live = j < w.len;
+    const int64_t row = w.row(j);
     const int FB = N * MAPF_OBS_BYTES_PER_AGENT;
     if (live) load_frame(s_frame, v.obs_bits + (size_t)row * N * MAPF_OBS_PACKED_BYTES_PER_AGENT, N);
     __syncthreads();
     expand_frame<0x3C00u>(s_frame, N, live, p.o.obs + ((size_t)b * W + j) * FB, (FB & 7) == 0);
-    // ---- communication mask frame: packed rows -> N * N bool bytes ----
-    const int CW = (N + 7) >> 3;
-    const uint8_t *src = v.comm_bits + (size_t)row * N * CW;
-    uint8_t *dst = p.o.comm_mask + ((size_t)b * W + j) * N * N;
-    for (int k = threadIdx.x; k < N * N; k += blockDim.x) {
-        const int i = k / N, c = k - i * N;
-        dst[k] = live ? (uint8_t)((__ldg(src + i * CW + (c >> 3)) >> (c & 7)) & 1u) : (uint8_t)0;
-    }
+    expand_comm_frame(v.comm_bits, row, N, live, p.o.comm_mask + ((size_t)b * W + j) * N * N);
 }
 
 // ---- present-agent rows (mapf_rl_b200/present.py): output row first[f] + a holds agent a < min(n[f], N) of frame f; first is
@@ -356,32 +374,19 @@ __global__ void __launch_bounds__(256)
 replay_gather_present_kernel(const PresentGatherParams p)
 {
     __shared__ __align__(16) uint8_t s_rows[kGatherRunRows * kGatherMaxW * MAPF_OBS_PACKED_BYTES_PER_AGENT];
-    __shared__ int64_t s_src[kGatherRunRows];  // leaf of the row's sample, -1: zero row
-    __shared__ int s_a[kGatherRunRows], s_f0[kGatherRunRows], s_len[kGatherRunRows];
+    __shared__ int64_t s_obs[kGatherRunRows];  // packed row of the row's agent in window frame 0
+    __shared__ int64_t s_hid[kGatherRunRows];  // leaf of the row's hidden vector, -1: zeros
+    __shared__ int s_len[kGatherRunRows];      // live window frames, 0 in zero rows
     const mapf_replay_view_compact &v = p.v;
     const int W = v.bt_steps + v.forward_steps;
     const int N = v.num_agents;
 
     if ((int)blockIdx.x >= p.runs) {
         const int64_t b = blockIdx.x - p.runs;
-        const int64_t idx = p.idx[b];
-        const int64_t g = idx / v.max_steps;
-        const int t = (int)(idx - g * v.max_steps);
-        const int size = v.size_buf[g];
-        const int steps = min(v.forward_steps, size - t);
-        const int f0 = max(0, t + 1 - v.bt_steps);
-        const int len = t + 1 + steps - f0;
-        if (threadIdx.x == 0) gather_scalars(v, p.o, p.err, b, idx, g, t, size, steps);
-        const int CW = (N + 7) >> 3;
-        for (int j = 0; j < W; ++j) {
-            const bool live = j < len;
-            const uint8_t *src = v.comm_bits + (size_t)(g * (v.max_steps + 1) + f0 + j) * N * CW;
-            uint8_t *dst = p.o.comm_mask + ((size_t)b * W + j) * N * N;
-            for (int k = threadIdx.x; k < N * N; k += blockDim.x) {
-                const int i = k / N, c = k - i * N;
-                dst[k] = live ? (uint8_t)((__ldg(src + i * CW + (c >> 3)) >> (c & 7)) & 1u) : (uint8_t)0;
-            }
-        }
+        const Window w = leaf_window(v, p.idx[b]);
+        if (threadIdx.x == 0) gather_scalars(v, p.o, p.err, b, w);
+        for (int j = 0; j < W; ++j)
+            expand_comm_frame(v.comm_bits, w.row(j), N, j < w.len, p.o.comm_mask + ((size_t)b * W + j) * N * N);
         return;
     }
 
@@ -389,27 +394,24 @@ replay_gather_present_kernel(const PresentGatherParams p)
     const int nrows = (int)min((int64_t)kGatherRunRows, p.out_rows - r0);
     if (threadIdx.x < kGatherRunRows) {
         const int i = threadIdx.x;
-        int64_t src = -1;
-        int a = 0, f0 = 0, len = 0;
+        int64_t obs = 0, hid = -1;
+        int len = 0;
         if (i < nrows) {
             const int64_t m = r0 + i;
             const int b = present_frame(p.first, p.batch, m);
             if (b >= 0) {
                 const int64_t idx = p.idx[b];
-                const int64_t g = idx / v.max_steps;
-                a = (int)(m - p.first[b]);
-                if (a < min((int)p.agents[g], N)) {
-                    const int t = (int)(idx - g * v.max_steps);
-                    const int steps = min(v.forward_steps, v.size_buf[g] - t);
-                    f0 = max(0, t + 1 - v.bt_steps);
-                    len = t + 1 + steps - f0;
-                    src = idx;
+                const int a = (int)(m - p.first[b]);
+                if (a < min((int)p.agents[idx / v.max_steps], N)) {
+                    const Window w = leaf_window(v, idx);
+                    obs = w.row(0) * N + a;
+                    hid = w.hidden_leaf(v.bt_steps);
+                    len = w.len;
                 }
             }
         }
-        s_src[i] = src;
-        s_a[i] = a;
-        s_f0[i] = f0;
+        s_obs[i] = obs;
+        s_hid[i] = hid;
         s_len[i] = len;
     }
     __syncthreads();
@@ -417,25 +419,34 @@ replay_gather_present_kernel(const PresentGatherParams p)
     for (int k = threadIdx.x; k < kGatherRunRows * W * 4; k += blockDim.x) {
         const int i = k / (W * 4), j = (k >> 2) - i * W;
         uint4 x = make_uint4(0, 0, 0, 0);
-        const int64_t idx = s_src[i];
-        if (idx >= 0 && j < s_len[i]) {
-            const int64_t g = idx / v.max_steps;
-            const int64_t row = g * (v.max_steps + 1) + s_f0[i] + j;
-            x = __ldg(reinterpret_cast<const uint4 *>(v.obs_bits + ((size_t)row * N + s_a[i]) * MAPF_OBS_PACKED_BYTES_PER_AGENT) + (k & 3));
+        if (j < s_len[i]) {
+            const uint8_t *src = v.obs_bits + (size_t)(s_obs[i] + (int64_t)j * N) * MAPF_OBS_PACKED_BYTES_PER_AGENT;
+            x = __ldg(reinterpret_cast<const uint4 *>(src) + (k & 3));
         }
         reinterpret_cast<uint4 *>(s_rows)[k] = x;
     }
     __syncthreads();
     expand_run<0x3C00u>(s_rows, kGatherRunRows * W, (int64_t)nrows * W * MAPF_OBS_BYTES_PER_AGENT,
                         p.o.obs + (size_t)r0 * W * MAPF_OBS_BYTES_PER_AGENT);
-    // hidden: the sample's stored vector of frame t - bt_steps, zeros while t < bt_steps and in zero rows
+    // hidden: the sample's stored vector, zeros while t < bt_steps and in zero rows
     const int D = v.latent_dim;
     for (int k = threadIdx.x; k < nrows * D; k += blockDim.x) {
         const int i = k / D, c = k - i * D;
-        const int64_t idx = s_src[i];
-        const bool has = idx >= 0 && idx - (idx / v.max_steps) * v.max_steps >= v.bt_steps;
-        p.o.hidden[(size_t)(r0 + i) * D + c] = has ? v.hid_buf[(size_t)(idx - v.bt_steps) * D + c] : (uint16_t)0;
+        const int64_t hid = s_hid[i];
+        p.o.hidden[(size_t)(r0 + i) * D + c] = hid >= 0 ? v.hid_buf[(size_t)hid * D + c] : (uint16_t)0;
     }
+}
+
+// the (W + 1, batch) grid: CTA (j, b) writes window frame j of sample b, CTA (W, b) its hidden rows and scalars
+template <typename View>
+int launch_window_gather(void (*kernel)(GatherParams<View>), const View *view, const int64_t *d_idx, int64_t batch,
+                         const mapf_replay_batch *out, int32_t *d_err, cudaStream_t st)
+{
+    const GatherParams<View> p{*view, *out, d_idx, d_err};
+    const int W = view->bt_steps + view->forward_steps;
+    kernel<<<dim3((unsigned)(W + 1), (unsigned)batch), 256, 0, st>>>(p);
+    MAPF_CUDA(cudaGetLastError());
+    return MAPF_OK;
 }
 
 }  // namespace
@@ -490,29 +501,11 @@ int mapf_launch_obs_unpack(const uint8_t *d_bits, const int64_t *d_rows, int64_t
 int mapf_launch_replay_gather_compact(const mapf_replay_view_compact *view, const int64_t *d_idx, int64_t batch,
                                       const mapf_replay_batch *out, int32_t *d_err, cudaStream_t st)
 {
-    CompactGatherParams p;
-    p.v = *view;
-    p.o = *out;
-    p.idx = d_idx;
-    p.err = d_err;
-    const int W = view->bt_steps + view->forward_steps;
-    replay_gather_compact_kernel<<<dim3((unsigned)(W + 1), (unsigned)batch), 256, 0, st>>>(p);
-    MAPF_CUDA(cudaGetLastError());
-    return MAPF_OK;
+    return launch_window_gather(replay_gather_compact_kernel, view, d_idx, batch, out, d_err, st);
 }
 
 int mapf_launch_replay_gather(const mapf_replay_view *view, const int64_t *d_idx, int64_t batch, const mapf_replay_batch *out,
                               int32_t *d_err, cudaStream_t st)
 {
-    GatherParams p;
-    p.v = *view;
-    p.o = *out;
-    p.idx = d_idx;
-    p.batch = batch;
-    p.err = d_err;
-    const int W = view->bt_steps + view->forward_steps;
-    dim3 grid((unsigned)(W + 1), (unsigned)batch);
-    replay_gather_kernel<<<grid, 256, 0, st>>>(p);
-    MAPF_CUDA(cudaGetLastError());
-    return MAPF_OK;
+    return launch_window_gather(replay_gather_kernel, view, d_idx, batch, out, d_err, st);
 }

@@ -23,7 +23,7 @@ from typing import List, Optional
 import numpy as np
 
 from . import _native, config, packed
-from .present import PresentRows
+from .present import PresentRows, unpack_obs_present
 from .buffer import SumTree
 
 
@@ -153,6 +153,43 @@ class ReplayStore:
         row0 = slot * (self.max_steps + 1) + first_frame
         return (self.obs_bits if self.compact else self.obs_buf)[row0:row0 + count]
 
+    def frame_out(self) -> dict:
+        """The keyword argument that makes `BatchedEnvironment.step` / `observe` (with `obs_rows`) write observations into
+        the store's frame rows: `out_obs`, or `out_bits` (packed rows) for a compact store."""
+        return dict(out_bits=self.obs_bits) if self.compact else dict(out_obs=self.obs_buf)
+
+    def current_frames(self, rows, present: Optional[PresentRows] = None):
+        """The observation frames at `rows` (int64 CUDA tensor [B], frame e of environment e) for the Q-network: uint8
+        [B, N, 6, 9, 9], or [M_pad, 6, 9, 9] in the present-agent rows of `present`."""
+        if self.compact:
+            return packed.unpack_obs(self.obs_bits, rows) if present is None else unpack_obs_present(self.obs_bits, rows, present)
+        obs = self.obs_buf.index_select(0, rows)
+        return obs if present is None else present.select(obs.flatten(0, 1))
+
+    def record_comm(self, env, rows):
+        """The comm mask of `env`'s current positions (model.py:196-208) -> uint8 CUDA tensor [B, N, N], also stored at frame
+        `rows` (comm_buf[size] = comm_mask, buffer.py:149)."""
+        if self.compact:
+            return env.comm_mask(out_bits=self.comm_bits, rows=rows)     # the packed rows in the same launch
+        comm = env.comm_mask()
+        self.comm_mask.index_copy_(0, rows, comm)
+        return comm
+
+    def close_comm(self, last_rows, done):
+        """comm_buf[size] of finished episodes (`last_rows`, their frame after the last step): the mask of the last step, which
+        `record_comm` stored at the row before, when the episode was cut at max_steps (worker.py:399-401; the reference re-runs
+        the model on the PREVIOUS observation there), zeros when it ended by `done` (buffer.py:124,155-156)."""
+        torch = _torch()
+        buf = self.comm_bits if self.compact else self.comm_mask
+        prev = buf[last_rows - 1]
+        buf[last_rows] = torch.where(done[:, None, None], torch.zeros_like(prev), prev)
+
+    def write_hidden(self, leaf, hidden):
+        """Agent 0's hidden vector (`hidden` [B, latent]) of the transitions at `leaf`: once in a compact store, in each agent's
+        row of a dense one, as the reference broadcasts it (buffer.py:148, SURVEY q8)."""
+        h = hidden.to(_torch().float16)
+        self.hid_buf[leaf] = h if self.compact else h[:, None, :].expand(-1, self.max_num_agents, -1)
+
     # -- GlobalBuffer.sample_batch (worker.py:106-184) ------------------------------------------------
     def _view(self):
         if self.compact:
@@ -174,44 +211,43 @@ class ReplayStore:
         idx = torch.as_tensor(idxes, dtype=torch.int64).to(self.device).contiguous()
         if present:
             return self._gather_present(idx)
-        B, n, W, dev = int(idx.numel()), self.max_num_agents, self.bt_steps + self.forward_steps, self.device
-        e = lambda shape, dt: torch.empty(shape, dtype=dt, device=dev)
-        out = dict(obs=e((B, W, n, *config.obs_shape), torch.float16), comm_mask=e((B, W, n, n), torch.uint8),
-                   hidden=e((B * n, self.latent_dim), torch.float16), action=e((B,), torch.int64),
+        B, n, W = int(idx.numel()), self.max_num_agents, self.bt_steps + self.forward_steps
+        out, batch = self._outputs(B, (B, W, n), B * n)
+        gather = self._lib.mapf_replay_gather_compact if self.compact else self._lib.mapf_replay_gather
+        _native.check(gather(C.byref(self._view()), C.c_void_p(idx.data_ptr()), B, C.byref(batch),
+                             C.c_void_p(self._err.data_ptr()), self._stream()))
+        return out
+
+    def _outputs(self, B: int, obs_rows, hidden_rows: int):
+        """Uninitialised outputs of a gather of B samples -> (dict, its `ReplayBatch`); obs is [*obs_rows, 6, 9, 9] and hidden
+        [hidden_rows, latent], in padded or present-agent rows."""
+        torch = _torch()
+        n, W = self.max_num_agents, self.bt_steps + self.forward_steps
+        e = lambda shape, dt: torch.empty(shape, dtype=dt, device=self.device)
+        out = dict(obs=e((*obs_rows, *config.obs_shape), torch.float16), comm_mask=e((B, W, n, n), torch.uint8),
+                   hidden=e((hidden_rows, self.latent_dim), torch.float16), action=e((B,), torch.int64),
                    reward=e((B,), torch.float16), done=e((B,), torch.float16), steps=e((B,), torch.float16),
                    bt_steps=e((B,), torch.int64))
-        view = self._view()
         batch = _native.ReplayBatch(*[out[k].data_ptr() for k in ("obs", "comm_mask", "hidden", "action", "reward", "done",
                                                                    "steps", "bt_steps")])
-        gather = self._lib.mapf_replay_gather_compact if self.compact else self._lib.mapf_replay_gather
-        _native.check(gather(C.byref(view), C.c_void_p(idx.data_ptr()), B, C.byref(batch), C.c_void_p(self._err.data_ptr()),
-                             self._stream()))
-        return out
+        return out, batch
 
     def _gather_present(self, idx):
         torch = _torch()
         # an entry above N reads as N, as mapf_replay_gather_present reads it
         counts = self.agents_buf[idx // self.max_steps].clamp(max=self.max_num_agents)
         pr = PresentRows(counts, int(counts.sum(dtype=torch.int64).item()), self.max_num_agents)
+        W = self.bt_steps + self.forward_steps
         if not self.compact:   # the padded gather, indexed: also the reference the kernel is tested against
             out = self.gather(idx)
-            B, W = pr.B, self.bt_steps + self.forward_steps
-            out["obs"] = pr.select(out["obs"].transpose(1, 2).reshape(B * pr.N, W, *config.obs_shape))
+            out["obs"] = pr.select(out["obs"].transpose(1, 2).reshape(pr.B * pr.N, W, *config.obs_shape))
             out["hidden"] = pr.select(out["hidden"])
             out["present"] = pr
             return out
-        B, n, W, dev = pr.B, self.max_num_agents, self.bt_steps + self.forward_steps, self.device
-        e = lambda shape, dt: torch.empty(shape, dtype=dt, device=dev)
-        out = dict(obs=e((pr.M_pad, W, *config.obs_shape), torch.float16), comm_mask=e((B, W, n, n), torch.uint8),
-                   hidden=e((pr.M_pad, self.latent_dim), torch.float16), action=e((B,), torch.int64),
-                   reward=e((B,), torch.float16), done=e((B,), torch.float16), steps=e((B,), torch.float16),
-                   bt_steps=e((B,), torch.int64))
-        view = self._view()
-        batch = _native.ReplayBatch(*[out[k].data_ptr() for k in ("obs", "comm_mask", "hidden", "action", "reward", "done",
-                                                                   "steps", "bt_steps")])
+        out, batch = self._outputs(pr.B, (pr.M_pad, W), pr.M_pad)
         _native.check(self._lib.mapf_replay_gather_present(
-            C.byref(view), C.c_void_p(self.agents_buf.data_ptr()), C.c_void_p(idx.data_ptr()), C.c_void_p(pr.first.data_ptr()),
-            B, pr.M_pad, C.byref(batch), C.c_void_p(self._err.data_ptr()), self._stream()))
+            C.byref(self._view()), C.c_void_p(self.agents_buf.data_ptr()), C.c_void_p(idx.data_ptr()),
+            C.c_void_p(pr.first.data_ptr()), pr.B, pr.M_pad, C.byref(batch), C.c_void_p(self._err.data_ptr()), self._stream()))
         out["present"] = pr
         return out
 
