@@ -528,6 +528,34 @@ int mapf_env_plan_prioritized(mapf_env *env, int32_t horizon, uint8_t *d_actions
 int mapf_env_plan_prioritized_orders(mapf_env *env, int32_t horizon, int32_t orders, uint64_t seed, uint64_t env_offset,
                                      uint8_t *d_actions, int32_t *d_arrival, int32_t *d_order, uint8_t *d_rank, void *stream);
 
+/* Plan improvement by large-neighbourhood search (MAPF-LNS, Li et al., IJCAI 2021) from a plan of the handle's current state,
+ * read and written in place in the layout mapf_env_plan_prioritized writes (an earlier output of this call is valid input):
+ *   d_actions   u8[horizon, B, N]  read; written where an iteration was accepted
+ *   d_arrival   i32[B, N]          read; written where an iteration was accepted
+ *   d_accepted  i32[B]             the accepted iterations; -1 for a failed plan, -2 for an invalid one
+ * Environment e has global index g = env_offset + e, n agents (n_e on a sized handle) on the l x l map.  Agent a < n follows
+ * p_0 = its position, p_t+1 = p_t + delta(actions[t, a]) for t < arrival[a], and parks on its goal for arrival[a] <= t <= H.
+ * Input check, once per environment: an arrival row of -1 (every present agent -1, a failed plan) leaves the environment
+ * unchanged with accepted -1; it is left unchanged with accepted -2 if an action id is > 4, some p_t is off the l x l map or
+ * on an obstacle, p_arrival[a] != goal[a], an action is non-zero at t >= arrival[a], arrival[a] is outside [0, H], two present
+ * agents share a cell at some t in [0, H] or swap cells between t and t + 1.  Rows of absent agents are neither read nor
+ * written.
+ * Iterations i = first_iteration .. first_iteration + iterations - 1: k_a = word 0 of Philox4x32-10 with counter
+ * (g_lo, g_hi, 5 | i << 8, a) and key (seed_lo, seed_hi); the neighbourhood S is the m = min(neighborhood, n) present agents
+ * of smallest (k_a, a), in that order.  The current paths of the agents outside S are reserved as mapf_env_plan_prioritized
+ * reserves a planned path, and the agents of S are planned in order by its rules against them and against the agents of S
+ * planned before.  The iteration is accepted if every agent of S finds a path within the horizon and their arrivals sum to
+ * strictly less than before: the new paths replace the old ones and accepted[e] += 1; otherwise nothing changes.
+ * The result is valid input again and its sum of costs never exceeds the input's; calls split by first_iteration give the
+ * result of one call over the same iterations.  With neighborhood >= n an iteration plans all agents in a fresh order.
+ * MAPF_EINVAL for a horizon outside 1 .. MAPF_PLAN_MAX_HORIZON, iterations < 0, a neighborhood outside 1 .. N,
+ * first_iteration + iterations > 2^24 or a NULL buffer, MAPF_ENOMEM if the planner's scratch (mapf_env_plan_prioritized's,
+ * plus the current and candidate paths, 4 bytes per agent and time step) cannot be allocated.  Reads the handle's state and
+ * writes nothing in it; asynchronous on `stream`. */
+#define MAPF_PLAN_LNS_MAX_ITERATION (1u << 24)
+int mapf_env_plan_lns(mapf_env *env, int32_t horizon, int32_t iterations, int32_t neighborhood, uint64_t seed, uint64_t env_offset,
+                      uint32_t first_iteration, uint8_t *d_actions, int32_t *d_arrival, int32_t *d_accepted, void *stream);
+
 /* ---- CBS expert / solvable-instance generator (search.py:58-442, test.py:23-79; SURVEY 8(f)4) -- HOST code ------------------
  * Conflict-based search over space-time A*: a collision-free set of paths of minimal sum of costs (search.py:17-21), as the
  * action script search.find_path returns (search.py:396-442).  All pointers are HOST memory; no kernel is launched.

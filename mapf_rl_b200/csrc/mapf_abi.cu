@@ -579,6 +579,22 @@ int mapf_env_plan_prioritized_orders(mapf_env *env, int32_t horizon, int32_t ord
     return mapf_launch_plan_orders(env, horizon, orders, seed, env_offset, d_actions, d_arrival, d_order, d_rank, st);
 }
 
+int mapf_env_plan_lns(mapf_env *env, int32_t horizon, int32_t iterations, int32_t neighborhood, uint64_t seed, uint64_t env_offset,
+                      uint32_t first_iteration, uint8_t *d_actions, int32_t *d_arrival, int32_t *d_accepted, void *stream)
+{
+    REQUIRE_ENV(env);
+    if (horizon < 1 || horizon > MAPF_PLAN_MAX_HORIZON || iterations < 0 || neighborhood < 1 || neighborhood > env->d.N ||
+        (uint64_t)first_iteration + (uint64_t)iterations > MAPF_PLAN_LNS_MAX_ITERATION || !d_actions || !d_arrival || !d_accepted) {
+        mapf_set_error("mapf_env_plan_lns: 1 <= horizon <= 1024, iterations >= 0, 1 <= neighborhood <= N, first_iteration + "
+                       "iterations <= 2^24 and non-NULL d_actions, d_arrival, d_accepted required");
+        return MAPF_EINVAL;
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    MAPF_DRAIN(env, st);
+    return mapf_launch_plan_lns(env, horizon, iterations, neighborhood, seed, env_offset, first_iteration, d_actions, d_arrival, d_accepted,
+                                st);
+}
+
 int mapf_env_step_observe_ex(mapf_env *env, const uint8_t *d_actions, uint8_t *d_obs, const int64_t *d_obs_rows, float *d_rewards,
                              uint8_t *d_codes, uint8_t *d_done, int32_t *d_steps, void *stream)
 {

@@ -23,6 +23,17 @@
 // Pass 1 plans every (environment, order) pair as a work item without writing actions and folds (sum of costs, r) of a
 // solved order into the environment's selection word with atomicMin, so the smallest sum of costs wins and ties go to the
 // smallest r whatever the schedule.  Pass 2 re-plans each environment's winning order and writes its results.
+//
+// Plan improvement (mapf_env_plan_lns, DESIGN.md §8 (f)6), large-neighbourhood search from a plan in the layout above: agent
+// a < n follows p_0 = its position, p_t+1 = p_t + delta(actions[t, a]) for t < arrival[a], and parks on its goal from
+// arrival[a] to H.  The input is checked once: a row of -1 (a failed plan) is left as it is with accepted -1; an action id
+// > 4, a p_t off the l x l map or on an obstacle, p_arrival != goal, a move at t >= arrival, an arrival outside [0, H], a
+// shared cell or a swap leave the environment as it is with accepted -2.  Iteration i draws k_a = word 0 of Philox of
+// (g, PURPOSE_LNS | i << 8, a); the neighbourhood S is the min(k, n) agents of smallest (k_a, a), in that order.  The paths
+// of the agents outside S are reserved as a planned path is committed, the agents of S are planned in order by the rules
+// above, and the new paths are kept (accepted += 1) if every agent of S finds one and their arrivals sum to strictly less
+// than before.  One warp runs all iterations of one environment with its tables kept across them; the path search,
+// read-back and commit are the functions plan_body uses.
 #include <algorithm>
 
 #include "mapf_bfs_device.cuh"
@@ -64,9 +75,159 @@ struct OrderArgs {
     uint8_t *rank;               // u8[B, N]: agent a's position in the winning order, 255
 };
 
+struct LnsArgs {
+    int I, K;                    // iterations, neighbourhood size
+    uint32_t first;              // the first iteration's index
+    uint2 key;                   // Philox key (seed)
+    uint64_t env_offset;         // global index of environment 0
+    int32_t *accepted;           // i32[B]: accepted iterations, -1 (failed plan), -2 (invalid plan)
+};
+
 // offsets of action k (environment.py:12): 0 stay, 1 x-1, 2 x+1, 3 y-1, 4 y+1
 __device__ __forceinline__ int act_dx(int k) { return k == 1 ? -1 : (k == 2 ? 1 : 0); }
 __device__ __forceinline__ int act_dy(int k) { return k == 3 ? -1 : (k == 4 ? 1 : 0); }
+
+// A warp's tables: Occ at `occ`, SB_k at occ + k * tbl (k = 1 .. 4), the frontier history F at occ + 5 * tbl, one table =
+// H + 1 time slices of WPT = 32 * RPL * RW words laid out [q][w][lane]; cell (x, y) is bit plan_bit(y) of word plan_cell(x, y).
+// These two are plain inline, not __forceinline__: forced inlining happens before they are simplified and moves the address
+// arithmetic of the planning kernels (more registers and instructions than with the local lambdas they replaced).
+template <int RW, int RPL>
+__device__ inline size_t plan_cell(int x, int y) { return (size_t)((x % RPL) * RW + ((y + 4) >> 5)) * 32 + x / RPL; }
+__device__ inline uint32_t plan_bit(int y) { return 1u << ((y + 4) & 31); }
+
+// The search of one agent from s to g against the reservations in the tables: last_busy(g), then the frontier F(0 .. t*),
+// stored in the history.  Returns t*, or -1 where the agent finds no path within H.
+template <int RW, int RPL>
+__device__ __forceinline__ int plan_search(const uint32_t *const occ, const uint32_t *const sb, uint32_t *const fh, const size_t tbl,
+                                           const int H, const int lane, const BfsFree<RW, RPL> &F, const uchar2 s, const uchar2 g)
+{
+    constexpr int WPT = 32 * RPL * RW;
+    const size_t gi = plan_cell<RW, RPL>(g.x, g.y);
+    const uint32_t gb = plan_bit(g.y);
+    const int gl = g.x / RPL, gq = g.x % RPL, gw = (g.y + 4) >> 5;
+    // last_busy(goal)
+    int lb = -1;
+#pragma unroll 4
+    for (int t = lane; t <= H; t += 32)
+        if (__ldcg(occ + (size_t)t * WPT + gi) & gb) lb = t;
+    lb = __reduce_max_sync(MAPF_FULL_MASK, lb);
+
+    uint32_t f[RPL][RW];
+#pragma unroll
+    for (int q = 0; q < RPL; ++q)
+#pragma unroll
+        for (int w = 0; w < RW; ++w) {
+            f[q][w] = (lane * RPL + q == s.x && ((s.y + 4) >> 5) == w) ? plan_bit(s.y) : 0u;
+            __stcg(fh + (q * RW + w) * 32 + lane, f[q][w]);
+        }
+    auto at_goal = [&](int t) -> bool {
+        uint32_t x = 0;
+#pragma unroll
+        for (int q = 0; q < RPL; ++q)
+#pragma unroll
+            for (int w = 0; w < RW; ++w)
+                if (q == gq && w == gw) x = f[q][w];
+        return __any_sync(MAPF_FULL_MASK, lane == gl && (x & gb)) && t > lb;
+    };
+
+    int tstar = -1;
+    if (at_goal(0)) {
+        tstar = 0;
+    } else if (lb < H) {
+        for (int t = 0; t < H; ++t) {
+            uint32_t on[RPL][RW], sbk[4][RPL][RW];
+#pragma unroll
+            for (int q = 0; q < RPL; ++q)
+#pragma unroll
+                for (int w = 0; w < RW; ++w) {
+                    const size_t o = (size_t)(q * RW + w) * 32 + lane;
+                    on[q][w] = __ldcg(occ + (size_t)(t + 1) * WPT + o);
+#pragma unroll
+                    for (int k = 0; k < 4; ++k) sbk[k][q][w] = __ldcg(sb + (k + 1) * tbl + (size_t)t * WPT + o);
+                }
+            uint32_t nf[RPL][RW];
+            uint32_t any = 0;
+#pragma unroll
+            for (int w = 0; w < RW; ++w) {
+                uint32_t above, below;
+                bfs_rows_around<RW, RPL, 32, false>(f, w, lane, above, below);
+#pragma unroll
+                for (int q = 0; q < RPL; ++q) {
+                    const uint32_t c = f[q][w];
+                    const uint32_t from_dn = q < RPL - 1 ? f[q < RPL - 1 ? q + 1 : q][w] : below;  // action 1 (x-1)
+                    const uint32_t from_up = q > 0 ? f[q > 0 ? q - 1 : 0][w] : above;              // action 2 (x+1)
+                    const uint32_t from_rt = w < RW - 1 ? __funnelshift_r(c, f[q][w < RW - 1 ? w + 1 : w], 1) : c >> 1;  // 3
+                    const uint32_t from_lt = w > 0 ? __funnelshift_l(f[q][w > 0 ? w - 1 : 0], c, 1) : c << 1;            // 4
+                    const uint32_t x = (c | (from_dn & ~sbk[0][q][w]) | (from_up & ~sbk[1][q][w]) | (from_rt & ~sbk[2][q][w]) |
+                                        (from_lt & ~sbk[3][q][w])) & F.v[q][w] & ~on[q][w];
+                    nf[q][w] = x;
+                    any |= x;
+                }
+            }
+#pragma unroll
+            for (int q = 0; q < RPL; ++q)
+#pragma unroll
+                for (int w = 0; w < RW; ++w) {
+                    f[q][w] = nf[q][w];
+                    __stcg(fh + (size_t)(t + 1) * WPT + (q * RW + w) * 32 + lane, nf[q][w]);
+                }
+            if (!__any_sync(MAPF_FULL_MASK, any != 0)) break;
+            if (at_goal(t + 1)) {
+                tstar = t + 1;
+                break;
+            }
+        }
+    }
+    return tstar;
+}
+
+// The path back from (g, t*) into path[0 .. t*] (x << 8 | y): lane k < 5 tests action k, the lowest admissible id wins
+template <int RW, int RPL>
+__device__ __forceinline__ void plan_read_back(const uint32_t *const sb, const uint32_t *const fh, const size_t tbl, const int L, const int lane,
+                                               const uchar2 g, const int tstar, uint16_t *const path)
+{
+    constexpr int WPT = 32 * RPL * RW;
+    int vx = g.x, vy = g.y;
+    if (lane == 0) path[tstar] = (uint16_t)(vx << 8 | vy);
+    for (int t = tstar; t >= 1; --t) {
+        bool ok = false;
+        if (lane < 5) {
+            const int ux = vx - act_dx(lane), uy = vy - act_dy(lane);
+            if (ux >= 0 && ux < L && uy >= 0 && uy < L) {
+                ok = (__ldcg(fh + (size_t)(t - 1) * WPT + plan_cell<RW, RPL>(ux, uy)) & plan_bit(uy)) != 0;
+                if (ok && lane > 0) ok = (__ldcg(sb + lane * tbl + (size_t)(t - 1) * WPT + plan_cell<RW, RPL>(vx, vy)) & plan_bit(vy)) == 0;
+            }
+        }
+        const unsigned m = __ballot_sync(MAPF_FULL_MASK, ok);
+        const int k = m ? __ffs(m) - 1 : 0;
+        vx -= act_dx(k), vy -= act_dy(k);
+        if (lane == 0) path[t - 1] = (uint16_t)(vx << 8 | vy);
+    }
+}
+
+// commit: path[0 .. t*] into Occ(0 .. t*), the goal into Occ(t* .. H), each move's origin into SB_opposite(k); with ACTIONS,
+// agent a's move ids into p.actions of environment e
+template <int RW, int RPL, bool ACTIONS>
+__device__ __forceinline__ void plan_commit(uint32_t *const occ, uint32_t *const sb, const size_t tbl, const int H, const int lane, const uchar2 g,
+                                            const int tstar, const uint16_t *const path, const PlanArgs &p, const unsigned e, const int a)
+{
+    constexpr int WPT = 32 * RPL * RW;
+    for (int t = lane; t <= H; t += 32) {
+        const int c = t <= tstar ? path[t] : (g.x << 8 | g.y);
+        const int x = c >> 8, y = c & 255;
+        uint32_t *o = occ + (size_t)t * WPT + plan_cell<RW, RPL>(x, y);
+        __stcg(o, __ldcg(o) | plan_bit(y));
+        if (t < tstar) {
+            const int x2 = path[t + 1] >> 8, y2 = path[t + 1] & 255;
+            const int k = x2 < x ? 1 : (x2 > x ? 2 : (y2 < y ? 3 : (y2 > y ? 4 : 0)));
+            if (k) {
+                if constexpr (ACTIONS) p.actions[((size_t)t * p.d.B + e) * p.d.N + a] = (uint8_t)k;
+                uint32_t *r = sb + (k & 1 ? k + 1 : k - 1) * tbl + (size_t)t * WPT + plan_cell<RW, RPL>(x, y);
+                __stcg(r, __ldcg(r) | plan_bit(y));
+            }
+        }
+    }
+}
 
 // The planner of one warp, all three kernels' code:
 //   kPlanIndex        plan_pp_kernel: environment e is a work item, its agents planned in index order, results written
@@ -89,8 +250,6 @@ __device__ __forceinline__ void plan_body(const PlanArgs &p, const OrderArgs &or
     uint32_t *const sb = occ;               // SB_k = sb + k * tbl, k = 1 .. 4
     uint32_t *const fh = occ + 5 * tbl;     // frontier history F(0 .. t*)
     uint16_t *const path = s_path[wid];
-    auto cell = [](int x, int y) -> size_t { return (size_t)((x % RPL) * RW + ((y + 4) >> 5)) * 32 + x / RPL; };
-    auto bit = [](int y) -> uint32_t { return 1u << ((y + 4) & 31); };
 
     uint8_t *agent = nullptr;  // the agent at each position of the order
     uint32_t *key = nullptr;
@@ -165,82 +324,7 @@ __device__ __forceinline__ void plan_body(const PlanArgs &p, const OrderArgs &or
             const int a = MODE == kPlanIndex ? j : agent[j];
             const uchar2 s = __ldcg(reinterpret_cast<const uchar2 *>(p.pos) + (size_t)e * d.N + a);
             const uchar2 g = __ldcg(reinterpret_cast<const uchar2 *>(p.goal) + (size_t)e * d.N + a);
-            const size_t gi = cell(g.x, g.y);
-            const uint32_t gb = bit(g.y);
-            const int gl = g.x / RPL, gq = g.x % RPL, gw = (g.y + 4) >> 5;
-            // last_busy(goal)
-            int lb = -1;
-#pragma unroll 4
-            for (int t = lane; t <= H; t += 32)
-                if (__ldcg(occ + (size_t)t * WPT + gi) & gb) lb = t;
-            lb = __reduce_max_sync(MAPF_FULL_MASK, lb);
-
-            uint32_t f[RPL][RW];
-#pragma unroll
-            for (int q = 0; q < RPL; ++q)
-#pragma unroll
-                for (int w = 0; w < RW; ++w) {
-                    f[q][w] = (lane * RPL + q == s.x && ((s.y + 4) >> 5) == w) ? bit(s.y) : 0u;
-                    __stcg(fh + (q * RW + w) * 32 + lane, f[q][w]);
-                }
-            auto at_goal = [&](int t) -> bool {
-                uint32_t x = 0;
-#pragma unroll
-                for (int q = 0; q < RPL; ++q)
-#pragma unroll
-                    for (int w = 0; w < RW; ++w)
-                        if (q == gq && w == gw) x = f[q][w];
-                return __any_sync(MAPF_FULL_MASK, lane == gl && (x & gb)) && t > lb;
-            };
-
-            int tstar = -1;
-            if (at_goal(0)) {
-                tstar = 0;
-            } else if (lb < H) {
-                for (int t = 0; t < H; ++t) {
-                    uint32_t on[RPL][RW], sbk[4][RPL][RW];
-#pragma unroll
-                    for (int q = 0; q < RPL; ++q)
-#pragma unroll
-                        for (int w = 0; w < RW; ++w) {
-                            const size_t o = (size_t)(q * RW + w) * 32 + lane;
-                            on[q][w] = __ldcg(occ + (size_t)(t + 1) * WPT + o);
-#pragma unroll
-                            for (int k = 0; k < 4; ++k) sbk[k][q][w] = __ldcg(sb + (k + 1) * tbl + (size_t)t * WPT + o);
-                        }
-                    uint32_t nf[RPL][RW];
-                    uint32_t any = 0;
-#pragma unroll
-                    for (int w = 0; w < RW; ++w) {
-                        uint32_t above, below;
-                        bfs_rows_around<RW, RPL, 32, false>(f, w, lane, above, below);
-#pragma unroll
-                        for (int q = 0; q < RPL; ++q) {
-                            const uint32_t c = f[q][w];
-                            const uint32_t from_dn = q < RPL - 1 ? f[q < RPL - 1 ? q + 1 : q][w] : below;  // action 1 (x-1)
-                            const uint32_t from_up = q > 0 ? f[q > 0 ? q - 1 : 0][w] : above;              // action 2 (x+1)
-                            const uint32_t from_rt = w < RW - 1 ? __funnelshift_r(c, f[q][w < RW - 1 ? w + 1 : w], 1) : c >> 1;  // 3
-                            const uint32_t from_lt = w > 0 ? __funnelshift_l(f[q][w > 0 ? w - 1 : 0], c, 1) : c << 1;            // 4
-                            const uint32_t x = (c | (from_dn & ~sbk[0][q][w]) | (from_up & ~sbk[1][q][w]) | (from_rt & ~sbk[2][q][w]) |
-                                                (from_lt & ~sbk[3][q][w])) & F.v[q][w] & ~on[q][w];
-                            nf[q][w] = x;
-                            any |= x;
-                        }
-                    }
-#pragma unroll
-                    for (int q = 0; q < RPL; ++q)
-#pragma unroll
-                        for (int w = 0; w < RW; ++w) {
-                            f[q][w] = nf[q][w];
-                            __stcg(fh + (size_t)(t + 1) * WPT + (q * RW + w) * 32 + lane, nf[q][w]);
-                        }
-                    if (!__any_sync(MAPF_FULL_MASK, any != 0)) break;
-                    if (at_goal(t + 1)) {
-                        tstar = t + 1;
-                        break;
-                    }
-                }
-            }
+            const int tstar = plan_search<RW, RPL>(occ, sb, fh, tbl, H, lane, F, s, g);
             __syncwarp();
 
             if (tstar < 0) {  // the environment (the order) fails: no plan, no actions, arrival row -1
@@ -253,41 +337,9 @@ __device__ __forceinline__ void plan_body(const PlanArgs &p, const OrderArgs &or
                 break;
             }
 
-            // back from (goal, t*): lane k < 5 tests action k, the lowest admissible id wins
-            int vx = g.x, vy = g.y;
-            if (lane == 0) path[tstar] = (uint16_t)(vx << 8 | vy);
-            for (int t = tstar; t >= 1; --t) {
-                bool ok = false;
-                if (lane < 5) {
-                    const int ux = vx - act_dx(lane), uy = vy - act_dy(lane);
-                    if (ux >= 0 && ux < d.L && uy >= 0 && uy < d.L) {
-                        ok = (__ldcg(fh + (size_t)(t - 1) * WPT + cell(ux, uy)) & bit(uy)) != 0;
-                        if (ok && lane > 0) ok = (__ldcg(sb + lane * tbl + (size_t)(t - 1) * WPT + cell(vx, vy)) & bit(vy)) == 0;
-                    }
-                }
-                const unsigned m = __ballot_sync(MAPF_FULL_MASK, ok);
-                const int k = m ? __ffs(m) - 1 : 0;
-                vx -= act_dx(k), vy -= act_dy(k);
-                if (lane == 0) path[t - 1] = (uint16_t)(vx << 8 | vy);
-            }
+            plan_read_back<RW, RPL>(sb, fh, tbl, d.L, lane, g, tstar, path);
             __syncwarp();
-
-            // commit: the path into Occ(0 .. t*), the goal into Occ(t* .. H), each move's origin into SB_opposite(k)
-            for (int t = lane; t <= H; t += 32) {
-                const int c = t <= tstar ? path[t] : (g.x << 8 | g.y);
-                const int x = c >> 8, y = c & 255;
-                uint32_t *o = occ + (size_t)t * WPT + cell(x, y);
-                __stcg(o, __ldcg(o) | bit(y));
-                if (t < tstar) {
-                    const int x2 = path[t + 1] >> 8, y2 = path[t + 1] & 255;
-                    const int k = x2 < x ? 1 : (x2 > x ? 2 : (y2 < y ? 3 : (y2 > y ? 4 : 0)));
-                    if (k) {
-                        if constexpr (MODE != kPlanOrders) p.actions[((size_t)t * d.B + e) * d.N + a] = (uint8_t)k;
-                        uint32_t *r = sb + (k & 1 ? k + 1 : k - 1) * tbl + (size_t)t * WPT + cell(x, y);
-                        __stcg(r, __ldcg(r) | bit(y));
-                    }
-                }
-            }
+            plan_commit<RW, RPL, MODE != kPlanOrders>(occ, sb, tbl, H, lane, g, tstar, path, p, e, a);
             if (MODE != kPlanOrders && lane == 0) arr[a] = tstar;
             soc += tstar;
             __syncwarp();
@@ -312,6 +364,215 @@ template <int RW, int RPL, int MODE>
 __global__ void __launch_bounds__(kPlanWarps * 32) plan_orders_kernel(const PlanArgs p, const OrderArgs o)
 {
     plan_body<RW, RPL, MODE>(p, o);
+}
+
+// the action id of the move from cell c to cell c2 (x << 8 | y each), 0 for a wait
+__device__ inline int plan_move(int c, int c2)
+{
+    const int x = c >> 8, y = c & 255, x2 = c2 >> 8, y2 = c2 & 255;
+    return x2 < x ? 1 : (x2 > x ? 2 : (y2 < y ? 3 : (y2 > y ? 4 : 0)));
+}
+
+// Takes the path pth[0 .. H] (x << 8 | y, parked on the goal from its arrival) out of the tables (SET = false) or puts it back
+// (SET = true): p_t in Occ(t), and p_t in SB_opposite(k)(t) for a move by action k.  In a valid plan every bit of the tables
+// belongs to exactly one agent, so clearing a path's bits removes that agent and nobody else.
+template <int RW, int RPL, bool SET>
+__device__ __forceinline__ void plan_mark(uint32_t *const occ, const size_t tbl, const int H, const int lane, const uint16_t *const pth)
+{
+    constexpr int WPT = 32 * RPL * RW;
+    for (int t = lane; t <= H; t += 32) {
+        const int c = pth[t], x = c >> 8, y = c & 255;
+        const uint32_t b = plan_bit(y);
+        uint32_t *o = occ + (size_t)t * WPT + plan_cell<RW, RPL>(x, y);
+        __stcg(o, SET ? (__ldcg(o) | b) : (__ldcg(o) & ~b));
+        const int k = t < H ? plan_move(c, pth[t + 1]) : 0;
+        if (k) {
+            uint32_t *r = occ + (k & 1 ? k + 1 : k - 1) * tbl + (size_t)t * WPT + plan_cell<RW, RPL>(x, y);
+            __stcg(r, SET ? (__ldcg(r) | b) : (__ldcg(r) & ~b));
+        }
+    }
+}
+
+// Plan improvement (mapf_env_plan_lns): one warp per environment, all I iterations on it.  The warp checks the input plan
+// while it reserves every path in its tables, then per iteration takes the neighbourhood S out of the tables, re-plans S's
+// agents one after the other with plan()'s search, read-back and commit, and keeps the new paths (already in the tables) if
+// every agent of S found one and their arrivals sum to less than before; otherwise it clears them and puts the old paths back.
+// The tables are kept across iterations; the current paths and the candidates live in the warp's scratch after its tables.
+template <int RW, int RPL>
+__global__ void __launch_bounds__(kPlanWarps * 32) plan_lns_kernel(const PlanArgs p, const LnsArgs z)
+{
+    __shared__ uint16_t s_path[kPlanWarps][MAPF_PLAN_MAX_HORIZON + 1];  // the agent being re-planned at t = 0 .. t*
+    __shared__ uint8_t s_agent[kPlanWarps][MAPF_MAX_AGENTS];             // S in planning order
+    __shared__ uint32_t s_key[kPlanWarps][MAPF_MAX_AGENTS];
+    __shared__ int16_t s_arr[kPlanWarps][MAPF_MAX_AGENTS];               // each agent's current arrival
+    __shared__ int16_t s_new[kPlanWarps][MAPF_MAX_AGENTS];               // the candidate arrival of S's j-th agent
+    constexpr int WPT = 32 * RPL * RW;
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const EnvDims &d = p.d;
+    const int H = p.H;
+    const size_t tbl = (size_t)(H + 1) * WPT;
+    uint32_t *const occ = p.scratch + kPlanCounterWords + (size_t)(blockIdx.x * kPlanWarps + wid) * p.warp_words;
+    uint32_t *const sb = occ;
+    uint32_t *const fh = occ + 5 * tbl;
+    uint16_t *const cur = reinterpret_cast<uint16_t *>(occ + kPlanTables * tbl);  // u16[N][H+1]: the current paths
+    uint16_t *const cand = cur + (size_t)d.N * (H + 1);                            // u16[N][H+1]: S's j-th candidate in row j
+    uint16_t *const path = s_path[wid];
+    uint8_t *const agent = s_agent[wid];
+    uint32_t *const key = s_key[wid];
+    int16_t *const arr_now = s_arr[wid], *const arr_new = s_new[wid];
+
+    for (;;) {
+        unsigned e = 0;
+        if (lane == 0) e = atomicAdd(p.scratch, 1u);
+        e = __shfl_sync(MAPF_FULL_MASK, e, 0);
+        if (e >= (unsigned)d.B) break;
+        const int n = p.sz_n ? (int)__ldcg(p.sz_n + e) : d.N;
+        const int l = p.sz_l ? (int)__ldcg(p.sz_l + e) : d.L;
+        const uchar2 *const pos = reinterpret_cast<const uchar2 *>(p.pos) + (size_t)e * d.N;
+        const uchar2 *const goal = reinterpret_cast<const uchar2 *>(p.goal) + (size_t)e * d.N;
+        const uint32_t *const ob = p.obst + (size_t)e * d.obst_stride;
+        int32_t *const arr = p.arrival + (size_t)e * d.N;
+
+        // a failed plan (every present arrival -1) stays as it is
+        bool failed = true;
+        for (int a = lane; a < n; a += 32) failed &= __ldcg(arr + a) == -1;
+        if (__all_sync(MAPF_FULL_MASK, failed)) {
+            if (lane == 0) z.accepted[e] = -1;
+            continue;
+        }
+
+        // clean tables, then every path reserved while it is checked: lane l walks agents l, l + 32, .. over t = 0 .. H
+        {
+            uint4 *zr = reinterpret_cast<uint4 *>(occ);
+            const size_t n4 = 5 * tbl / 4;
+            for (size_t i = lane; i < n4; i += 32) __stcg(zr + i, make_uint4(0u, 0u, 0u, 0u));
+        }
+        __syncwarp();
+        bool bad = false;
+        for (int a = lane; a < n && !bad; a += 32) {
+            const int ar = __ldcg(arr + a);
+            arr_now[a] = (int16_t)ar;
+            if (ar < 0 || ar > H) {
+                bad = true;
+                break;
+            }
+            const uchar2 s = __ldcg(pos + a), g = __ldcg(goal + a);
+            uint16_t *const pa = cur + (size_t)a * (H + 1);
+            int x = s.x, y = s.y;
+            for (int t = 0;; ++t) {
+                // off the l x l map or on an obstacle; a vertex conflict (the bit is somebody else's); not on the goal at arrival
+                if (x < 0 || x >= l || y < 0 || y >= l || (__ldcg(ob + (x + 4) * d.RWS + ((y + 4) >> 5)) & plan_bit(y)) ||
+                    (atomicOr(occ + (size_t)t * WPT + plan_cell<RW, RPL>(x, y), plan_bit(y)) & plan_bit(y)) ||
+                    (t == ar && (x != g.x || y != g.y))) {
+                    bad = true;
+                    break;
+                }
+                pa[t] = (uint16_t)(x << 8 | y);
+                if (t == H) break;
+                const int k = p.actions[((size_t)t * d.B + e) * d.N + a];
+                if (k > 4 || (k && t >= ar)) {  // an unknown action, a move after arrival
+                    bad = true;
+                    break;
+                }
+                if (k) {
+                    atomicOr(sb + (k & 1 ? k + 1 : k - 1) * tbl + (size_t)t * WPT + plan_cell<RW, RPL>(x, y), plan_bit(y));
+                    x += act_dx(k), y += act_dy(k);
+                }
+            }
+        }
+        bad = __any_sync(MAPF_FULL_MASK, bad);
+        __syncwarp();
+        if (!bad) {
+            // a swap: agent a's move u -> v by action k meets another agent's move v -> u, which put v into SB_k(t)
+            for (int a = lane; a < n; a += 32) {
+                const uint16_t *const pa = cur + (size_t)a * (H + 1);
+                for (int t = 0; t < arr_now[a]; ++t) {
+                    const int k = plan_move(pa[t], pa[t + 1]), x = pa[t + 1] >> 8, y = pa[t + 1] & 255;
+                    if (k && (__ldcg(sb + k * tbl + (size_t)t * WPT + plan_cell<RW, RPL>(x, y)) & plan_bit(y))) bad = true;
+                }
+            }
+            bad = __any_sync(MAPF_FULL_MASK, bad);
+        }
+        if (bad) {
+            if (lane == 0) z.accepted[e] = -2;
+            continue;
+        }
+
+        EnvDims df = d;  // the free cells: l_e x l_e on a sized handle
+        df.L = l;
+        BfsFree<RW, RPL> F;
+        bfs_load_free<RW, RPL, 1>(df, ob, F);
+        const int m = min(z.K, n);
+        const uint64_t ge = z.env_offset + e;  // the environment's global index
+        int acc = 0;
+        for (uint32_t i = z.first; i < z.first + (uint32_t)z.I; ++i) {
+            // S: the m agents of smallest (k_a, a), in that order
+            for (int a = lane; a < n; a += 32)
+                key[a] = philox4x32_10(make_uint4((uint32_t)ge, (uint32_t)(ge >> 32), PURPOSE_LNS | (i << 8), (uint32_t)a), z.key).x;
+            __syncwarp();
+            for (int a = lane; a < n; a += 32) {
+                const uint32_t ka = key[a];
+                int r = 0;
+                for (int b = 0; b < n; ++b) r += key[b] < ka || (key[b] == ka && b < a);
+                if (r < m) agent[r] = (uint8_t)a;
+            }
+            __syncwarp();
+            int old = 0;
+            for (int j = 0; j < m; ++j) {
+                const int a = agent[j];
+                plan_mark<RW, RPL, false>(occ, tbl, H, lane, cur + (size_t)a * (H + 1));
+                old += arr_now[a];
+                __syncwarp();
+            }
+            int j = 0, soc = 0;
+            for (; j < m; ++j) {
+                const int a = agent[j];
+                const uchar2 s = __ldcg(pos + a), g = __ldcg(goal + a);
+                const int tstar = plan_search<RW, RPL>(occ, sb, fh, tbl, H, lane, F, s, g);
+                __syncwarp();
+                if (tstar < 0) break;
+                plan_read_back<RW, RPL>(sb, fh, tbl, d.L, lane, g, tstar, path);
+                __syncwarp();
+                plan_commit<RW, RPL, false>(occ, sb, tbl, H, lane, g, tstar, path, p, e, a);
+                uint16_t *const pc = cand + (size_t)j * (H + 1);
+                for (int t = lane; t <= H; t += 32) pc[t] = t <= tstar ? path[t] : (uint16_t)(g.x << 8 | g.y);
+                if (lane == 0) arr_new[j] = (int16_t)tstar;
+                soc += tstar;
+                __syncwarp();
+            }
+            if (j == m && soc < old) {  // accepted: the candidates are in the tables already
+                for (int q = 0; q < m; ++q) {
+                    const int a = agent[q];
+                    const uint16_t *const pc = cand + (size_t)q * (H + 1);
+                    uint16_t *const pa = cur + (size_t)a * (H + 1);
+                    for (int t = lane; t <= H; t += 32) pa[t] = pc[t];
+                    if (lane == 0) arr_now[a] = arr_new[q];
+                }
+                ++acc;
+            } else {  // rejected: the candidates planned so far out of the tables, the old paths back in
+                for (int q = 0; q < j; ++q) {
+                    plan_mark<RW, RPL, false>(occ, tbl, H, lane, cand + (size_t)q * (H + 1));
+                    __syncwarp();
+                }
+                for (int q = 0; q < m; ++q) {
+                    plan_mark<RW, RPL, true>(occ, tbl, H, lane, cur + (size_t)agent[q] * (H + 1));
+                    __syncwarp();
+                }
+            }
+            __syncwarp();
+        }
+
+        if (acc > 0) {  // the final paths: arrivals, and the actions that follow them (0 from the arrival on)
+            for (int a = lane; a < n; a += 32) arr[a] = arr_now[a];
+            for (int t = 0; t < H; ++t)
+                for (int a = lane; a < n; a += 32) {
+                    const uint16_t *const pa = cur + (size_t)a * (H + 1);
+                    p.actions[((size_t)t * d.B + e) * d.N + a] = (uint8_t)plan_move(pa[t], pa[t + 1]);
+                }
+        }
+        if (lane == 0) z.accepted[e] = acc;
+        __syncwarp();
+    }
 }
 
 // The handle's planner scratch: at least `bytes`, allocated on first use and grown when a call needs more
@@ -411,6 +672,30 @@ int launch_plan_orders(mapf_env *env, int H, int R, uint64_t seed, uint64_t env_
     return MAPF_OK;
 }
 
+template <int RW, int RPL>
+int launch_plan_lns(mapf_env *env, int H, int I, int K, uint64_t seed, uint64_t env_offset, uint32_t first, uint8_t *d_actions,
+                    int32_t *d_arrival, int32_t *d_accepted, cudaStream_t st)
+{
+    const EnvDims &d = env->d;
+    // the six tables, then the current and the candidate paths (u16[N][H+1] each), rounded to 16 bytes
+    const size_t warp_words = ((size_t)kPlanTables * (H + 1) * 32 * RPL * RW + (size_t)d.N * (H + 1) + 3) & ~(size_t)3;
+    const int64_t block_bytes = (int64_t)kPlanWarps * warp_words * 4;
+    int64_t blocks = 0;
+    int rc = plan_blocks(env, plan_lns_kernel<RW, RPL>, d.B, block_bytes, blocks);
+    if (rc != MAPF_OK) return rc;
+    rc = reserve_plan_scratch(env, (int64_t)kPlanCounterWords * 4 + blocks * block_bytes, st, "mapf_env_plan_lns: scratch");
+    if (rc != MAPF_OK) return rc;
+    LnsArgs z;
+    z.I = I, z.K = K, z.first = first;
+    z.key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
+    z.env_offset = env_offset;
+    z.accepted = d_accepted;
+    MAPF_CUDA(cudaMemsetAsync(env->pp_scratch, 0, 4, st));
+    plan_lns_kernel<RW, RPL><<<(unsigned)blocks, kPlanWarps * 32, 0, st>>>(plan_args(env, H, warp_words, d_actions, d_arrival), z);
+    MAPF_CUDA(cudaGetLastError());
+    return MAPF_OK;
+}
+
 }  // namespace
 
 // rows per lane RPL = ceil(L / 32) next to the handle's RW: L <= 24 (1, 1), <= 56 (2, 1..2), <= 88 (3, 2..3), <= 120 (4, 3..4)
@@ -447,5 +732,27 @@ int mapf_launch_plan_orders(mapf_env *env, int H, int R, uint64_t seed, uint64_t
     }
 #undef MAPF_PLAN_ORDERS_CASE
     mapf_set_error("mapf_env_plan_prioritized_orders: unsupported map size");
+    return MAPF_EINVAL;
+}
+
+int mapf_launch_plan_lns(mapf_env *env, int H, int iterations, int neighborhood, uint64_t seed, uint64_t env_offset, uint32_t first_iteration,
+                         uint8_t *d_actions, int32_t *d_arrival, int32_t *d_accepted, cudaStream_t st)
+{
+    const int rpl = (env->d.L + 31) / 32;
+#define MAPF_PLAN_LNS_CASE(rw, r)                                                                                             \
+    case rw * 8 + r:                                                                                                          \
+        return launch_plan_lns<rw, r>(env, H, iterations, neighborhood, seed, env_offset, first_iteration, d_actions, d_arrival, \
+                                      d_accepted, st)
+    switch (env->d.RW * 8 + rpl) {
+        MAPF_PLAN_LNS_CASE(1, 1);
+        MAPF_PLAN_LNS_CASE(2, 1);
+        MAPF_PLAN_LNS_CASE(2, 2);
+        MAPF_PLAN_LNS_CASE(3, 2);
+        MAPF_PLAN_LNS_CASE(3, 3);
+        MAPF_PLAN_LNS_CASE(4, 3);
+        MAPF_PLAN_LNS_CASE(4, 4);
+    }
+#undef MAPF_PLAN_LNS_CASE
+    mapf_set_error("mapf_env_plan_lns: unsupported map size");
     return MAPF_EINVAL;
 }
