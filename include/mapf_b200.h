@@ -556,6 +556,46 @@ int mapf_env_plan_prioritized_orders(mapf_env *env, int32_t horizon, int32_t ord
 int mapf_env_plan_lns(mapf_env *env, int32_t horizon, int32_t iterations, int32_t neighborhood, uint64_t seed, uint64_t env_offset,
                       uint32_t first_iteration, uint8_t *d_actions, int32_t *d_arrival, int32_t *d_accepted, void *stream);
 
+/* Plan repair by collision-based large-neighbourhood search (MAPF-LNS2, Li et al., AAAI 2022): environments whose plan failed
+ * are planned again with vertex collisions allowed but counted, and small groups of agents are re-planned until no collision
+ * is left.  In place, in the layout mapf_env_plan_prioritized writes:
+ *   d_actions     u8[horizon, B, N]  written for every repaired environment
+ *   d_arrival     i32[B, N]          read; written for every repaired environment
+ *   d_collisions  i32[B]             0: repaired, collision-free; G > 0: the vertex collisions left when the iterations ran
+ *                                    out; -1: some agent has no path even with collisions; -2: not a failed plan
+ * Environment e has global index g = env_offset + e, n agents (n_e on a sized handle) on the l x l map.  Only an environment
+ * whose arrival row is -1 for every present agent is repaired; any other is passed through (its arrival row read, nothing
+ * written, collisions -2), whether its plan is valid or not.
+ * Obstacles, the map bound and swaps (mapf_env_plan_prioritized's SB tables) are hard constraints, a vertex conflict costs 1.
+ * The soft search of one agent against the reserved paths keeps layers c = 0 .. MAPF_PLAN_REPAIR_MAX_COLLISIONS: F_c(t) is
+ * the set of cells reached at t with exactly c vertex collisions and no fewer, F_0(0) = {start},
+ *   R_c(t) = (F_c(t) | OR_k (shift_k F_c(t) & ~SB_k(t))) & Free,
+ *   F_c(t+1) = ((R_c(t) & ~Occ(t+1)) | (R_c-1(t) & Occ(t+1))) minus F_0(t+1) .. F_c-1(t+1).
+ * With park(t) = #{t' in (t, H] : goal in Occ(t')} and c(t) the layer holding the goal, the agent's cost is the minimum over
+ * t <= H of c(t) + park(t), its arrival t* the earliest t of that minimum (no layer holding the goal: no path).  The path is
+ * read back from (goal, t*, c(t*)): at (v, t, c), c' = c - [v in Occ(t)] and the first action id k whose predecessor v - delta_k
+ * is in F_c'(t-1) and, for a move, v is not in SB_k(t-1); it is reserved as mapf_env_plan_prioritized reserves a path.  With
+ * cost 0 this is mapf_env_plan_prioritized's search: where that call solves an environment, the initial plan is its plan.
+ * Initial plan: every agent in index order by the soft search, each against the agents before it.  The plan's collision
+ * count G is the vertex excess, the sum over t in [0, H] and cells of max(0, occupants - 1).
+ * Iterations i = 0 .. iterations - 1, while G > 0: K is the set of agents with a vertex collision, k_a = word 0 of
+ * Philox4x32-10 with counter (g_lo, g_hi, 6 | i << 8, a) and key (seed_lo, seed_hi), and S the first m = min(neighborhood, n)
+ * agents by ([a not in K], k_a, a).  With X the agents outside S, f_old = G - G(X); the agents of S are re-planned in that
+ * order against X and the new paths of S before them, and f_new is the sum of their costs.  The iteration is accepted if
+ * every agent of S finds a path and (f_new, sum of S's new arrivals) < (f_old, sum of the old ones) lexicographically: the new
+ * paths replace the old ones and G becomes G - f_old + f_new (which is the new plan's excess); otherwise nothing changes.
+ * Output: a repaired environment is written as mapf_env_plan_prioritized writes a solved one (actions 0 from each arrival
+ * on, arrival 0 and actions 0 for absent agents); collisions -1 and G > 0 write its failure form (arrival row -1, actions 0).
+ * The result depends only on the state, horizon, iterations, neighborhood, seed and env_offset.
+ * MAPF_EINVAL for a horizon outside 1 .. MAPF_PLAN_MAX_HORIZON, iterations outside 0 .. 2^24, a neighborhood outside 1 .. N or
+ * a NULL buffer, MAPF_ENOMEM if the planner's scratch (per resident warp: 10 tables of (horizon + 1) x 32 x ceil(L / 32) x RW
+ * words, where mapf_env_plan_prioritized keeps 6, plus the current and candidate paths, 4 bytes per agent and time step,
+ * rounded up to 16 bytes) cannot be allocated.  Reads the handle's state and writes nothing in it; asynchronous on `stream`. */
+#define MAPF_PLAN_REPAIR_MAX_COLLISIONS 15
+#define MAPF_PLAN_REPAIR_MAX_ITERATIONS (1 << 24)
+int mapf_env_plan_repair(mapf_env *env, int32_t horizon, int32_t iterations, int32_t neighborhood, uint64_t seed, uint64_t env_offset,
+                         uint8_t *d_actions, int32_t *d_arrival, int32_t *d_collisions, void *stream);
+
 /* ---- CBS expert / solvable-instance generator (search.py:58-442, test.py:23-79; SURVEY 8(f)4) -- HOST code ------------------
  * Conflict-based search over space-time A*: a collision-free set of paths of minimal sum of costs (search.py:17-21), as the
  * action script search.find_path returns (search.py:396-442).  All pointers are HOST memory; no kernel is launched.

@@ -362,6 +362,37 @@ class BatchedEnvironment:
         soc = torch.where(failed, -1, arrival.sum(1)).to(torch.int32)
         return actions, arrival, makespan, soc, accepted
 
+    def plan_repair(self, actions, arrival, iterations: int = 16, neighborhood: int = 8, seed: int = 0, env_offset: int = 0):
+        """Repairs the failed environments of a plan on the device by collision-based large-neighbourhood search
+        (mapf_env_plan_repair, MAPF-LNS2): an environment whose arrival row is -1 is planned again in index order with vertex
+        collisions allowed but minimised, then up to `iterations` times a group of `neighborhood` agents (those with a
+        collision first, in Philox order) is re-planned against the others and kept if the collision count drops, until no
+        collision is left.  `actions` uint8[H,B,N] and `arrival` int32[B,N] are CUDA tensors laid out as `plan` /
+        `plan_orders` / `plan_lns` return them; they are copied, not changed.  Returns (actions, arrival, makespan, soc,
+        collisions) CUDA tensors on the current stream: the plan as `plan` returns one, and collisions int32[B]: 0 where the
+        environment was repaired (a collision-free plan, valid input for `plan_lns`), G > 0 where G collisions were left
+        (written as a failed plan), -1 where some agent has no path within H even with collisions, and -2 where the input was
+        not a failed plan (returned as it came).  Where `plan` solves an environment, repairing its row of -1 gives `plan`'s
+        plan.  The handle's state is not changed.  Defaults (DESIGN §8 (f)7, measured on a B200): 16 iterations of 8
+        agents; after plan() on 8192 x 32 @ 40 they repair 1125 of 1141 failed environments in 82 ms, the solved fraction of
+        plan_orders(32) in under a quarter of its time.  Environments left unrepaired run every iteration and set the call's
+        time, so more iterations cost time almost linearly and repaired few more there."""
+        torch = _torch()
+        B, N = self.num_envs, self.num_agents
+        assert actions.is_cuda and actions.dtype == torch.uint8 and actions.is_contiguous() and actions.dim() == 3
+        assert tuple(actions.shape[1:]) == (B, N), "actions must be uint8 [H, B, N]"
+        assert arrival.is_cuda and arrival.dtype == torch.int32 and tuple(arrival.shape) == (B, N), "arrival must be int32 [B, N]"
+        H = int(actions.shape[0])
+        actions, arrival = actions.clone(), arrival.contiguous().clone()
+        collisions = torch.empty(B, dtype=torch.int32, device=self.device)
+        _native.check(self._lib.mapf_env_plan_repair(
+            self._h, H, int(iterations), int(neighborhood), int(seed), int(env_offset), C.c_void_p(actions.data_ptr()),
+            C.c_void_p(arrival.data_ptr()), C.c_void_p(collisions.data_ptr()), self._stream()))
+        failed = (arrival < 0).any(1)
+        makespan = torch.where(failed, -1, arrival.max(1).values).to(torch.int32)
+        soc = torch.where(failed, -1, arrival.sum(1)).to(torch.int32)
+        return actions, arrival, makespan, soc, collisions
+
     def set_autoreset(self, max_steps: int = config.max_steps, seed: int = 0, env_offset: int = 0, stride: Optional[int] = None,
                       density: Optional[float] = None):
         """Episode handling inside `rollout` (worker.py:390,422-428): a step that finds its environment finished (done, or

@@ -595,6 +595,21 @@ int mapf_env_plan_lns(mapf_env *env, int32_t horizon, int32_t iterations, int32_
                                 st);
 }
 
+int mapf_env_plan_repair(mapf_env *env, int32_t horizon, int32_t iterations, int32_t neighborhood, uint64_t seed, uint64_t env_offset,
+                         uint8_t *d_actions, int32_t *d_arrival, int32_t *d_collisions, void *stream)
+{
+    REQUIRE_ENV(env);
+    if (horizon < 1 || horizon > MAPF_PLAN_MAX_HORIZON || iterations < 0 || iterations > MAPF_PLAN_REPAIR_MAX_ITERATIONS || neighborhood < 1 ||
+        neighborhood > env->d.N || !d_actions || !d_arrival || !d_collisions) {
+        mapf_set_error("mapf_env_plan_repair: 1 <= horizon <= 1024, 0 <= iterations <= 2^24, 1 <= neighborhood <= N and non-NULL "
+                       "d_actions, d_arrival, d_collisions required");
+        return MAPF_EINVAL;
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    MAPF_DRAIN(env, st);
+    return mapf_launch_plan_repair(env, horizon, iterations, neighborhood, seed, env_offset, d_actions, d_arrival, d_collisions, st);
+}
+
 int mapf_env_step_observe_ex(mapf_env *env, const uint8_t *d_actions, uint8_t *d_obs, const int64_t *d_obs_rows, float *d_rewards,
                              uint8_t *d_codes, uint8_t *d_done, int32_t *d_steps, void *stream)
 {

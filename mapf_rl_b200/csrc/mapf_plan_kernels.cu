@@ -34,7 +34,17 @@
 // above, and the new paths are kept (accepted += 1) if every agent of S finds one and their arrivals sum to strictly less
 // than before.  One warp runs all iterations of one environment with its tables kept across them; the path search,
 // read-back and commit are the functions plan_body uses.
+//
+// Plan repair (mapf_env_plan_repair, DESIGN.md §8 (f)7), collision-based large-neighbourhood search (MAPF-LNS2) on the
+// environments whose plan failed: vertex conflicts become soft, each costing 1, while obstacles and swaps stay hard.  The
+// soft search keeps one frontier per collision count c = 0 .. C, F_c(t) the cells reached at t with exactly c vertex
+// collisions and no fewer; a cell is in at most one layer, so the history stores a "reached" plane and the layer's four bits
+// (5 tables instead of C + 1).  The agents are planned in index order with collisions allowed, then each iteration re-plans a
+// group S (the agents with a collision first, in Philox order) against the others and keeps the new paths if their collision
+// count (then their sum of costs) drops.  The tables are rebuilt from the current paths every iteration: in a colliding plan
+// a bit can belong to two agents, so clearing one agent's bits is not undone by reserving it again.
 #include <algorithm>
+#include <climits>
 
 #include "mapf_bfs_device.cuh"
 #include "mapf_common.cuh"
@@ -74,6 +84,16 @@ struct OrderArgs {
     int32_t *order;              // i32[B]: the winning r, -1
     uint8_t *rank;               // u8[B, N]: agent a's position in the winning order, 255
 };
+
+struct RepairArgs {
+    int I, K;                    // iterations, neighbourhood size
+    uint2 key;                   // Philox key (seed)
+    uint64_t env_offset;         // global index of environment 0
+    int32_t *collisions;         // i32[B]: collisions left, -1 (no path), -2 (not a failed plan)
+};
+
+constexpr int kRepairTables = 10;  // Occ, SB_1 .. SB_4, the layer history: reached, the layer's bits 0 .. 3
+static_assert(MAPF_PLAN_REPAIR_MAX_COLLISIONS >= 1 && MAPF_PLAN_REPAIR_MAX_COLLISIONS <= 15, "layers are stored in four bits");
 
 struct LnsArgs {
     int I, K;                    // iterations, neighbourhood size
@@ -575,6 +595,352 @@ __global__ void __launch_bounds__(kPlanWarps * 32) plan_lns_kernel(const PlanArg
     }
 }
 
+// The soft search of one agent from s to g against the reservations in the tables (mapf_env_plan_repair): the layers
+// F_c(0 .. t*) go into the history as a reached plane at lh and the layer's bit j at lh + (1 + j) * tbl.  Returns t*, the
+// earliest t of least c(t) + park(t), and its cost and c(t*) in cost / cstar, or -1 where the goal is in no layer up to H.
+// Layers below the lowest and above the highest non-empty one are skipped.  The search stops once t >= last_busy(g) and the
+// best cost is at most the lowest non-empty layer: that layer never decreases with t and park(t) = 0 from last_busy(g) on,
+// so no later t is cheaper.  The current slice's planes are read back from the history, so that no instantiation spills.
+template <int RW, int RPL>
+__device__ __forceinline__ int repair_search(const uint32_t *const occ, uint32_t *const lh, const size_t tbl, const int H, const int lane,
+                                             const BfsFree<RW, RPL> &F, const uchar2 s, const uchar2 g, int &cost, int &cstar)
+{
+    constexpr int WPT = 32 * RPL * RW;
+    constexpr int C = MAPF_PLAN_REPAIR_MAX_COLLISIONS;
+    const uint32_t *const sb = occ;
+    const size_t gi = plan_cell<RW, RPL>(g.x, g.y);
+    const uint32_t gb = plan_bit(g.y);
+    const int gl = g.x / RPL, gq = g.x % RPL, gw = (g.y + 4) >> 5;
+    // last_busy(goal), and the count of t with the goal in Occ(t): park(t) = nb - seen(t), seen(t) = #{t' <= t : busy}
+    int lb = -1;
+    unsigned nb = 0;
+#pragma unroll 4
+    for (int t = lane; t <= H; t += 32)
+        if (__ldcg(occ + (size_t)t * WPT + gi) & gb) lb = t, ++nb;
+    lb = __reduce_max_sync(MAPF_FULL_MASK, lb);
+    nb = __reduce_add_sync(MAPF_FULL_MASK, nb);
+    int seen = (__ldcg(occ + gi) & gb) ? 1 : 0;
+
+#pragma unroll
+    for (int q = 0; q < RPL; ++q)
+#pragma unroll
+        for (int w = 0; w < RW; ++w) {
+            const size_t o = (q * RW + w) * 32 + lane;
+            __stcg(lh + o, (lane * RPL + q == s.x && ((s.y + 4) >> 5) == w) ? plan_bit(s.y) : 0u);
+#pragma unroll
+            for (int j = 1; j <= 4; ++j) __stcg(lh + j * tbl + o, 0u);
+        }
+    int best = INT_MAX, tstar = -1, cb = 0;
+    if (s.x == g.x && s.y == g.y) best = (int)nb - seen, tstar = 0;
+    int low = 0, top = 0;  // the lowest and the highest non-empty layer at t
+    for (int t = 0; t < H && !(t >= lb && best <= low); ++t) {
+        const size_t ot = (size_t)t * WPT;
+        uint32_t on[RPL][RW], nr[RPL][RW], nbit[4][RPL][RW], rp[RPL][RW];  // Occ(t+1), reached at t+1, its bits, R_c-1(t)
+#pragma unroll
+        for (int q = 0; q < RPL; ++q)
+#pragma unroll
+            for (int w = 0; w < RW; ++w) {
+                on[q][w] = __ldcg(occ + ot + WPT + (q * RW + w) * 32 + lane);
+                nr[q][w] = rp[q][w] = 0u;
+#pragma unroll
+                for (int j = 0; j < 4; ++j) nbit[j][q][w] = 0u;
+            }
+        int nlow = -1, ntop = -1;
+        const int chi = min(top + 1, C);
+#pragma unroll 1
+        for (int c = low; c <= chi; ++c) {
+            uint32_t fc[RPL][RW];  // F_c(t)
+#pragma unroll
+            for (int q = 0; q < RPL; ++q)
+#pragma unroll
+                for (int w = 0; w < RW; ++w) {
+                    const size_t o = ot + (q * RW + w) * 32 + lane;
+                    uint32_t x = 0u;
+                    if (c <= top) {
+                        x = __ldcg(lh + o);
+#pragma unroll
+                        for (int j = 0; j < 4; ++j) {
+                            const uint32_t b = __ldcg(lh + (1 + j) * tbl + o);
+                            x &= (c >> j & 1) ? b : ~b;
+                        }
+                    }
+                    fc[q][w] = x;
+                }
+            uint32_t any = 0;
+#pragma unroll
+            for (int w = 0; w < RW; ++w) {
+                uint32_t above, below;
+                bfs_rows_around<RW, RPL, 32, false>(fc, w, lane, above, below);
+#pragma unroll
+                for (int q = 0; q < RPL; ++q) {
+                    const size_t o = ot + (q * RW + w) * 32 + lane;
+                    const uint32_t x = fc[q][w];
+                    const uint32_t from_dn = q < RPL - 1 ? fc[q < RPL - 1 ? q + 1 : q][w] : below;  // action 1 (x-1)
+                    const uint32_t from_up = q > 0 ? fc[q > 0 ? q - 1 : 0][w] : above;              // action 2 (x+1)
+                    const uint32_t from_rt = w < RW - 1 ? __funnelshift_r(x, fc[q][w < RW - 1 ? w + 1 : w], 1) : x >> 1;  // 3
+                    const uint32_t from_lt = w > 0 ? __funnelshift_l(fc[q][w > 0 ? w - 1 : 0], x, 1) : x << 1;            // 4
+                    const uint32_t r = (x | (from_dn & ~__ldcg(sb + tbl + o)) | (from_up & ~__ldcg(sb + 2 * tbl + o)) |
+                                        (from_rt & ~__ldcg(sb + 3 * tbl + o)) | (from_lt & ~__ldcg(sb + 4 * tbl + o))) & F.v[q][w];
+                    const uint32_t nf = ((r & ~on[q][w]) | (rp[q][w] & on[q][w])) & ~nr[q][w];  // F_c(t+1)
+                    rp[q][w] = r;
+                    nr[q][w] |= nf;
+#pragma unroll
+                    for (int j = 0; j < 4; ++j)
+                        if (c >> j & 1) nbit[j][q][w] |= nf;
+                    any |= nf;
+                }
+            }
+            if (__any_sync(MAPF_FULL_MASK, any != 0)) {
+                ntop = c;
+                if (nlow < 0) nlow = c;
+            }
+        }
+        uint32_t xr = 0, xo = 0;
+        int xc = 0;
+#pragma unroll
+        for (int q = 0; q < RPL; ++q)
+#pragma unroll
+            for (int w = 0; w < RW; ++w) {
+                const size_t o = ot + WPT + (q * RW + w) * 32 + lane;
+                __stcg(lh + o, nr[q][w]);
+#pragma unroll
+                for (int j = 0; j < 4; ++j) __stcg(lh + (1 + j) * tbl + o, nbit[j][q][w]);
+                if (q == gq && w == gw) {
+                    xr = nr[q][w], xo = on[q][w];
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) xc |= (nbit[j][q][w] & gb) ? 1 << j : 0;
+                }
+            }
+        low = nlow, top = ntop;
+        if (top < 0) break;  // nothing reachable at t + 1
+        seen += __any_sync(MAPF_FULL_MASK, lane == gl && (xo & gb)) ? 1 : 0;
+        const int cg = __shfl_sync(MAPF_FULL_MASK, (xr & gb) ? xc : -1, gl);  // c(t+1)
+        if (cg >= 0 && cg + (int)nb - seen < best) best = cg + (int)nb - seen, tstar = t + 1, cb = cg;
+    }
+    cost = best, cstar = cb;
+    return tstar;
+}
+
+// The path back from (g, t*, c(t*)) into path[0 .. t*] (x << 8 | y): at (v, t, c) the layer c' = c - [v in Occ(t)], and lane
+// k < 5 tests action k, whose predecessor must be in F_c'(t-1); the lowest admissible id wins
+template <int RW, int RPL>
+__device__ __forceinline__ void repair_read_back(const uint32_t *const occ, const uint32_t *const lh, const size_t tbl, const int L,
+                                                 const int lane, const uchar2 g, const int tstar, int c, uint16_t *const path)
+{
+    constexpr int WPT = 32 * RPL * RW;
+    const uint32_t *const sb = occ;
+    int vx = g.x, vy = g.y;
+    if (lane == 0) path[tstar] = (uint16_t)(vx << 8 | vy);
+    for (int t = tstar; t >= 1; --t) {
+        c -= (__ldcg(occ + (size_t)t * WPT + plan_cell<RW, RPL>(vx, vy)) & plan_bit(vy)) != 0;
+        bool ok = false;
+        if (lane < 5) {
+            const int ux = vx - act_dx(lane), uy = vy - act_dy(lane);
+            if (ux >= 0 && ux < L && uy >= 0 && uy < L) {
+                const size_t o = (size_t)(t - 1) * WPT + plan_cell<RW, RPL>(ux, uy);
+                const uint32_t b = plan_bit(uy);
+                ok = (__ldcg(lh + o) & b) != 0;
+                for (int j = 0; j < 4; ++j) ok &= ((__ldcg(lh + (1 + j) * tbl + o) & b) != 0) == ((c >> j & 1) != 0);
+                if (ok && lane > 0) ok = (__ldcg(sb + lane * tbl + (size_t)(t - 1) * WPT + plan_cell<RW, RPL>(vx, vy)) & plan_bit(vy)) == 0;
+            }
+        }
+        const unsigned m = __ballot_sync(MAPF_FULL_MASK, ok);
+        const int k = m ? __ffs(m) - 1 : 0;
+        vx -= act_dx(k), vy -= act_dy(k);
+        if (lane == 0) path[t - 1] = (uint16_t)(vx << 8 | vy);
+    }
+}
+
+// Clean tables (Occ, SB_1 .. SB_4, and with DUP the plane at occ + 5 * tbl), then the current paths cur[a][0 .. H] of the
+// agents with skip[a] == 0 reserved; lane l owns the time slices l, l + 32, ..  Returns on every lane the reservations that
+// found their Occ bit set already, the vertex excess of those agents whatever their order.  With DUP such a cell is set in
+// the plane at occ + 5 * tbl.
+template <int RW, int RPL, bool DUP>
+__device__ __forceinline__ int repair_reserve(uint32_t *const occ, const size_t tbl, const int H, const int lane, const int n,
+                                              const uint16_t *const cur, const uint8_t *const skip)
+{
+    constexpr int WPT = 32 * RPL * RW;
+    {
+        uint4 *zr = reinterpret_cast<uint4 *>(occ);
+        const size_t n4 = (DUP ? 6 : 5) * tbl / 4;
+        for (size_t i = lane; i < n4; i += 32) __stcg(zr + i, make_uint4(0u, 0u, 0u, 0u));
+    }
+    __syncwarp();
+    unsigned hits = 0;
+    for (int t = lane; t <= H; t += 32)
+        for (int a = 0; a < n; ++a) {
+            if (skip[a]) continue;
+            const uint16_t *const pa = cur + (size_t)a * (H + 1);
+            const int c = pa[t], x = c >> 8, y = c & 255;
+            const size_t o = (size_t)t * WPT + plan_cell<RW, RPL>(x, y);
+            const uint32_t b = plan_bit(y), old = __ldcg(occ + o);
+            if (old & b) {
+                ++hits;
+                if constexpr (DUP) __stcg(occ + 5 * tbl + o, __ldcg(occ + 5 * tbl + o) | b);
+            } else {
+                __stcg(occ + o, old | b);
+            }
+            const int k = t < H ? plan_move(c, pa[t + 1]) : 0;
+            if (k) {
+                uint32_t *r = occ + (k & 1 ? k + 1 : k - 1) * tbl + o;
+                __stcg(r, __ldcg(r) | b);
+            }
+        }
+    __syncwarp();
+    return (int)__reduce_add_sync(MAPF_FULL_MASK, hits);
+}
+
+// Plan repair (mapf_env_plan_repair): one warp per environment, the initial soft plan and all I iterations on it.  Per
+// iteration the tables are built twice from the current paths: once with every agent, which marks the cells of more than one
+// agent and so K, and once with the agents outside S, which gives G(X); S is then planned into them.
+template <int RW, int RPL>
+__global__ void __launch_bounds__(kPlanWarps * 32, RW * RPL <= 4 ? 3 : 1) plan_repair_kernel(const PlanArgs p, const RepairArgs z)
+{
+    __shared__ uint16_t s_path[kPlanWarps][MAPF_PLAN_MAX_HORIZON + 1];  // the agent being planned at t = 0 .. t*
+    __shared__ uint8_t s_agent[kPlanWarps][MAPF_MAX_AGENTS];             // S in planning order
+    __shared__ uint8_t s_ink[kPlanWarps][MAPF_MAX_AGENTS];               // a in K
+    __shared__ uint8_t s_ins[kPlanWarps][MAPF_MAX_AGENTS];               // a in S
+    __shared__ uint32_t s_key[kPlanWarps][MAPF_MAX_AGENTS];
+    __shared__ int16_t s_arr[kPlanWarps][MAPF_MAX_AGENTS];               // each agent's current arrival
+    __shared__ int16_t s_new[kPlanWarps][MAPF_MAX_AGENTS];               // the candidate arrival of S's j-th agent
+    constexpr int WPT = 32 * RPL * RW;
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const EnvDims &d = p.d;
+    const int H = p.H;
+    const size_t tbl = (size_t)(H + 1) * WPT;
+    uint32_t *const occ = p.scratch + kPlanCounterWords + (size_t)(blockIdx.x * kPlanWarps + wid) * p.warp_words;
+    uint32_t *const sb = occ;
+    uint32_t *const lh = occ + 5 * tbl;                                            // the layer history, 5 tables
+    uint16_t *const cur = reinterpret_cast<uint16_t *>(occ + kRepairTables * tbl);  // u16[N][H+1]: the current paths
+    uint16_t *const cand = cur + (size_t)d.N * (H + 1);                            // u16[N][H+1]: S's j-th candidate in row j
+    uint16_t *const path = s_path[wid];
+    uint8_t *const agent = s_agent[wid], *const in_k = s_ink[wid], *const in_s = s_ins[wid];
+    uint32_t *const key = s_key[wid];
+    int16_t *const arr_now = s_arr[wid], *const arr_new = s_new[wid];
+
+    for (;;) {
+        unsigned e = 0;
+        if (lane == 0) e = atomicAdd(p.scratch, 1u);
+        e = __shfl_sync(MAPF_FULL_MASK, e, 0);
+        if (e >= (unsigned)d.B) break;
+        const int n = p.sz_n ? (int)__ldcg(p.sz_n + e) : d.N;
+        const uchar2 *const pos = reinterpret_cast<const uchar2 *>(p.pos) + (size_t)e * d.N;
+        const uchar2 *const goal = reinterpret_cast<const uchar2 *>(p.goal) + (size_t)e * d.N;
+        int32_t *const arr = p.arrival + (size_t)e * d.N;
+
+        // only a failed plan (every present arrival -1) is repaired
+        bool failed = true;
+        for (int a = lane; a < n; a += 32) failed &= __ldcg(arr + a) == -1;
+        if (!__all_sync(MAPF_FULL_MASK, failed)) {
+            if (lane == 0) z.collisions[e] = -2;
+            continue;
+        }
+
+        {
+            uint4 *zr = reinterpret_cast<uint4 *>(occ);
+            const size_t n4 = 5 * tbl / 4;
+            for (size_t i = lane; i < n4; i += 32) __stcg(zr + i, make_uint4(0u, 0u, 0u, 0u));
+        }
+        EnvDims df = d;  // the free cells: l_e x l_e on a sized handle
+        if (p.sz_l) df.L = (int)__ldcg(p.sz_l + e);
+        BfsFree<RW, RPL> F;
+        bfs_load_free<RW, RPL, 1>(df, p.obst + (size_t)e * d.obst_stride, F);
+        __syncwarp();
+
+        // the initial plan: every agent in index order against the agents before it
+        int G = 0, res = 0;
+        for (int a = 0; a < n; ++a) {
+            const uchar2 s = __ldcg(pos + a), g = __ldcg(goal + a);
+            int cost, c;
+            const int tstar = repair_search<RW, RPL>(occ, lh, tbl, H, lane, F, s, g, cost, c);
+            __syncwarp();
+            if (tstar < 0) {
+                res = -1;
+                break;
+            }
+            repair_read_back<RW, RPL>(occ, lh, tbl, d.L, lane, g, tstar, c, path);
+            __syncwarp();
+            plan_commit<RW, RPL, false>(occ, sb, tbl, H, lane, g, tstar, path, p, e, a);
+            uint16_t *const pa = cur + (size_t)a * (H + 1);
+            for (int t = lane; t <= H; t += 32) pa[t] = t <= tstar ? path[t] : (uint16_t)(g.x << 8 | g.y);
+            if (lane == 0) arr_now[a] = (int16_t)tstar;
+            G += cost;
+            __syncwarp();
+        }
+
+        if (res == 0) {
+            const int m = min(z.K, n);
+            const uint64_t ge = z.env_offset + e;  // the environment's global index
+            for (uint32_t i = 0; i < (uint32_t)z.I && G > 0; ++i) {
+                // K: the agents on a cell of more than one agent at some t
+                for (int a = lane; a < n; a += 32) in_k[a] = 0, in_s[a] = 0;
+                __syncwarp();
+                repair_reserve<RW, RPL, true>(occ, tbl, H, lane, n, cur, in_s);
+                for (int t = lane; t <= H; t += 32)
+                    for (int a = 0; a < n; ++a) {
+                        const int c = cur[(size_t)a * (H + 1) + t], y = c & 255;
+                        if (__ldcg(lh + (size_t)t * WPT + plan_cell<RW, RPL>(c >> 8, y)) & plan_bit(y)) in_k[a] = 1;
+                    }
+                for (int a = lane; a < n; a += 32)
+                    key[a] = philox4x32_10(make_uint4((uint32_t)ge, (uint32_t)(ge >> 32), PURPOSE_REPAIR | (i << 8), (uint32_t)a), z.key).x;
+                __syncwarp();
+                // S: the first m agents by ([a not in K], k_a, a)
+                for (int a = lane; a < n; a += 32) {
+                    const uint64_t ka = (uint64_t)!in_k[a] << 32 | key[a];
+                    int r = 0;
+                    for (int b = 0; b < n; ++b) {
+                        const uint64_t kb = (uint64_t)!in_k[b] << 32 | key[b];
+                        r += kb < ka || (kb == ka && b < a);
+                    }
+                    if (r < m) agent[r] = (uint8_t)a, in_s[a] = 1;
+                }
+                __syncwarp();
+                const int f_old = G - repair_reserve<RW, RPL, false>(occ, tbl, H, lane, n, cur, in_s);
+                int old = 0;
+                for (int j = 0; j < m; ++j) old += arr_now[agent[j]];
+                int j = 0, f_new = 0, soc = 0;
+                for (; j < m; ++j) {
+                    const int a = agent[j];
+                    const uchar2 s = __ldcg(pos + a), g = __ldcg(goal + a);
+                    int cost, c;
+                    const int tstar = repair_search<RW, RPL>(occ, lh, tbl, H, lane, F, s, g, cost, c);
+                    __syncwarp();
+                    if (tstar < 0) break;
+                    repair_read_back<RW, RPL>(occ, lh, tbl, d.L, lane, g, tstar, c, path);
+                    __syncwarp();
+                    plan_commit<RW, RPL, false>(occ, sb, tbl, H, lane, g, tstar, path, p, e, a);
+                    uint16_t *const pc = cand + (size_t)j * (H + 1);
+                    for (int t = lane; t <= H; t += 32) pc[t] = t <= tstar ? path[t] : (uint16_t)(g.x << 8 | g.y);
+                    if (lane == 0) arr_new[j] = (int16_t)tstar;
+                    f_new += cost, soc += tstar;
+                    __syncwarp();
+                }
+                if (j == m && (f_new < f_old || (f_new == f_old && soc < old))) {  // accepted
+                    for (int q = 0; q < m; ++q) {
+                        const uint16_t *const pc = cand + (size_t)q * (H + 1);
+                        uint16_t *const pa = cur + (size_t)agent[q] * (H + 1);
+                        for (int t = lane; t <= H; t += 32) pa[t] = pc[t];
+                        if (lane == 0) arr_now[agent[q]] = arr_new[q];
+                    }
+                    G += f_new - f_old;
+                }
+                __syncwarp();
+            }
+            res = G;
+        }
+
+        // collision-free: the paths as plan() writes them; otherwise plan()'s failure form
+        for (int a = lane; a < d.N; a += 32) arr[a] = res ? -1 : (a < n ? arr_now[a] : 0);
+        for (int t = 0; t < H; ++t)
+            for (int a = lane; a < d.N; a += 32) {
+                const uint16_t *const pa = cur + (size_t)a * (H + 1);
+                p.actions[((size_t)t * d.B + e) * d.N + a] = res || a >= n ? 0 : (uint8_t)plan_move(pa[t], pa[t + 1]);
+            }
+        if (lane == 0) z.collisions[e] = res;
+        __syncwarp();
+    }
+}
+
 // The handle's planner scratch: at least `bytes`, allocated on first use and grown when a call needs more
 int reserve_plan_scratch(mapf_env *env, int64_t bytes, cudaStream_t st, const char *what)
 {
@@ -696,6 +1062,30 @@ int launch_plan_lns(mapf_env *env, int H, int I, int K, uint64_t seed, uint64_t 
     return MAPF_OK;
 }
 
+template <int RW, int RPL>
+int launch_plan_repair(mapf_env *env, int H, int I, int K, uint64_t seed, uint64_t env_offset, uint8_t *d_actions, int32_t *d_arrival,
+                       int32_t *d_collisions, cudaStream_t st)
+{
+    const EnvDims &d = env->d;
+    // the ten tables, then the current and the candidate paths (u16[N][H+1] each), rounded to 16 bytes
+    const size_t warp_words = ((size_t)kRepairTables * (H + 1) * 32 * RPL * RW + (size_t)d.N * (H + 1) + 3) & ~(size_t)3;
+    const int64_t block_bytes = (int64_t)kPlanWarps * warp_words * 4;
+    int64_t blocks = 0;
+    int rc = plan_blocks(env, plan_repair_kernel<RW, RPL>, d.B, block_bytes, blocks);
+    if (rc != MAPF_OK) return rc;
+    rc = reserve_plan_scratch(env, (int64_t)kPlanCounterWords * 4 + blocks * block_bytes, st, "mapf_env_plan_repair: scratch");
+    if (rc != MAPF_OK) return rc;
+    RepairArgs z;
+    z.I = I, z.K = K;
+    z.key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
+    z.env_offset = env_offset;
+    z.collisions = d_collisions;
+    MAPF_CUDA(cudaMemsetAsync(env->pp_scratch, 0, 4, st));
+    plan_repair_kernel<RW, RPL><<<(unsigned)blocks, kPlanWarps * 32, 0, st>>>(plan_args(env, H, warp_words, d_actions, d_arrival), z);
+    MAPF_CUDA(cudaGetLastError());
+    return MAPF_OK;
+}
+
 }  // namespace
 
 // rows per lane RPL = ceil(L / 32) next to the handle's RW: L <= 24 (1, 1), <= 56 (2, 1..2), <= 88 (3, 2..3), <= 120 (4, 3..4)
@@ -754,5 +1144,25 @@ int mapf_launch_plan_lns(mapf_env *env, int H, int iterations, int neighborhood,
     }
 #undef MAPF_PLAN_LNS_CASE
     mapf_set_error("mapf_env_plan_lns: unsupported map size");
+    return MAPF_EINVAL;
+}
+
+int mapf_launch_plan_repair(mapf_env *env, int H, int iterations, int neighborhood, uint64_t seed, uint64_t env_offset, uint8_t *d_actions,
+                            int32_t *d_arrival, int32_t *d_collisions, cudaStream_t st)
+{
+    const int rpl = (env->d.L + 31) / 32;
+#define MAPF_PLAN_REPAIR_CASE(rw, r) \
+    case rw * 8 + r: return launch_plan_repair<rw, r>(env, H, iterations, neighborhood, seed, env_offset, d_actions, d_arrival, d_collisions, st)
+    switch (env->d.RW * 8 + rpl) {
+        MAPF_PLAN_REPAIR_CASE(1, 1);
+        MAPF_PLAN_REPAIR_CASE(2, 1);
+        MAPF_PLAN_REPAIR_CASE(2, 2);
+        MAPF_PLAN_REPAIR_CASE(3, 2);
+        MAPF_PLAN_REPAIR_CASE(3, 3);
+        MAPF_PLAN_REPAIR_CASE(4, 3);
+        MAPF_PLAN_REPAIR_CASE(4, 4);
+    }
+#undef MAPF_PLAN_REPAIR_CASE
+    mapf_set_error("mapf_env_plan_repair: unsupported map size");
     return MAPF_EINVAL;
 }

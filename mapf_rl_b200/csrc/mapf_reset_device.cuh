@@ -42,7 +42,10 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k)
 // PURPOSE_LEVEL: the setting a sized handle's reset draws for the slot (reset_levels_kernel), counter (g, 3, 0)
 // PURPOSE_ORDER: agent a's key in priority order r of the planner (plan_orders_kernel), counter (g, 4 | r << 8, a)
 // PURPOSE_LNS: agent a's key in iteration i of plan improvement (plan_lns_kernel), counter (g, 5 | i << 8, a)
-enum : uint32_t { PURPOSE_DENSITY = 0, PURPOSE_MAP = 1, PURPOSE_AGENT = 2, PURPOSE_LEVEL = 3, PURPOSE_ORDER = 4, PURPOSE_LNS = 5 };
+// PURPOSE_REPAIR: agent a's key in iteration i of plan repair (plan_repair_kernel), counter (g, 6 | i << 8, a)
+enum : uint32_t {
+    PURPOSE_DENSITY = 0, PURPOSE_MAP = 1, PURPOSE_AGENT = 2, PURPOSE_LEVEL = 3, PURPOSE_ORDER = 4, PURPOSE_LNS = 5, PURPOSE_REPAIR = 6
+};
 
 #ifdef MAPF_ENABLE_DIAG
 // diagnosis build: cycles of the generator's phases for environment 0 (profiles/tools/r2_generator_phases.py); accumulated in
